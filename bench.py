@@ -20,6 +20,7 @@ One "step" = one pass of the fused Viterbi path (sapr_viterbi through the C ABI)
   audio   : configs[4] shape: 16 kHz synthetic audio -> fused MFCC kernel -> Viterbi recognition on the device
 
 `--impl reference` times the reference's algorithm on the host cores instead (oracle port, all threads).
+`--dump-outputs DIR` saves what the last timed step returned, so that two builds can be compared output for output.
 """
 import argparse
 import json
@@ -33,11 +34,15 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 
 M_WORDS, N_STATES, DIM, T_FRAMES = 11, 8, 39, 200
 ALG_BYTES_PER_UTT = 4 * T_FRAMES * DIM + T_FRAMES + 4 + 8          # 31 412 (SURVEY 8d, cfg 2)
 ESTEP_BYTES_PER_UTT = 4 * T_FRAMES * DIM + 8                       # 31 208 (cfg 3)
 SEED = 20241118 + 2
+# --dump-outputs keeps under 64 MB: words and scores of at most 2 M utterances (20 B each with the utterance id) and the state
+# paths of at most 16 384 utterances (200 frames x 4 B each, 13 MB); larger batches are sampled with a fixed seed
+DUMP_WORD_UTTS, DUMP_PATH_UTTS = 1 << 21, 1 << 14
 
 
 def peaks():
@@ -126,6 +131,26 @@ def cpu_sample(corpus_host, offs_host, labels_host, A, means, var, leg, target_s
     return nu * per / dt, nu, nthreads, dt
 
 
+def dump_outputs(out_dir, out, B):
+    """Write what the timed Viterbi call returned in its last step as .npy files: best_word (float32, -1 = no word) and
+    best_score (float64) per utterance, path (float32, [utterances, T] state indices), and the utterance ids of their rows
+    (utterance, path_utterance; float64).  The inputs depend on the arguments only, so two builds can be compared file by file."""
+    def pick(n):
+        if B <= n:
+            return np.arange(B)
+        return np.sort(np.random.default_rng(SEED).choice(B, n, replace=False))
+
+    os.makedirs(out_dir, exist_ok=True)
+    uw, up = pick(DUMP_WORD_UTTS), pick(DUMP_PATH_UTTS)
+    arrays = {"best_word": out["best_word"].cpu().numpy()[uw].astype(np.float32),
+              "best_score": out["best_score"].cpu().numpy()[uw].astype(np.float64),
+              "utterance": uw.astype(np.float64),
+              "path": out["path"].view(B, T_FRAMES).cpu().numpy()[up].astype(np.float32),
+              "path_utterance": up.astype(np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def reference_arm(args):
     """--impl reference: the reference's algorithm on the host cores (oracle port; the Python reference does
     not travel to the GPU box and runs ~1e4x slower)."""
@@ -176,7 +201,14 @@ def main():
     ap.add_argument("--precision", default="fp32", choices=["fp32", "fp64"])
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the words, scores and (a sample of the) state paths of the last step to "
+                         "DIR/<name>.npy (rank 0's shard)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the sapr_b200 path; --impl reference decodes another corpus")
     if args.impl == "reference":
         return reference_arm(args)
 
@@ -239,6 +271,8 @@ def main():
     ms_per_step = float(ms.item()) / args.steps
     value = world * updates_per_step / (ms_per_step / 1e3)
     clocks = sampler.stop(t0, t1) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, B)
 
     # ---- roofline of the dominant kernel (this rank) ----
     peak, peak_src = peaks()
