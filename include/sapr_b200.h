@@ -66,7 +66,8 @@ int sapr_sync(sapr_ctx *ctx);
  * dominant kernels on the ctx stream.  sapr_profile_read synchronises, then returns the summed duration (ms)
  * and launch count of kernel class `which` (0 = fused Viterbi, 1 = Viterbi finish/back-trace,
  * 2 = fused E-step forward/backward, 3 = E-step feature statistics, 4 = ergodic tensor-core emission,
- * 5 = ergodic tensor-core forward) since the last sapr_profile(ctx, 1). */
+ * 5 = ergodic tensor-core forward, 6 = fp32 word near-tie re-decoding, 7 = dense-topology fused Viterbi (its arg-max / back-trace
+ * counts as 1), 8 = float64 re-decoding of dense-topology word near-ties) since the last sapr_profile(ctx, 1). */
 int sapr_profile(sapr_ctx *ctx, int enable);
 int sapr_profile_read(sapr_ctx *ctx, int which, double *ms, int64_t *launches);
 
@@ -88,6 +89,13 @@ int sapr_init_stats(sapr_ctx *ctx, const float *X, int ldx, const int64_t *offse
 
 /* ---- batched Viterbi: custom_hmm.py:462-514 (decode) for every utterance x model, plus the
  * strict-'>' argmax over models of decoder.py:42-47.  DIAG emission + ENTRY_EXIT topology, fused.
+ * DIAG emission + DENSE topology (hmmlearn GaussianHMM.decode per model, S <= 32, else SAPR_E_RANGE: large ergodic models keep
+ * sapr_hl_decode): delta_0(j) = ln pi_j + e_0(j), delta_t(j) = max_i (delta_{t-1}(i) + ln A_ij) + e_t(j), a model's score is
+ * max_j delta_{T-1}(j) (no exit arc), the back-trace takes the first maximum (lowest index).  best_word is the strict-'>' arg-max
+ * (first best wins, -1 when every model scores -inf; best_path then holds model 0's path), best_path holds states 0..S-1.
+ * SAPR_FP64 equals sapr_hl_decode per model bit for bit; SAPR_FP32 is the fused fp32 kernel (csrc/viterbi_dense.cu) with the
+ * near-tie pass below.  DENSE sets refuse first_frames > 0, all_paths and model_of_utt (SAPR_E_INVALID); max_T must cover the
+ * longest utterance.
  *   model_of_utt  int32[B] or NULL; NULL = score against all M models
  *   max_T         the longest utterance of the batch; it sizes the scratch, and an utterance longer than max_T is decoded
  *                 on its first max_T frames only (never past the scratch)
@@ -101,7 +109,7 @@ int sapr_viterbi(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, const i
                  int64_t total_frames, int max_T, const int32_t *model_of_utt, int precision,
                  int first_frames, int32_t *best_word, double *best_score, double *scores,
                  uint8_t *best_path, uint8_t *all_paths);
-/* fp32 production mode (tensor-core kernels, all models, all_paths == NULL): an utterance whose best and second-best word
+/* fp32 production mode (tensor-core kernels or the DENSE kernel, all models, all_paths == NULL): an utterance whose best and second-best word
  * scores differ by less than 8e-6 |best| -- closer than the fp32 scores resolve -- is re-decoded in float64 inside the same
  * call (word, score, score row and path then are the verification mode's), so the recognised word equals the float64 one
  * except on exact float64 ties (decoder.py:42-47 keeps the first).  n = utterances flagged by the last call on this context

@@ -140,6 +140,16 @@ extern "C" int sapr_models_create(sapr_ctx *ctx, int M, int N, int D, int emissi
         rc |= dalloc(ctx, &m->P, (size_t)M * S * D * D);
         rc |= dalloc(ctx, &m->cstS, (size_t)M * S);
     }
+    if (!rc && emission == SAPR_EMIT_DIAG && topology == SAPR_TOPO_DENSE && S <= 32 && m->Dp <= 1024) {
+        float2 *arc = nullptr;
+        rc |= dalloc(ctx, &m->dn_piv, (size_t)m->Dp);
+        rc |= dalloc(ctx, &m->dn_w, (size_t)M * nch * S * 8);
+        rc |= dalloc(ctx, &m->dn_cst, (size_t)M * S);
+        rc |= dalloc(ctx, &m->dn_lpi, (size_t)M * S);
+        rc |= dalloc(ctx, &arc, (size_t)M * S * S);
+        rc |= dalloc(ctx, &m->dn_start, (size_t)M * (S + 1));
+        m->dn_arc = arc;
+    }
     if (!rc && sapr_tc_eligible(m)) {
         unsigned char *img = nullptr;
         rc |= dalloc(ctx, &img, sapr_tc_image_bytes(m, nullptr, nullptr));
@@ -154,7 +164,8 @@ extern "C" int sapr_models_destroy(sapr_models *m) {
     if (!m) return SAPR_OK;
     cudaStreamSynchronize(m->ctx->stream);
     void *ptrs[] = {m->mean, m->cov, m->A, m->pi, m->logA, m->logpi, m->la64, m->lb64, m->la32, m->lb32,
-                    m->pk64, m->pk32, m->cst64, m->cst32, m->P, m->cstS, m->tc_image};
+                    m->pk64, m->pk32, m->cst64, m->cst32, m->P, m->cstS, m->tc_image, m->dn_piv, m->dn_w, m->dn_cst,
+                    m->dn_lpi, m->dn_arc, m->dn_start};
     for (void *p : ptrs) if (p) cudaFree(p);
     delete m;
     return SAPR_OK;
@@ -296,6 +307,10 @@ int sapr_models_prepare(sapr_models *m) {
         SAPR_LAUNCH_CHECK(ctx);
         if (m->tc_image) {
             int rc = sapr_tc_prepare(m);
+            if (rc) return rc;
+        }
+        if (m->dn_w) {
+            int rc = sapr_dense_prepare(m);
             if (rc) return rc;
         }
     } else {

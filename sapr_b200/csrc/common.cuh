@@ -90,6 +90,12 @@ struct sapr_models {
     // tensor-core Viterbi image (viterbi_tc.cu): fp16 hi/lo weights in shared-memory layout + (g, s) + transitions
     void *tc_image = nullptr;
     int tc_ctas_per_sm = 1;
+    // DENSE + DIAG sets with S <= 32 (viterbi_dense.cu): pivot p[Dp]; per model [chunk][state][8] = (a x4, b x4) with
+    // a = (mu - p) / var, b = -1 / (2 var); cst[S] = -0.5 (D ln 2pi + sum ln var + sum (mu - p)^2 / var); ln pi [S];
+    // finite arcs (ln A, source) grouped by destination [S*S] float2 with start[S + 1]
+    float *dn_piv = nullptr, *dn_w = nullptr, *dn_cst = nullptr, *dn_lpi = nullptr;
+    void *dn_arc = nullptr;
+    int32_t *dn_start = nullptr;
     bool valid = false;
 };
 
@@ -145,6 +151,10 @@ int sapr_flag_setup(sapr_ctx *ctx, SaprFlag *flag, bool first_chunk);   // works
 int sapr_ws_reserve(sapr_ctx *ctx, int slot, size_t bytes);   // grows ctx->ws[slot]
 int sapr_pin_reserve(sapr_ctx *ctx, int slot, size_t bytes);  // grows ctx->pin[slot]
 int sapr_models_prepare(sapr_models *m);                      // recompute the derived arrays on device
+int sapr_dense_prepare(sapr_models *m);                       // fp32 arrays of the dense Viterbi (viterbi_dense.cu)
+int sapr_viterbi_dense(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, const int64_t *offsets, int B, int64_t total_frames,
+                       int max_T, const int32_t *model_of_utt, int precision, int first_frames, int32_t *best_word, double *best_score,
+                       double *scores, uint8_t *best_path, uint8_t *all_paths);
 // float64 emission matrix E[total_frames][S] of model mi for a batch (DIAG or SAPR emission)
 bool sapr_tc_eligible(const sapr_models *m);
 size_t sapr_tc_image_bytes(const sapr_models *m, int *nck_out, int *ncols_out);

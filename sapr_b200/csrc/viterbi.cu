@@ -621,6 +621,9 @@ extern "C" int sapr_viterbi(sapr_ctx *ctx, sapr_models *m, const float *X, int l
                             uint8_t *best_path, uint8_t *all_paths) {
     if (!ctx || !m || !X || !offsets) return SAPR_E_INVALID;
     if (!m->valid) SAPR_FAIL(ctx, SAPR_E_INVALID, "viterbi: model parameters not set");
+    if (m->topology == SAPR_TOPO_DENSE)
+        return sapr_viterbi_dense(ctx, m, X, ldx, offsets, B, total_frames, max_T, model_of_utt, precision, first_frames, best_word,
+                                  best_score, scores, best_path, all_paths);
     if (m->emission != SAPR_EMIT_DIAG || m->topology != SAPR_TOPO_ENTRY_EXIT)
         SAPR_FAIL(ctx, SAPR_E_INVALID, "viterbi: fused kernel needs DIAG emission + ENTRY_EXIT topology");
     if (ldx % 4 || ldx < m->Dp) SAPR_FAIL(ctx, SAPR_E_INVALID, "viterbi: ldx must be a multiple of 4 and >= D padded");

@@ -1,7 +1,9 @@
 """Drop-in for assignment2/decoder.py: same ``Decoder`` class (constructor, ``load_models``,
 ``decode_sequence``, ``decode_word_samples``, ``decode_vocabulary``) plus ``decode_batch``, which scores
 every utterance against every word model in ONE fused Viterbi launch (the per-model Python loop of
-decoder.py:42-47 becomes the in-kernel argmax).
+decoder.py:42-47 becomes the in-kernel argmax).  ``decode_batch`` takes custom models trained with
+semantics="standard" (left-to-right, entry/exit states) and hmmlearn-style models (every state emits,
+dense transmat + startprob, up to 32 states; csrc/viterbi_dense.cu).
 
 Model order: the reference iterates ``impl_dir.glob(pattern)`` (filesystem order, SURVEY D8) and keeps the
 first best under strict ``>``; pass ``vocab_order`` to fix the order explicitly.
@@ -15,11 +17,28 @@ from typing import Dict, List, Tuple
 
 import numpy as np
 
-from ._lib import EMIT_DIAG, FP32, FP64, TOPO_ENTRY_EXIT
+from ._lib import EMIT_DIAG, FP32, FP64, TOPO_DENSE, TOPO_ENTRY_EXIT
 from .engine import PackedBatch, WordModels
 from .mfcc_extract import load_mfccs_by_word
 
 logging.basicConfig(level=logging.INFO)
+
+
+def stack_hmmlearn_models(models) -> Tuple[np.ndarray, np.ndarray, np.ndarray, np.ndarray]:
+    """(means [M, S, D], variances [M, S, D], transmat [M, S, S], startprob [M, S]) of hmmlearn-style GaussianHMM models with
+    diagonal covariances.  Reads only the public attributes ``means_``, ``covars_`` (the getter's expanded (S, D, D) form;
+    its diagonal is taken), ``transmat_`` and ``startprob_``, so pickles of hmmlearn's own class stack too.  Every model must
+    have the same number of states and features (ValueError otherwise)."""
+    means = [np.asarray(m.means_, dtype=np.float64) for m in models]
+    shapes = {mu.shape for mu in means}
+    if len(shapes) != 1:
+        raise ValueError(f"batched decoding needs models of one shape (states, features); got {sorted(shapes)}")
+    var = []
+    for m in models:
+        c = np.asarray(m.covars_, dtype=np.float64)
+        var.append(np.diagonal(c, axis1=1, axis2=2) if c.ndim == 3 else c)
+    return (np.stack(means), np.stack(var), np.stack([np.asarray(m.transmat_, dtype=np.float64) for m in models]),
+            np.stack([np.asarray(m.startprob_, dtype=np.float64) for m in models]))
 
 
 class Decoder:
@@ -61,8 +80,14 @@ class Decoder:
                 best_score, best_word, best_states = log_prob, word, states
         return best_word, best_score, best_states
 
-    # ---- batched path: custom "standard"-semantics models only (diagonal emission, all frames) ----
+    # ---- batched path: custom "standard"-semantics models (diagonal emission, all frames) or hmmlearn models ----
     def _word_models(self) -> WordModels:
+        if self._dev is None and self.implementation == "hmmlearn":
+            means, var, tm, sp = stack_hmmlearn_models([self.models[w] for w in self.vocab])
+            M, S, D = means.shape
+            dev = WordModels(M, S, D, EMIT_DIAG, TOPO_DENSE)
+            dev.set(means, var, tm, sp)
+            self._dev = dev
         if self._dev is None:
             ms = [self.models[w] for w in self.vocab]
             if any(getattr(m, "semantics", None) != "standard" for m in ms):
@@ -76,7 +101,11 @@ class Decoder:
         return self._dev
 
     def decode_batch(self, features: List[np.ndarray], true_labels=None):
-        """features: list of (D, T_u) arrays.  Returns (words, scores, paths) for the whole list; with ``true_labels``
+        """features: list of (D, T_u) arrays.  Returns (words, scores, paths) for the whole list; a word is None when no model
+        can produce the utterance.  ``precision="fp64"`` (constructor) selects the float64 verification mode; the fp32
+        default re-decodes word near-ties in float64, so its words are the float64 ones.  Custom models give the reference's
+        decode (entry/exit states); hmmlearn models give GaussianHMM.decode per model (paths over states 0..S-1, the first
+        best model wins ties as in decoder.py:42-47).  With ``true_labels``
         (vocabulary indices) the confusion counts and the accuracy of eval.py:28-38 are accumulated on the device from the
         kernel's predictions and left in ``self.last_confusion`` = (int64 [M, M + 1] array, accuracy)."""
         dev = self._word_models()
@@ -110,7 +139,8 @@ class Decoder:
     def decode_vocabulary(self, feature_set: str = "feature_set", verbose: bool = True) -> Dict[str, List[Dict]]:
         """decoder.py:79-95.  Custom models with the standard (diagonal, all-frames) semantics are recognised in ONE fused
         Viterbi launch per word list instead of utterances x models calls (same result dictionaries; SAPR_DECODE_LOOP=1 keeps the
-        reference's per-sequence loop)."""
+        reference's per-sequence loop).  hmmlearn models keep the per-sequence loop here; ``decode_batch`` and
+        ``eval_hmm(..., batched=True)`` are their batched route."""
         import os
         batched = self._batchable() and os.environ.get("SAPR_DECODE_LOOP", "0") != "1"
         all_results = {}

@@ -107,11 +107,14 @@ class WordModels:
         self.ctx.check(self.lib.sapr_models_get(self.h, ptr(means), ptr(covars), ptr(A), ptr(sp)))
         return means, covars, A, sp
 
-    # ---- decoding (custom_hmm.py:462-514 + decoder.py:42-47) ----
+    # ---- decoding (custom_hmm.py:462-514 / GaussianHMM.decode + decoder.py:42-47) ----
     def viterbi(self, batch: PackedBatch, model_of_utt=None, precision=FP32, first_frames=0, want_scores=False,
                 want_path=True, all_paths=False):
         torch = _torch()
         dev = batch.X.device
+        if first_frames > 0 and self.topology == TOPO_DENSE:
+            raise _lib.SaprError(-1, "first_frames > 0 (walk only the first frames) is the custom models' as-written decode; "
+                                     "dense (hmmlearn) models always decode every frame")
         if first_frames > 0 and batch.min_T < first_frames:
             raise IndexError("utterance shorter than the frames decode walks (reference: custom_hmm.py:466 with T_frames < D)")
         B, M = batch.B, self.M

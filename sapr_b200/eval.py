@@ -1,8 +1,9 @@
 """Drop-in for the metrics half of assignment2/eval.py: ``extract_labels`` (eval.py:16-25),
 ``calculate_metrics`` (eval.py:28-38), ``log_per_word_accuracy`` (eval.py:99-105) and ``eval_hmm``
 (eval.py:108-136) with the same arguments and the same result dictionary.  Decoding goes through the drop-in
-``Decoder``; with ``batched=True`` (custom models trained with semantics="standard") the whole evaluation set
-is recognised in ONE fused Viterbi launch instead of utterances x models Python calls.
+``Decoder``; with ``batched=True`` (custom models trained with semantics="standard", or hmmlearn models of one shape
+with up to 32 states) the whole evaluation set is recognised in ONE fused Viterbi launch instead of utterances x models
+Python calls.  The default (``batched=False``) keeps the reference's per-sequence loop for both implementations.
 
 The confusion matrix follows sklearn.metrics.confusion_matrix as eval.py:35 calls it (no ``labels=``): rows and
 columns are the sorted union of the label indices that occur, so a word that is never seen nor predicted has no

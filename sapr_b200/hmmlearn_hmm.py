@@ -6,6 +6,10 @@ settable ``means_ / covars_ / transmat_ / startprob_``, ``fit / score / decode /
 ``monitor_.history``.  hmmlearn 0.3.3 itself is not vendored in the reference and not installable here, so
 the arithmetic follows SURVEY.md Appendix B (parity unpinned by the reference); it runs on the DENSE-topology
 float64 kernels of csrc/hmmlearn.cu.  ``HMMLearnModel`` is the reference's wrapper class, same signature.
+
+``decode`` is one model at a time, as decoder.py:43 calls it.  To recognise many utterances against a vocabulary of such
+models at once, ``Decoder.decode_batch`` stacks them into one DENSE ``WordModels`` set (fp32 fused kernel of
+csrc/viterbi_dense.cu for up to 32 states; its float64 verification mode equals this class's ``decode`` bit for bit).
 """
 from __future__ import annotations
 
