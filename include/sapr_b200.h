@@ -67,7 +67,8 @@ int sapr_sync(sapr_ctx *ctx);
  * and launch count of kernel class `which` (0 = fused Viterbi, 1 = Viterbi finish/back-trace,
  * 2 = fused E-step forward/backward, 3 = E-step feature statistics, 4 = ergodic tensor-core emission,
  * 5 = ergodic tensor-core forward, 6 = fp32 word near-tie re-decoding, 7 = dense-topology fused Viterbi (its arg-max / back-trace
- * counts as 1), 8 = float64 re-decoding of dense-topology word near-ties) since the last sapr_profile(ctx, 1). */
+ * counts as 1), 8 = float64 re-decoding of dense-topology word near-ties, 9 = dense-topology fp32 E-step forward / backward,
+ * 10 = its feature statistics) since the last sapr_profile(ctx, 1). */
 int sapr_profile(sapr_ctx *ctx, int enable);
 int sapr_profile_read(sapr_ctx *ctx, int which, double *ms, int64_t *launches);
 
@@ -140,6 +141,14 @@ int sapr_viterbi_host(sapr_ctx *ctx, sapr_models *m, const float *X_host, int ld
  *           sum gamma (x-mu_old)^2 [S*D]
  *   loglik  float64[B]  logsumexp(alpha_scaled[T-1,:]) as the reference reports it (SURVEY D6)
  *   gamma_out float32/float64 [sum_T * N] nullable debug output (emitting states only)            */
+/* DIAG emission + DENSE topology (hmmlearn GaussianHMM.fit's E-step, every model at once): model_of_utt is required (NULL =
+ * SAPR_E_INVALID), order as above.  stats float64[M * sapr_hl_stats_len(S, D)], zeroed by the call, per model
+ * [start S | trans S*S | post S | obs S*D | obs2 S*D] as sapr_hl_estep gives it; loglik = log P(X_u); gamma_out [sum_T][S]
+ * (fp32 in SAPR_FP32, float64 in SAPR_FP64).  SAPR_FP64 runs sapr_hl_estep per model on that model's utterances in batch order,
+ * so stats and loglik equal GaussianHMM.fit's E-step for the word bit for bit (any S sapr_hl_estep takes).  SAPR_FP32 is the
+ * fused kernel of csrc/estep_dense.cu (S <= 32, else SAPR_E_RANGE; max_T must cover the longest utterance): per-frame
+ * log-shifted linear recursions, so utterances far from their model stay finite; an utterance the model cannot produce gets
+ * loglik -inf and contributes nothing.  Two identical calls give identical bits.  */
 int64_t sapr_stats_stride(int N, int D);
 int sapr_estep(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, const int64_t *offsets, int B,
                int64_t total_frames, int max_T, const int32_t *model_of_utt, const int32_t *order,

@@ -141,14 +141,16 @@ extern "C" int sapr_models_create(sapr_ctx *ctx, int M, int N, int D, int emissi
         rc |= dalloc(ctx, &m->cstS, (size_t)M * S);
     }
     if (!rc && emission == SAPR_EMIT_DIAG && topology == SAPR_TOPO_DENSE && S <= 32 && m->Dp <= 1024) {
-        float2 *arc = nullptr;
+        float2 *arc = nullptr, *arcs = nullptr;
         rc |= dalloc(ctx, &m->dn_piv, (size_t)m->Dp);
         rc |= dalloc(ctx, &m->dn_w, (size_t)M * nch * S * 8);
         rc |= dalloc(ctx, &m->dn_cst, (size_t)M * S);
         rc |= dalloc(ctx, &m->dn_lpi, (size_t)M * S);
         rc |= dalloc(ctx, &arc, (size_t)M * S * S);
         rc |= dalloc(ctx, &m->dn_start, (size_t)M * (S + 1));
-        m->dn_arc = arc;
+        rc |= dalloc(ctx, &arcs, (size_t)M * S * S);
+        rc |= dalloc(ctx, &m->dn_starts, (size_t)M * (S + 1));
+        m->dn_arc = arc; m->dn_arcs = arcs;
     }
     if (!rc && sapr_tc_eligible(m)) {
         unsigned char *img = nullptr;
@@ -165,7 +167,7 @@ extern "C" int sapr_models_destroy(sapr_models *m) {
     cudaStreamSynchronize(m->ctx->stream);
     void *ptrs[] = {m->mean, m->cov, m->A, m->pi, m->logA, m->logpi, m->la64, m->lb64, m->la32, m->lb32,
                     m->pk64, m->pk32, m->cst64, m->cst32, m->P, m->cstS, m->tc_image, m->dn_piv, m->dn_w, m->dn_cst,
-                    m->dn_lpi, m->dn_arc, m->dn_start};
+                    m->dn_lpi, m->dn_arc, m->dn_start, m->dn_arcs, m->dn_starts};
     for (void *p : ptrs) if (p) cudaFree(p);
     delete m;
     return SAPR_OK;

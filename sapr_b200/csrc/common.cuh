@@ -92,10 +92,11 @@ struct sapr_models {
     int tc_ctas_per_sm = 1;
     // DENSE + DIAG sets with S <= 32 (viterbi_dense.cu): pivot p[Dp]; per model [chunk][state][8] = (a x4, b x4) with
     // a = (mu - p) / var, b = -1 / (2 var); cst[S] = -0.5 (D ln 2pi + sum ln var + sum (mu - p)^2 / var); ln pi [S];
-    // finite arcs (ln A, source) grouped by destination [S*S] float2 with start[S + 1]
+    // finite arcs (ln A, source) grouped by destination [S*S] float2 with start[S + 1]; the same arcs (A, destination) grouped
+    // by source with starts[S + 1] (the E-step's backward sweep, estep_dense.cu)
     float *dn_piv = nullptr, *dn_w = nullptr, *dn_cst = nullptr, *dn_lpi = nullptr;
-    void *dn_arc = nullptr;
-    int32_t *dn_start = nullptr;
+    void *dn_arc = nullptr, *dn_arcs = nullptr;
+    int32_t *dn_start = nullptr, *dn_starts = nullptr;
     bool valid = false;
 };
 
@@ -164,6 +165,9 @@ int sapr_viterbi_tc_launch(sapr_ctx *ctx, sapr_models *m, const float *X, int ld
                            double *scores, uint8_t *best_path, uint8_t *all_paths, float *dbgE);
 int sapr_estep_tc_launch(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, const int64_t *offsets, int B, int max_T,
                          const int32_t *order, const int32_t *model_start, float *gamma, float *ustats, double *loglik);
+int sapr_estep_dense(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, const int64_t *offsets, int B, int64_t total_frames,
+                     int max_T, const int32_t *model_of_utt, const int32_t *order, int precision, double *stats, double *loglik,
+                     void *gamma_out);
 int sapr_emission_into(sapr_ctx *ctx, sapr_models *m, int mi, const float *X, int ldx, const int64_t *offsets, int B,
                        int64_t total_frames, double *E);
 

@@ -754,6 +754,8 @@ extern "C" int sapr_estep(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx
                           int precision, double *stats, double *loglik, void *gamma_out) {
     if (!ctx || !m || !X || !offsets || !model_of_utt || !stats || !loglik) return SAPR_E_INVALID;
     if (!m->valid) SAPR_FAIL(ctx, SAPR_E_INVALID, "estep: model parameters not set");
+    if (m->topology == SAPR_TOPO_DENSE)
+        return sapr_estep_dense(ctx, m, X, ldx, offsets, B, total_frames, max_T, model_of_utt, order, precision, stats, loglik, gamma_out);
     if (m->emission != SAPR_EMIT_DIAG || m->topology != SAPR_TOPO_ENTRY_EXIT)
         SAPR_FAIL(ctx, SAPR_E_INVALID, "estep: fused kernel needs DIAG emission + ENTRY_EXIT topology");
     if (ldx % 4 || ldx < m->Dp) SAPR_FAIL(ctx, SAPR_E_INVALID, "estep: ldx must be a multiple of 4 and >= D padded");

@@ -34,11 +34,12 @@ template <int NMAX> struct DnBits {
 static int dn_nb(int S) { return S <= 8 ? 3 : (S <= 16 ? 4 : 5); }
 
 // ------------------------------------------------------------------------------------------------
-// derived parameters (sapr_models_prepare): pivot, fp32 emission weights, ln pi, arc lists.  One block.
+// derived parameters (sapr_models_prepare): pivot, fp32 emission weights, ln pi, arc lists (by destination with ln A for the
+// Viterbi, by source with A for the E-step's backward sweep, csrc/estep_dense.cu).  One block.
 __global__ void k_dense_prepare(int M, int S, int D, int Dp, const double *__restrict__ mean, const double *__restrict__ var,
                                 const double *__restrict__ A, const double *__restrict__ pi, float *__restrict__ piv,
                                 float *__restrict__ w, float *__restrict__ cst, float *__restrict__ lpi, float2 *__restrict__ arc,
-                                int32_t *__restrict__ start) {
+                                int32_t *__restrict__ start, float2 *__restrict__ arcs, int32_t *__restrict__ starts) {
     __shared__ double s_p[1024];
     const int nch = Dp / 4;
     for (int d = threadIdx.x; d < Dp; d += blockDim.x) {
@@ -79,13 +80,23 @@ __global__ void k_dense_prepare(int M, int S, int D, int Dp, const double *__res
             }
         }
         start[(size_t)m * (S + 1) + S] = n;
+        n = 0;
+        for (int i = 0; i < S; i++) {                          // the same arcs grouped by source, destinations ascending
+            starts[(size_t)m * (S + 1) + i] = n;
+            for (int j = 0; j < S; j++) {
+                const double a = Am[(size_t)i * S + j];
+                if (log(a) > -INFINITY) arcs[(size_t)m * S * S + n++] = make_float2((float)a, (float)j);
+            }
+        }
+        starts[(size_t)m * (S + 1) + S] = n;
     }
 }
 
 int sapr_dense_prepare(sapr_models *m) {
     sapr_ctx *ctx = m->ctx;
     k_dense_prepare<<<1, 256, 0, ctx->stream>>>(m->M, m->S, m->D, m->Dp, m->mean, m->cov, m->A, m->pi, m->dn_piv, m->dn_w,
-                                                m->dn_cst, m->dn_lpi, (float2 *)m->dn_arc, m->dn_start);
+                                                m->dn_cst, m->dn_lpi, (float2 *)m->dn_arc, m->dn_start,
+                                                (float2 *)m->dn_arcs, m->dn_starts);
     SAPR_LAUNCH_CHECK(ctx);
     return SAPR_OK;
 }

@@ -157,9 +157,14 @@ class WordModels:
 
     # ---- training (custom_hmm.py:402-460) ----
     def stats_stride(self):
+        if self.topology == TOPO_DENSE:
+            return int(self.lib.sapr_hl_stats_len(self.S, self.D))
         return int(self.lib.sapr_stats_stride(self.N, self.D))
 
     def estep(self, batch: PackedBatch, model_of_utt, order=None, precision=FP32, want_gamma=False):
+        """One E-step, utterance u against model ``model_of_utt[u]``: (stats [M, stats_stride()], per-utterance loglik, gamma or
+        None).  DENSE sets give hmmlearn's statistics per model (``unpack_stats``) and log P(X_u); fp32 = csrc/estep_dense.cu,
+        FP64 = GaussianHMM.fit's E-step per model, bit for bit."""
         torch = _torch()
         dev = batch.X.device
         stats = torch.empty((self.M, self.stats_stride()), dtype=torch.float64, device=dev)
@@ -192,9 +197,14 @@ class WordModels:
         self.ctx.check(self.lib.sapr_mstep(self.ctx.h, self.h, ptr(stats), ptr(fv)))
 
     def unpack_stats(self, stats):
-        """stats tensor/array (M, stride) -> dict of numpy views (G, Xi, occ, s1, s2)."""
+        """stats tensor/array (M, stride) -> dict of numpy views: (G, Xi, occ, s1, s2) for ENTRY_EXIT sets, hmmlearn's
+        (start, trans, post, obs, obs2) for DENSE sets."""
         st = stats.cpu().numpy() if hasattr(stats, "cpu") else np.asarray(stats)
         S, D = self.S, self.D
+        if self.topology == TOPO_DENSE:
+            o = np.cumsum([0, S, S * S, S, S * D])
+            return dict(start=st[:, :o[1]], trans=st[:, o[1]:o[2]].reshape(self.M, S, S), post=st[:, o[2]:o[3]],
+                        obs=st[:, o[3]:o[4]].reshape(self.M, S, D), obs2=st[:, o[4]:].reshape(self.M, S, D))
         return dict(G=st[:, :S], Xi=st[:, S:2 * S], occ=st[:, 2 * S:3 * S],
                     s1=st[:, 3 * S:3 * S + S * D].reshape(self.M, S, D),
                     s2=st[:, 3 * S + S * D:].reshape(self.M, S, D))

@@ -10,6 +10,8 @@ float64 kernels of csrc/hmmlearn.cu.  ``HMMLearnModel`` is the reference's wrapp
 ``decode`` is one model at a time, as decoder.py:43 calls it.  To recognise many utterances against a vocabulary of such
 models at once, ``Decoder.decode_batch`` stacks them into one DENSE ``WordModels`` set (fp32 fused kernel of
 csrc/viterbi_dense.cu for up to 32 states; its float64 verification mode equals this class's ``decode`` bit for bit).
+``fit`` is one model at a time too; ``fit_vocabulary`` fits every word's model at once, with one E-step over all utterances
+of the vocabulary per iteration (csrc/estep_dense.cu) and each model's own M-step.
 """
 from __future__ import annotations
 
@@ -275,3 +277,51 @@ class HMMLearnModel:
             return self.model, log_likelihood
         except Exception as e:   # the reference swallows and returns None (hmmlearn_hmm.py:107-108)
             logging.error(f"Error occurred while training {self.model_name} HMM: {e}")
+
+
+def fit_vocabulary(models: List[GaussianHMM], features, precision: str = "fp32") -> List[GaussianHMM]:
+    """Fit every model of a vocabulary at once: ``features[m]`` is model m's list of (D, T) arrays.  The end state equals
+    ``models[m].fit(X_m, lengths_m)`` for each m: every iteration runs ONE dense E-step over all utterances (each against its
+    own word's model), then, for each model still active, its own ``_do_mstep`` and ``monitor_.report`` -- the order
+    ``GaussianHMM.fit`` uses -- so priors, ``params`` and the zero masks of ``startprob_`` / ``transmat_`` behave as in the
+    per-model fit.  A model leaves the active set when its monitor has converged (its own ``n_iter`` and ``tol``); its
+    parameters then stay as they are.  ``precision="fp64"`` runs GaussianHMM.fit's float64 E-step per model and is bit-identical
+    to the per-model fits; ``"fp32"`` is the fused kernel (up to 32 states).  Returns ``models``."""
+    from ._lib import FP32, FP64
+    from .decoder import stack_hmmlearn_models
+    if precision not in ("fp32", "fp64"):
+        raise ValueError("precision must be 'fp32' or 'fp64'")
+    if len(models) != len(features):
+        raise ValueError(f"{len(models)} models but {len(features)} feature lists")
+    for i, (mdl, f) in enumerate(zip(models, features)):
+        if len(f) == 0:
+            raise ValueError(f"model {i} has no utterances to fit")
+        mdl._check()
+    means, var, tm, sp = stack_hmmlearn_models(models)
+    M, S, D = means.shape
+    feats = [np.asarray(x, dtype=np.float32) for f in features for x in f]
+    if any(x.ndim != 2 or x.shape[0] != D for x in feats):
+        raise ValueError(f"every utterance must be a (D, T) array with D = {D} features")
+    counts = np.array([len(f) for f in features])
+    bounds = np.concatenate([[0], np.cumsum(counts)])
+    batch = PackedBatch.from_features(feats, labels=np.repeat(np.arange(M), counts))
+    dev = WordModels(M, S, D, EMIT_DIAG, TOPO_DENSE)
+    prec = FP64 if precision == "fp64" else FP32
+    for mdl in models:
+        mdl.monitor_ = ConvergenceMonitor(mdl.tol, mdl.n_iter, mdl.verbose)
+        mdl.monitor_._reset()
+    active = [i for i, mdl in enumerate(models) if mdl.n_iter > 0]
+    while active:
+        dev.set(*stack_hmmlearn_models(models))
+        stats, loglik, _ = dev.estep(batch, batch.labels, None, prec)
+        st = dev.unpack_stats(stats)
+        ll = loglik.cpu().numpy()
+        still = []
+        for i in active:
+            mdl = models[i]
+            mdl._do_mstep({k: v[i] for k, v in st.items()})
+            mdl.monitor_.report(float(ll[bounds[i]:bounds[i + 1]].sum()))
+            if not mdl.monitor_.converged:
+                still.append(i)
+        active = still
+    return models

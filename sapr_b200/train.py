@@ -6,6 +6,9 @@ drop-in ``HMM`` / ``HMMLearnModel`` classes, so every E-step / M-step below runs
 Not rebuilt: ``plot_training_progress`` (train.py:16-48, matplotlib figure) -- the per-word log-likelihood
 histories it would plot are returned in ``train_hmm.histories`` instead.
 
+``batched=True`` (hmmlearn models only) fits the whole vocabulary at once with ``hmmlearn_hmm.fit_vocabulary``: one E-step over
+every word's utterances per iteration instead of one per word, same pickles, return value and histories.
+
 ``semantics`` is an addition: ``"sapr"`` (default) = custom_hmm.py as written, ``"standard"`` = diagonal
 Gaussian emission over all frames (SURVEY 0.1); it is forwarded to the custom ``HMM`` only.
 """
@@ -20,7 +23,7 @@ import numpy as np
 import pandas as pd
 
 from .custom_hmm import HMM
-from .hmmlearn_hmm import HMMLearnModel
+from .hmmlearn_hmm import HMMLearnModel, fit_vocabulary
 from .mfcc_extract import load_mfccs, load_mfccs_by_word
 
 VOCABS = ["heed", "hid", "head", "had", "hard", "hud", "hod", "hoard", "hood", "whod", "heard"]   # train.py:89-92
@@ -49,7 +52,9 @@ def save_model(model, model_path: Path) -> None:
 def train_hmm(implementation: Literal["custom", "hmmlearn"] = "hmmlearn", num_states: int = 8, num_features: int = 13,
               n_iter: int = 15, min_covar: float = 0.01, var_floor_factor: float = 0.001,
               feature_set_path: str = "feature_set", models_dir: str = "trained_models", vocabs: List[str] = None,
-              semantics: str = "sapr") -> Dict[str, Union[HMM, HMMLearnModel]]:
+              semantics: str = "sapr", batched: bool = False) -> Dict[str, Union[HMM, HMMLearnModel]]:
+    if batched and implementation != "hmmlearn":
+        raise ValueError("batched=True fits hmmlearn models; custom models train per word (engine.train_words batches them)")
     vocabs = list(VOCABS if vocabs is None else vocabs)
     impl_dir = Path(models_dir) / implementation
     impl_dir.mkdir(parents=True, exist_ok=True)
@@ -60,6 +65,17 @@ def train_hmm(implementation: Literal["custom", "hmmlearn"] = "hmmlearn", num_st
     assert total_features_length == len(feature_set)
 
     hmms, histories = {}, {}
+    if batched:
+        for word in vocabs:
+            hmms[word] = HMMLearnModel(num_states=num_states, model_name=word, n_iter=n_iter, min_covar=min_covar,
+                                       feature_set=feature_set)
+        logging.info(f"Training {len(vocabs)} hmmlearn models at once in {n_iter} iterations...")
+        fit_vocabulary([hmms[w].model for w in vocabs], [features[w] for w in vocabs])
+        for word in vocabs:
+            histories[word] = list(hmms[word].model.monitor_.history)
+            save_model(hmms[word].model, impl_dir / f"{word}_{implementation}_{n_iter}.pkl")
+        train_hmm.histories = histories
+        return hmms
     for word in vocabs:
         logging.info(f"\nTraining model for word: {word}")
         model_path = impl_dir / f"{word}_{implementation}_{n_iter}.pkl"
