@@ -154,17 +154,6 @@ int sapr_estep(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, const int
                int64_t total_frames, int max_T, const int32_t *model_of_utt, const int32_t *order,
                int precision, double *stats, double *loglik, void *gamma_out);
 
-/* Same E-step for the layout the reference trains from -- utterances grouped by word (train.py:94
- * load_mfccs_by_word -> hmm.baum_welch(features[word]), train.py:106-113) -- when they are also equal-length and stored
- * contiguously: X float32 [B*T][ldx], utterance u = frames [u*T, (u+1)*T), utterances model_start_host[m] ..
- * model_start_host[m+1]-1 belong to model m (HOST int32[M+1], model_start_host[0] = 0, [M] = B).  One fused kernel:
- * forward sweep, then the backward sweep with gamma . [x, x^2, 1] accumulated on the tensor cores -- no gamma / emission
- * arrays in HBM (csrc/estep_grouped.cu).  fp32 production mode only (verification: sapr_estep with SAPR_FP64); needs
- * N = 8, M <= 12, D <= 47, T >= 16.  stats / loglik as sapr_estep (loglik indexed by utterance).  The last frame of an
- * utterance whose exit state is unreachable contributes nothing to the feature sums (the reference propagates NaN).   */
-int sapr_estep_grouped(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, int T, int B,
-                       const int32_t *model_start_host, double *stats, double *loglik);
-
 /* ---- M-step: custom_hmm.py:351-400 from the packed statistics (after the cross-GPU all-reduce).
  * floor_var[M] HOST float64: var_floor_factor * mean(diag(global_covariance)) per model.
  * Diagonal statistics: var_j = sum gamma (x-c)^2/occ - (mu_j - c)^2 (equals the diagonal of the

@@ -57,7 +57,6 @@ SIGNATURES = {
     "sapr_decode_mat": (_i32, [_vp, _vp, _i32, _vp, _i32, _vp, _vp]),
     "sapr_update_A": (_i32, [_vp, _vp, _i32, _vp, _vp]),
     "sapr_update_B": (_i32, [_vp, _vp, _i32, _vp, _i32, _i64, _vp, _dbl]),
-    "sapr_estep_grouped": (_i32, [_vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _vp]),
     "sapr_estep_compat": (_i32, [_vp, _vp, _i32, _vp, _i32, _vp, _i32, _i64, _vp, _vp, _vp, _vp]),
     "sapr_decode_compat": (_i32, [_vp, _vp, _i32, _vp, _i32, _i32, _i32, _vp, _vp]),
     "sapr_hl_score": (_i32, [_vp, _vp, _i32, _vp, _i32, _vp, _i32, _i64, _vp]),

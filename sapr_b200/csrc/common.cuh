@@ -37,8 +37,6 @@ struct sapr_ctx {
     struct ProfRec { cudaEvent_t a, b; int which; };
     std::vector<ProfRec> prof;       // used records
     std::vector<ProfRec> prof_pool;  // recycled event pairs
-    // sapr_estep_grouped: the tile table of the last call (re-uploaded only when the grouping changes)
-    std::vector<int32_t> eg_tab;
     bool flag_valid = false;         // ws[8] holds the flag counters of the last fp32 Viterbi call (sapr_viterbi_flagged)
     int flag_maxT = 0, flag_M = 0;   // longest utterance / models of that call (size the re-decoding scratch)
 };

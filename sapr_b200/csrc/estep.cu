@@ -668,17 +668,14 @@ static int launch_estep(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, 
     bool tc_done = false;
     if (std::is_same<R, float>::value && m->tc_image && sapr_tc_eligible(m)) {
         // production fp32 path: emission on the tensor cores, forward and backward sweep of a tile in one persistent CTA
-        const char *env = getenv("SAPR_TC");
-        if (!env || env[0] != '0') {
-            if ((rc = sapr_ws_reserve(ctx, 1, sizeof(float) * (size_t)B * 3 * N))) return rc;
-            if ((rc = sapr_estep_tc_launch(ctx, m, X, ldx, offsets, B, max_T, order, model_start, (float *)gamma,
-                                           (float *)ctx->ws[1], loglik)))
-                return rc;
-            k_reduce_triples<float><<<dim3(3 * N, M), 256, 0, ctx->stream>>>(model_start, N, S, (const float *)ctx->ws[1], 0, B,
-                                                                             stats, stride);
-            SAPR_LAUNCH_CHECK(ctx);
-            tc_done = true;
-        }
+        if ((rc = sapr_ws_reserve(ctx, 1, sizeof(float) * (size_t)B * 3 * N))) return rc;
+        if ((rc = sapr_estep_tc_launch(ctx, m, X, ldx, offsets, B, max_T, order, model_start, (float *)gamma,
+                                       (float *)ctx->ws[1], loglik)))
+            return rc;
+        k_reduce_triples<float><<<dim3(3 * N, M), 256, 0, ctx->stream>>>(model_start, N, S, (const float *)ctx->ws[1], 0, B,
+                                                                         stats, stride);
+        SAPR_LAUNCH_CHECK(ctx);
+        tc_done = true;
     }
     if (!tc_done) {
     // forward/backward lattice scratch, chunked over pairs so it stays bounded (<= ~1 GB)

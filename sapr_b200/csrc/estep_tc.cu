@@ -585,7 +585,7 @@ int sapr_estep_tc_launch(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx,
     prm.scratch = (float *)ctx->ws[7]; prm.maxT = max_T;
     prm.gamma = gamma; prm.ustats = ustats; prm.loglik = loglik;
     prm.Fshift = Fshift; prm.nst_shift = nst_shift; prm.rstride = rstride;
-    prm.pf = getenv("SAPR_ET_PF") ? atoi(getenv("SAPR_ET_PF")) : ET_PF;      // tuning aid
+    prm.pf = ET_PF;
     prm.trace = nullptr;
     const char *trace_path = getenv("SAPR_ET_TRACE");
     if (trace_path) {       // tuning aid: one traced launch, timestamps to a text file

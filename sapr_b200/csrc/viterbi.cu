@@ -633,12 +633,9 @@ extern "C" int sapr_viterbi(sapr_ctx *ctx, sapr_models *m, const float *X, int l
 #define GO(R, BP, NM)                                                                                       \
     return launch_viterbi<R, BP, NM>(ctx, m, X, ldx, offsets, B, total_frames, max_T, model_of_utt,        \
                                      first_frames, best_word, best_score, scores, best_path, all_paths)
-    if (precision == SAPR_FP32 && !model_of_utt && m->tc_image && sapr_tc_eligible(m)) {
-        const char *env = getenv("SAPR_TC");
-        if (!env || env[0] != '0')
-            return sapr_viterbi_tc_launch(ctx, m, X, ldx, offsets, B, total_frames, max_T, first_frames, best_word, best_score,
-                                          scores, best_path, all_paths, nullptr);
-    }
+    if (precision == SAPR_FP32 && !model_of_utt && m->tc_image && sapr_tc_eligible(m))
+        return sapr_viterbi_tc_launch(ctx, m, X, ldx, offsets, B, total_frames, max_T, first_frames, best_word, best_score,
+                                      scores, best_path, all_paths, nullptr);
     if (precision == SAPR_FP32 || precision == SAPR_FP32_SIMT) {
         if (m->N <= 8) GO(float, uint16_t, 8);
         if (m->N <= 15) GO(float, uint16_t, 15);

@@ -638,7 +638,7 @@ __host__ __device__ inline TmSmem tm_smem_layout(int M, int nck, int ncols, int 
     return L;
 }
 
-template <int MG, int NKS, bool BATCH = false>
+template <int MG, int NKS>
 __global__ void __launch_bounds__(TM_THREADS, 1) k_viterbi_tma(const TcParams p, const __grid_constant__ CUtensorMap tmap) {
     extern __shared__ __align__(128) unsigned char smem[];
     const int nck = p.nck, ncols = p.ncols, M = p.M;
@@ -890,31 +890,6 @@ __global__ void __launch_bounds__(TM_THREADS, 1) k_viterbi_tma(const TcParams p,
                     const uint32_t tacc = acc_ready();
                     acc_next();
                     const bool rn = (t & 7) == 0;
-                    if (BATCH) {
-                        // all of this thread's accumulator columns in one go, one wait: the models' recursions are independent
-                        // instruction streams the scheduler can interleave
-                        uint32_t ev[MCMAX][8];
-#pragma unroll
-                        for (int k = 0; k < MCMAX; k++)
-                            if (k < mc) tmem_ld8(tacc + 8u * k, ev[k]);
-                        tmem_ld_wait();
-                        uint32_t bits[MCMAX];
-#pragma unroll
-                        for (int k = 0; k < MCMAX; k++) {
-                            if (k < mc) {
-                                const float4 c03 = lds4(trS + (TC_TRQ * 16u) * k), c47 = lds4(trS + (TC_TRQ * 16u) * k + 16u), cm = lds4(trS + (TC_TRQ * 16u) * k + 32u);
-                                bits[k] = vit_step<false>(U[k], Ux[k], c03, c47, cm.x, cm.y, ev[k], t);
-                            }
-                        }
-#pragma unroll
-                        for (int k = 0; k < MCMAX; k++)
-                            if (k < mc) p.bp[bpo + (uint32_t)k * bp_model] = (uint16_t)bits[k];
-                        if (rn) {
-#pragma unroll
-                            for (int k = 0; k < MCMAX; k++)
-                                if (k < mc) vit_renorm(U[k], Ux[k], base[k]);
-                        }
-                    } else {
 #pragma unroll
                     for (int k = 0; k < MCMAX; k++) {
                         if (k < mc) {
@@ -933,7 +908,6 @@ __global__ void __launch_bounds__(TM_THREADS, 1) k_viterbi_tma(const TcParams p,
                             p.bp[bpo + (uint32_t)k * bp_model] = (uint16_t)bits;
                             if (rn) vit_renorm(U[k], Ux[k], base[k]);
                         }
-                    }
                     }
                     tc_fence_before();
                     bpo += bp_frame;
@@ -1046,14 +1020,11 @@ int sapr_viterbi_tc_launch(sapr_ctx *ctx, sapr_models *m, const float *X, int ld
     const size_t smem = L.total;
     const int MG = (M + TC_GROUPS - 1) / TC_GROUPS;
     // equal-length contiguous batch, best path only: the re-cut kernel (viterbi_v3.cu) when the shape fits it
-    {
-        const char *v3_env = getenv("SAPR_V3");
-        if (!dbgE && !all_paths && Tm > 0 && total_frames == (int64_t)B * max_T && (!v3_env || v3_env[0] != '0') && !getenv("SAPR_TC_TRACE")) {
-            bool taken = false;
-            if ((rc = sapr_viterbi_v3_launch(ctx, m, X, ldx, offsets, B, max_T, first_frames, best_word, best_score, scores, best_path, &taken)))
-                return rc;
-            if (taken) return SAPR_OK;
-        }
+    if (!dbgE && !all_paths && Tm > 0 && total_frames == (int64_t)B * max_T && !getenv("SAPR_TC_TRACE")) {
+        bool taken = false;
+        if ((rc = sapr_viterbi_v3_launch(ctx, m, X, ldx, offsets, B, max_T, first_frames, best_word, best_score, scores, best_path, &taken)))
+            return rc;
+        if (taken) return SAPR_OK;
     }
     // equal-length contiguous batch (every utterance has max_T frames): TMA tensor-map loads, k_viterbi_tma
     const char *tma_env = getenv("SAPR_TMA");
@@ -1155,7 +1126,6 @@ int sapr_viterbi_tc_launch(sapr_ctx *ctx, sapr_models *m, const float *X, int ld
             prm.Fshift = tm_Fshift; prm.nst_shift = 1; prm.rstride = tm_rw;
             if (MG <= 1) rc = launch_tma(k_viterbi_tma<1, 0>, prm, grid);
             else if (MG <= 2) rc = launch_tma(k_viterbi_tma<2, 0>, prm, grid);
-            else if (nck == 10 && getenv("SAPR_TM_BATCH") && getenv("SAPR_TM_BATCH")[0] == '1') rc = launch_tma(k_viterbi_tma<3, 5, true>, prm, grid);
             else if (nck == 10) rc = launch_tma(k_viterbi_tma<3, 5>, prm, grid);
             else if (nck == 4) rc = launch_tma(k_viterbi_tma<3, 2>, prm, grid);
             else rc = launch_tma(k_viterbi_tma<3, 0>, prm, grid);

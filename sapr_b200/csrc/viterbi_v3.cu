@@ -31,10 +31,8 @@ struct V3Params {
     int mod0[TC_GROUPS], nmod[TC_GROUPS], pair0[TC_GROUPS], npair[TC_GROUPS];
     uint32_t rw;                        // bytes per row of the raw ring: (nck + 1) * 16
     long long *trace;                   // [V4_TRACE_ROLES][V4_TRACE_FRAMES][4] clock64 stamps of CTA 0 or null (SAPR_V_TRACE=file)
-    int split_col;                      // SPLIT kernels: accumulator columns of model groups 0-1 (a multiple of 16)
-    int halves;                         // SPLIT kernels: 1 = two CTAs per tile, one column half each (the partial round of a batch)
-    int hmod0[2][4], hnmod[2][4], hplane[2][4], hshift[2][4], hroles[2];      // halves: per half and warp group: first model, models (0-2), decision-word plane and byte, active groups
-    int flags;                          // tuning what-ifs (SAPR_V_EXP, k_viterbi_v4<.., EXP = true>): 1 = no MMAs, 2 = no recursion arithmetic, 4 = no conversion arithmetic, 8 = no back-pointer stores, 16 = every tile of a CTA re-reads its first tile (L2 hits)
+    int split_col;                      // HALF kernels: accumulator columns of model groups 0-1 (a multiple of 16)
+    int hmod0[2][4], hnmod[2][4], hplane[2][4], hshift[2][4], hroles[2];      // HALF kernels: per half and warp group: first model, models (0-2), decision-word plane and byte, active groups
 };
 
 struct V3Smem { uint32_t w, raw, tr, sb, bar, total; };
@@ -403,9 +401,10 @@ __device__ __forceinline__ void mbar_wait2(uint32_t bar_a, uint32_t par_a, uint3
         ::"r"(bar_a), "r"(par_a), "r"(bar_b), "r"(par_b) : "memory");
 }
 
-// SPLIT: each frame's product is issued as two column halves (model groups 0-1 | 2-3) with their own acc_full / acc_empty
-// barriers, so a recursion warp waits for half the MMAs and hands its half of a stage back on its own.
-template <int NKS, bool TRACE = false, bool EXP = false, bool SPLIT = false>      // nck = 2 * NKS feature chunks; EXP: the what-if flags are honoured
+// HALF: the partial round of a batch, TWO CTAs per tile.  Each issues the product of one column half (model groups 0-1 | 2-3,
+// with that half's acc_full / acc_empty barriers) and deals the half's models to all four recursion warp groups (at most two
+// models per thread, V3Params::h*); both convert the tile's features.
+template <int NKS, bool TRACE = false, bool HALF = false>      // nck = 2 * NKS feature chunks
 __global__ void __launch_bounds__(V4_THREADS, 1) k_viterbi_v4(const V3Params p, const __grid_constant__ CUtensorMap tmap) {
     extern __shared__ __align__(128) unsigned char smem[];
     constexpr int nck = 2 * NKS;
@@ -421,9 +420,7 @@ __global__ void __launch_bounds__(V4_THREADS, 1) k_viterbi_v4(const V3Params p, 
     uint32_t *sTmem = reinterpret_cast<uint32_t *>(sBar + 24);
     const uint32_t barRawFull = smem_u32(sBar), barRawEmpty = barRawFull + 16, barAFull = barRawFull + 32, barAEmpty = barRawFull + 64;
     const uint32_t barAccFull = barRawFull + 96, barAccEmpty = barRawFull + 128;      // + 16 * stage + 8 * half
-    // SPLIT kernels with p.halves set: TWO CTAs per tile, each with the products of one column half; the half's models are dealt
-    // to all four recursion warp groups (at most two models per thread, V3Params::h*)
-    const int half = (SPLIT && p.halves) ? (int)(blockIdx.x & 1u) : -1;
+    const int half = HALF ? (int)(blockIdx.x & 1u) : 0;
 
     {
         const uint4 *src = reinterpret_cast<const uint4 *>(p.wimg);
@@ -437,7 +434,7 @@ __global__ void __launch_bounds__(V4_THREADS, 1) k_viterbi_v4(const V3Params p, 
     if (tid == 0) {
         for (int s = 0; s < 2; s++) { mbar_init(barRawFull + 8 * s, 1); mbar_init(barRawEmpty + 8 * s, V4_CONV_WARPS); }
         for (int s = 0; s < 4; s++) { mbar_init(barAFull + 8 * s, V4_CONV_WARPS); mbar_init(barAEmpty + 8 * s, 1); }
-        for (int s = 0; s < 4; s++) { mbar_init(barAccFull + 8 * s, 1); mbar_init(barAccEmpty + 8 * s, half >= 0 ? 4 * p.hroles[half] : SPLIT ? V4_REC_WARPS / 2 : V4_REC_WARPS); }
+        for (int s = 0; s < 4; s++) { mbar_init(barAccFull + 8 * s, 1); mbar_init(barAccEmpty + 8 * s, HALF ? 4 * p.hroles[half] : V4_REC_WARPS); }
         fence_barrier_init();
     }
     constexpr uint32_t a_cols = 8u * nck;
@@ -449,7 +446,7 @@ __global__ void __launch_bounds__(V4_THREADS, 1) k_viterbi_v4(const V3Params p, 
     const uint32_t tmem_base = *sTmem;
     const uint32_t tmem_acc = tmem_base, tmem_a = tmem_base + 2u * ncols;
     const int Tt = p.Tt, Tpad = p.Tpad;
-    const int cta = half >= 0 ? (int)(blockIdx.x >> 1) : (int)blockIdx.x, ncta = half >= 0 ? (int)(gridDim.x >> 1) : (int)gridDim.x;
+    const int cta = HALF ? (int)(blockIdx.x >> 1) : (int)blockIdx.x, ncta = HALF ? (int)(gridDim.x >> 1) : (int)gridDim.x;
     const int my_tiles = (p.ntiles - cta + ncta - 1) / ncta;
     const int nblk = my_tiles * (Tpad / V3_FB);          // four-frame blocks this CTA walks
     auto trace = [&](int role, int frame, int ev) {
@@ -462,7 +459,7 @@ __global__ void __launch_bounds__(V4_THREADS, 1) k_viterbi_v4(const V3Params p, 
             tma_prefetch_desc(&tmap);
             uint32_t G = 0;
             for (int tile = cta; tile < p.ntiles; tile += ncta) {
-                const int urow = (EXP && (p.flags & 16)) ? p.u0 + cta * TC_ROWS : p.u0 + tile * TC_ROWS;      // what-if 16: L2-resident features
+                const int urow = p.u0 + tile * TC_ROWS;
                 for (int t0 = 0; t0 < Tpad; t0 += V3_FB, G++) {
                     const uint32_t s = G & 1u, ph = (G >> 1) & 1u;
                     const uint32_t bar = barRawFull + 8 * s;
@@ -497,45 +494,35 @@ __global__ void __launch_bounds__(V4_THREADS, 1) k_viterbi_v4(const V3Params p, 
                     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns));
                     p.trace[((size_t)0 * V4_TRACE_FRAMES + 4 * b + i) * 4 + 1] = (long long)ns;
                 }
-                mbar_wait2(barAFull + 8 * i, aph, barAccEmpty + 16 * (i & 1) + (half == 1 ? 8 : 0), ((i >> 1) & 1) ^ 1);
+                mbar_wait2(barAFull + 8 * i, aph, barAccEmpty + 16 * (i & 1) + 8 * half, ((i >> 1) & 1) ^ 1);
                 trace(0, 4 * b + i, 2);
                 tc_fence_after();
                 const uint32_t d_tmem = tmem_acc + (uint32_t)(i & 1) * (uint32_t)ncols;
                 const uint32_t a_hi = tmem_a + (uint32_t)i * a_cols, a_lo = a_hi + 8u;
-                if (!SPLIT) {
+                if (!HALF) {
                     if (elect_one()) {
                         // the two correction products first: the large hi * W_hi partial sums see the fewest truncating steps
-                        if (!EXP || !(p.flags & 1)) {
 #pragma unroll
-                            for (int ks = 0; ks < NKS; ks++) umma_f16_ts(d_tmem, a_lo + ks * 16, dW_hi + (uint64_t)(16 * ks), idesc, ks > 0);
+                        for (int ks = 0; ks < NKS; ks++) umma_f16_ts(d_tmem, a_lo + ks * 16, dW_hi + (uint64_t)(16 * ks), idesc, ks > 0);
 #pragma unroll
-                            for (int ks = 0; ks < NKS; ks++) umma_f16_ts(d_tmem, a_hi + ks * 16, dW_lo + (uint64_t)(16 * ks), idesc, 1);
+                        for (int ks = 0; ks < NKS; ks++) umma_f16_ts(d_tmem, a_hi + ks * 16, dW_lo + (uint64_t)(16 * ks), idesc, 1);
 #pragma unroll
-                            for (int ks = 0; ks < NKS; ks++) umma_f16_ts(d_tmem, a_hi + ks * 16, dW_hi + (uint64_t)(16 * ks), idesc, 1);
-                        }
+                        for (int ks = 0; ks < NKS; ks++) umma_f16_ts(d_tmem, a_hi + ks * 16, dW_hi + (uint64_t)(16 * ks), idesc, 1);
                         umma_commit(barAccFull + 16 * (i & 1));
                         umma_commit(barAEmpty + 8 * i);
                     }
-                } else {
+                } else if (elect_one()) {
+                    const uint32_t dh = d_tmem + (half ? colA : 0u);
+                    const uint32_t idh = half ? idescB : idescA;
+                    const uint64_t wh = dW_hi + (half ? wofs : 0ull), wl = dW_lo + (half ? wofs : 0ull);
 #pragma unroll
-                    for (int h = 0; h < 2; h++) {
-                        if (half >= 0 && h != half) continue;
-                        if (h == 1 && half < 0) { mbar_wait(barAccEmpty + 16 * (i & 1) + 8, ((i >> 1) & 1) ^ 1); tc_fence_after(); }
-                        if (elect_one()) {
-                            const uint32_t dh = d_tmem + (h ? colA : 0u);
-                            const uint32_t idh = h ? idescB : idescA;
-                            const uint64_t wh = dW_hi + (h ? wofs : 0ull), wl = dW_lo + (h ? wofs : 0ull);
+                    for (int ks = 0; ks < NKS; ks++) umma_f16_ts(dh, a_lo + ks * 16, wh + (uint64_t)(16 * ks), idh, ks > 0);
 #pragma unroll
-                            for (int ks = 0; ks < NKS; ks++) umma_f16_ts(dh, a_lo + ks * 16, wh + (uint64_t)(16 * ks), idh, ks > 0);
+                    for (int ks = 0; ks < NKS; ks++) umma_f16_ts(dh, a_hi + ks * 16, wl + (uint64_t)(16 * ks), idh, 1);
 #pragma unroll
-                            for (int ks = 0; ks < NKS; ks++) umma_f16_ts(dh, a_hi + ks * 16, wl + (uint64_t)(16 * ks), idh, 1);
-#pragma unroll
-                            for (int ks = 0; ks < NKS; ks++) umma_f16_ts(dh, a_hi + ks * 16, wh + (uint64_t)(16 * ks), idh, 1);
-                            umma_commit(barAccFull + 16 * (i & 1) + 8 * h);
-                            if (h == 1 || half == 0) umma_commit(barAEmpty + 8 * i);
-                        }
-                        __syncwarp();
-                    }
+                    for (int ks = 0; ks < NKS; ks++) umma_f16_ts(dh, a_hi + ks * 16, wh + (uint64_t)(16 * ks), idh, 1);
+                    umma_commit(barAccFull + 16 * (i & 1) + 8 * half);
+                    umma_commit(barAEmpty + 8 * i);
                 }
                 __syncwarp();
                 trace(0, 4 * b + i, 3);
@@ -572,11 +559,7 @@ __global__ void __launch_bounds__(V4_THREADS, 1) k_viterbi_v4(const V3Params p, 
 #pragma unroll
                 for (int c = 0; c < NKS; c++) {
                     uint32_t hi[4], lo[4];
-                    if (EXP && (p.flags & 4)) {
-                        hi[0] = __float_as_uint(x[c].x); hi[1] = __float_as_uint(x[c].y); hi[2] = __float_as_uint(x[c].z); hi[3] = __float_as_uint(x[c].w);
-                        lo[0] = lo[1] = lo[2] = lo[3] = 0u;
-                    } else
-                        v3_split4(x[c], v3_lds4(sbS + 16u * c), v3_lds4(sbB + 16u * c), hi, lo);
+                    v3_split4(x[c], v3_lds4(sbS + 16u * c), v3_lds4(sbB + 16u * c), hi, lo);
                     const uint32_t cg = c0 + (uint32_t)c;
                     const uint32_t tc = ta + 16u * (cg >> 1) + 4u * (cg & 1u);      // chunk cg: 4 columns of the hi half, 4 of the lo half of its K step
                     tmem_st4(tc, hi[0], hi[1], hi[2], hi[3]);
@@ -596,11 +579,11 @@ __global__ void __launch_bounds__(V4_THREADS, 1) k_viterbi_v4(const V3Params p, 
         // ===================== recursion: thread = (row, model group) =====================
         asm volatile("setmaxnreg.inc.sync.aligned.u32 80;");
         const int rwp = warp - V4_REC_WARP0, q = rwp & 3, g = rwp >> 2, r = q * 32 + lane;
-        const int mbeg = half >= 0 ? p.hmod0[half][g] : p.mod0[g];
+        const int mbeg = HALF ? p.hmod0[half][g] : p.mod0[g];
         const uint32_t acc0 = pin_reg(tmem_acc + ((uint32_t)(q * 32) << 16) + (uint32_t)mbeg * 8u);
         const uint32_t acc1 = pin_reg(acc0 + (uint32_t)ncols);
         const uint32_t lane0 = pin_reg(lane == 0 ? 1u : 0u);
-        const uint32_t hb = SPLIT ? 8u * (uint32_t)(half >= 0 ? half : (g >> 1)) : 0u;      // this group's column half
+        const uint32_t hb = 8u * (uint32_t)half;            // this CTA's column half
         const uint32_t bFull = pin_reg(barAccFull + hb), bEmpty = pin_reg(barAccEmpty + hb);
         const uint32_t bstride = pin_reg(p.Bpad);
         uint32_t *const bpp = p.bp;
@@ -636,10 +619,10 @@ __global__ void __launch_bounds__(V4_THREADS, 1) k_viterbi_v4(const V3Params p, 
                 }
                 // decision words: plane = the model group of the one-CTA layout; a column-half CTA's thread owns one or two of
                 // the word's bytes (same layout, narrower stores), so the arg-max / back-trace kernel does not change
-                uint32_t bpo = (uint32_t)(half >= 0 ? p.hplane[half][g] : g) * (uint32_t)Tpad * p.Bpad + (uint32_t)ul;
-                const uint32_t bsh = half >= 0 ? (uint32_t)p.hshift[half][g] : 0u;
+                uint32_t bpo = (uint32_t)(HALF ? p.hplane[half][g] : g) * (uint32_t)Tpad * p.Bpad + (uint32_t)ul;
+                const uint32_t bsh = HALF ? (uint32_t)p.hshift[half][g] : 0u;
                 auto store_bp = [&](uint32_t v) {
-                    if (SPLIT && half >= 0 && MC < 3) {
+                    if (HALF && MC < 3) {
                         uint8_t *b = reinterpret_cast<uint8_t *>(bpp + bpo) + bsh;
                         if (MC == 2) *reinterpret_cast<uint16_t *>(b) = (uint16_t)v;
                         else *b = (uint8_t)v;
@@ -664,23 +647,18 @@ __global__ void __launch_bounds__(V4_THREADS, 1) k_viterbi_v4(const V3Params p, 
                     if (TRACE && trole >= 0) trace(trole, fbase + t0 + I, 1);
                     const int t = t0 + I;
                     if (!GEN) {
-                        if (EXP && (p.flags & 2)) {
+                        // one sign-bit chain per model (independent instruction streams), merged bytewise
+                        uint32_t sbk[MC];
 #pragma unroll
-                            for (int k = 0; k < MC; k++) { sb += ev[k][0]; tmem_ld8(nacc + 8u * k, ev[k]); }
-                        } else {
-                            // one sign-bit chain per model (independent instruction streams), merged bytewise
-                            uint32_t sbk[MC];
-#pragma unroll
-                            for (int k = 0; k < MC; k++) {
-                                sbk[k] = 0;
-                                v3_step(W[k], Wx[k], aex[k], ev[k], sbk[k]);
-                                tmem_ld8(nacc + 8u * k, ev[k]);
-                            }
-                            sb = sbk[0];
-                            if (MC == 2) sb = __byte_perm(sbk[0], sbk[1], 0x3340);
-                            if (MC == 3) sb = __byte_perm(__byte_perm(sbk[0], sbk[1], 0x3340), sbk[2], 0x3410);
+                        for (int k = 0; k < MC; k++) {
+                            sbk[k] = 0;
+                            v3_step(W[k], Wx[k], aex[k], ev[k], sbk[k]);
+                            tmem_ld8(nacc + 8u * k, ev[k]);
                         }
-                        if (!EXP || !(p.flags & 8)) store_bp(sb);
+                        sb = sbk[0];
+                        if (MC == 2) sb = __byte_perm(sbk[0], sbk[1], 0x3340);
+                        if (MC == 3) sb = __byte_perm(__byte_perm(sbk[0], sbk[1], 0x3340), sbk[2], 0x3410);
+                        store_bp(sb);
                     } else {
                         if (t < Tt) {
                             if (t == 0) {
@@ -739,303 +717,9 @@ __global__ void __launch_bounds__(V4_THREADS, 1) k_viterbi_v4(const V3Params p, 
                 }
             }
         };
-        const int mcnt = half >= 0 ? p.hnmod[half][g] : p.nmod[g];
-        if (mcnt == 0 && half >= 0) { }
+        const int mcnt = HALF ? p.hnmod[half][g] : p.nmod[g];
+        if (HALF && mcnt == 0) { }
         else if (mcnt == 3) run(std::integral_constant<int, 3>{});
-        else if (mcnt == 2) run(std::integral_constant<int, 2>{});
-        else if (mcnt == 1) run(std::integral_constant<int, 1>{});
-        else __trap();
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == V4_MMA_WARP) tmem_dealloc(tmem_base, 512);
-}
-
-// ------------------------------------------------------------------------------------------------
-// k_viterbi_v5: k_viterbi_v4 with the TMEM budget moved from the A operand to the accumulators: THREE accumulator stages and
-// TWO A stages (3 x 96 + 2 x 80 = 448 columns).  In v4 the MMA issuer and the recursion warps wait on each other through a
-// two-deep accumulator ring (the hand-back of a stage and the next-but-one frame's product are one round trip apart); the
-// conversions, which ran four stages ahead, keep two.  MEASURED SLOWER than v4 (0.98 vs 0.85 ms per 94 720 utterances: the
-// low-priority conversion warps need the depth of the A ring more than the recursion needs a third accumulator), kept behind
-// SAPR_VK=5 as the record of that experiment.  Frames go in blocks of SIX (stage indices
-// i & 1 and i % 3 stay compile-time constants), tiles are padded to a multiple of six frames, the raw ring is four stages of
-// two frames (run-time index), renormalisation once per block.
-#define V5_FB 6
-#define V5_RAW_STAGES 4
-#define V5_RAW_FRAMES 2
-
-struct V5Smem { uint32_t w, raw, tr, sb, bar, total; };
-__host__ __device__ inline V5Smem v5_smem_layout(int M, int nck, int ncols, uint32_t rw) {
-    V5Smem L;
-    L.w = 0;
-    L.raw = ((uint32_t)2 * (ncols / 8) * nck * 128 + 127u) & ~127u;
-    L.tr = L.raw + (uint32_t)V5_RAW_STAGES * V5_RAW_FRAMES * TC_ROWS * rw;
-    L.sb = L.tr + (uint32_t)M * TC_TRQ * 16;
-    L.bar = (L.sb + (uint32_t)8 * nck * 4 + 15u) & ~15u;
-    L.total = L.bar + 18 * 8 + 16;      // raw_full[4], raw_empty[4], A_full[2], A_empty[2], acc_full[3], acc_empty[3]
-    return L;
-}
-
-template <int NKS>
-__global__ void __launch_bounds__(V4_THREADS, 1) k_viterbi_v5(const V3Params p, const __grid_constant__ CUtensorMap tmap) {
-    extern __shared__ __align__(128) unsigned char smem[];
-    constexpr int nck = 2 * NKS;
-    const int ncols = p.ncols, M = p.M;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const uint32_t rw = p.rw, frame_bytes = TC_ROWS * rw, stage_bytes = V5_RAW_FRAMES * frame_bytes;
-    const V5Smem L = v5_smem_layout(M, nck, ncols, rw);
-    const uint32_t w_plane = (uint32_t)(ncols / 8) * nck * 128;
-    unsigned char *sW = smem + L.w;
-    const uint32_t sRaw = smem_u32(smem + L.raw);
-    const float4 *sTr = reinterpret_cast<const float4 *>(smem + L.tr);
-    uint64_t *sBar = reinterpret_cast<uint64_t *>(smem + L.bar);
-    uint32_t *sTmem = reinterpret_cast<uint32_t *>(sBar + 18);
-    const uint32_t barRawFull = smem_u32(sBar), barRawEmpty = barRawFull + 32, barAFull = barRawFull + 64, barAEmpty = barRawFull + 80;
-    const uint32_t barAccFull = barRawFull + 96, barAccEmpty = barRawFull + 120;
-
-    {
-        const uint4 *src = reinterpret_cast<const uint4 *>(p.wimg);
-        uint4 *dst = reinterpret_cast<uint4 *>(sW);
-        for (uint32_t i = tid; i < 2 * w_plane / 16; i += V4_THREADS) dst[i] = src[i];
-        float4 *dtr = reinterpret_cast<float4 *>(smem + L.tr);
-        for (int i = tid; i < M * TC_TRQ; i += V4_THREADS) dtr[i] = p.trp[i];
-        float *dsb = reinterpret_cast<float *>(smem + L.sb);
-        for (int i = tid; i < 8 * nck; i += V4_THREADS) dsb[i] = p.sb[i];
-    }
-    if (tid == 0) {
-        for (int s = 0; s < V5_RAW_STAGES; s++) { mbar_init(barRawFull + 8 * s, 1); mbar_init(barRawEmpty + 8 * s, V4_CONV_WARPS); }
-        for (int s = 0; s < 2; s++) { mbar_init(barAFull + 8 * s, V4_CONV_WARPS); mbar_init(barAEmpty + 8 * s, 1); }
-        for (int s = 0; s < 3; s++) { mbar_init(barAccFull + 8 * s, 1); mbar_init(barAccEmpty + 8 * s, V4_REC_WARPS); }
-        fence_barrier_init();
-    }
-    constexpr uint32_t a_cols = 8u * nck;
-    if (warp == V4_MMA_WARP) tmem_alloc(smem_u32(sTmem), 512);
-    fence_proxy_async();
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *sTmem;
-    const uint32_t tmem_acc = tmem_base, tmem_a = tmem_base + 3u * ncols;
-    const int Tt = p.Tt, Tpad = p.Tpad;
-    const int my_tiles = (p.ntiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
-    const int nblk = my_tiles * (Tpad / V5_FB);          // six-frame blocks this CTA walks
-
-    if (warp == V4_TMA_WARP) {
-        // ===================== TMA producer: one ring stage = two frames of a tile =====================
-        if (lane == 0) {
-            tma_prefetch_desc(&tmap);
-            uint32_t G = 0;
-            for (int tile = blockIdx.x; tile < p.ntiles; tile += gridDim.x) {
-                const int urow = p.u0 + tile * TC_ROWS;
-                for (int t0 = 0; t0 < Tpad; t0 += V5_RAW_FRAMES, G++) {
-                    const uint32_t s = G & (V5_RAW_STAGES - 1), ph = (G / V5_RAW_STAGES) & 1u;
-                    const uint32_t bar = barRawFull + 8 * s;
-                    mbar_wait(barRawEmpty + 8 * s, ph ^ 1u);
-                    mbar_arrive_tx(bar, stage_bytes);
-                    const uint32_t dst = sRaw + s * stage_bytes;
-#pragma unroll
-                    for (int fi = 0; fi < V5_RAW_FRAMES; fi++) tma_load_3d(dst + (uint32_t)fi * frame_bytes, &tmap, 0, t0 + fi, urow, bar);
-                }
-            }
-        }
-    } else if (warp == V4_MMA_WARP) {
-        // ===================== MMA issuer =====================
-        const uint32_t idesc = (1u << 4) | ((uint32_t)(ncols >> 3) << 17) | ((uint32_t)(TC_ROWS >> 4) << 24);
-        const uint32_t sW_hi = smem_u32(sW), sW_lo = sW_hi + w_plane;
-        const uint32_t sboW = (uint32_t)nck * 128u;
-        const uint64_t dW_hi = make_desc(sW_hi, 128, sboW), dW_lo = make_desc(sW_lo, 128, sboW);
-        uint32_t bph = 0;                                 // block parity: an A stage is used three times per block
-        for (int b = 0; b < nblk; b++, bph ^= 1u) {
-#pragma unroll
-            for (int i = 0; i < V5_FB; i++) {
-                // A stage i & 1: use 3 b + i / 2 of that stage; accumulator stage i % 3: use 2 b + i / 3
-                mbar_wait2(barAFull + 8 * (i & 1), bph ^ (uint32_t)((i >> 1) & 1), barAccEmpty + 8 * (i % 3), (uint32_t)(((i / 3) & 1) ^ 1));
-                tc_fence_after();
-                if (elect_one()) {
-                    const uint32_t d_tmem = tmem_acc + (uint32_t)(i % 3) * (uint32_t)ncols;
-                    const uint32_t a_hi = tmem_a + (uint32_t)(i & 1) * a_cols, a_lo = a_hi + 8u;
-#pragma unroll
-                    for (int ks = 0; ks < NKS; ks++) umma_f16_ts(d_tmem, a_lo + ks * 16, dW_hi + (uint64_t)(16 * ks), idesc, ks > 0);
-#pragma unroll
-                    for (int ks = 0; ks < NKS; ks++) umma_f16_ts(d_tmem, a_hi + ks * 16, dW_lo + (uint64_t)(16 * ks), idesc, 1);
-#pragma unroll
-                    for (int ks = 0; ks < NKS; ks++) umma_f16_ts(d_tmem, a_hi + ks * 16, dW_hi + (uint64_t)(16 * ks), idesc, 1);
-                    umma_commit(barAccFull + 8 * (i % 3));
-                    umma_commit(barAEmpty + 8 * (i & 1));
-                }
-                __syncwarp();
-            }
-        }
-    } else if (warp < V4_REC_WARP0) {
-        // ===================== conversion: thread = (row, chunk half) =====================
-        asm volatile("setmaxnreg.dec.sync.aligned.u32 56;");
-        const int cw = warp, q = cw & 3, h = cw >> 2, r = q * 32 + lane;
-        const uint32_t c0 = (uint32_t)(h * NKS);
-        const uint32_t raw0 = pin_reg(sRaw + (uint32_t)r * rw + 16u * c0);
-        const uint32_t ta0 = pin_reg(tmem_a + ((uint32_t)(q * 32) << 16));
-        const uint32_t sbS = pin_reg(smem_u32(smem + L.sb) + 16u * c0), sbB = sbS + 16u * nck;
-        const uint32_t lane0 = pin_reg(lane == 0 ? 1u : 0u);
-        const uint32_t sbytes = pin_reg(stage_bytes), fbytes = pin_reg(frame_bytes);
-        uint32_t G = 0, bph = 0;
-        for (int b = 0; b < nblk; b++, bph ^= 1u) {
-#pragma unroll
-            for (int fi = 0; fi < V5_FB; fi++) {
-                const uint32_t s = G & (V5_RAW_STAGES - 1);
-                if ((fi & 1) == 0) mbar_wait(barRawFull + 8 * s, (G / V5_RAW_STAGES) & 1u);
-                const uint32_t src = raw0 + s * sbytes + (uint32_t)(fi & 1) * fbytes;
-                float4 x[NKS];
-#pragma unroll
-                for (int c = 0; c < NKS; c++) x[c] = v3_lds4(src + 16u * c);
-                mbar_wait(barAEmpty + 8 * (fi & 1), bph ^ (uint32_t)((fi >> 1) & 1) ^ 1u);
-                tc_fence_after();
-                const uint32_t ta = ta0 + (uint32_t)(fi & 1) * a_cols;
-#pragma unroll
-                for (int c = 0; c < NKS; c++) {
-                    uint32_t hi[4], lo[4];
-                    v3_split4(x[c], v3_lds4(sbS + 16u * c), v3_lds4(sbB + 16u * c), hi, lo);
-                    const uint32_t cg = c0 + (uint32_t)c;
-                    const uint32_t tc = ta + 16u * (cg >> 1) + 4u * (cg & 1u);
-                    tmem_st4(tc, hi[0], hi[1], hi[2], hi[3]);
-                    tmem_st4(tc + 8u, lo[0], lo[1], lo[2], lo[3]);
-                }
-                tmem_st_wait();
-                tc_fence_before();
-                __syncwarp();
-                if (lane0) {
-                    mbar_arrive(barAFull + 8 * (fi & 1));
-                    if (fi & 1) mbar_arrive(barRawEmpty + 8 * s);
-                }
-                if (fi & 1) G++;
-            }
-        }
-    } else {
-        // ===================== recursion: thread = (row, model group) =====================
-        asm volatile("setmaxnreg.inc.sync.aligned.u32 80;");
-        const int rwp = warp - V4_REC_WARP0, q = rwp & 3, g = rwp >> 2, r = q * 32 + lane;
-        const int mbeg = p.mod0[g];
-        const uint32_t acc0 = pin_reg(tmem_acc + ((uint32_t)(q * 32) << 16) + (uint32_t)mbeg * 8u);
-        const uint32_t acc1 = pin_reg(acc0 + (uint32_t)ncols), acc2 = pin_reg(acc0 + 2u * (uint32_t)ncols);
-        const uint32_t lane0 = pin_reg(lane == 0 ? 1u : 0u);
-        const uint32_t bstride = pin_reg(p.Bpad);
-        uint32_t *const bpp = p.bp;
-        auto run = [&](auto MCc) {
-            constexpr int MC = decltype(MCc)::value;
-            // the exit self-loop constants are re-read from shared memory at each use and the renormalisation offsets live in shared
-            // memory (touched once per block): the state, the rolling fetch and the sign-bit chains fill the 80 registers
-            const uint32_t aexS = pin_reg(smem_u32(sTr) + (uint32_t)(mbeg * TC_TRQ + 2) * 16u);
-            float *const baseS = reinterpret_cast<float *>(smem + L.total) + (warp - V4_REC_WARP0) * 32 * 3 + lane;
-            auto aex = [&](int k) -> float {
-                float v;
-                asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(aexS + (uint32_t)k * (TC_TRQ * 16u)));
-                return v;
-            };
-            uint32_t ev[MC][8];                     // rolling accumulator fetch, as in k_viterbi_v4
-            if (my_tiles > 0) {
-                mbar_wait(barAccFull, 0);
-                tc_fence_after();
-#pragma unroll
-                for (int k = 0; k < MC; k++) tmem_ld8(acc0 + 8u * k, ev[k]);
-                tmem_ld_wait();
-                tc_fence_before();
-                __syncwarp();
-                if (lane0) mbar_arrive(barAccEmpty);
-            }
-            int tiles_left = my_tiles;
-            for (int tile = blockIdx.x; tile < p.ntiles; tile += gridDim.x) {
-                tiles_left--;
-                const int ul = tile * TC_ROWS + r;
-                float W[MC][8], Wx[MC];
-#pragma unroll
-                for (int k = 0; k < MC; k++) {
-                    Wx[k] = -INFINITY; baseS[k * 32] = 0.f;
-#pragma unroll
-                    for (int j = 0; j < 8; j++) W[k][j] = -INFINITY;
-                }
-                uint32_t bpo = (uint32_t)g * (uint32_t)Tpad * p.Bpad + (uint32_t)ul;
-                uint32_t sb = 0;
-                // frame t0 + I: its columns are in ev; frame t0 + I + 1 (stage (I + 1) % 3, phase ((I + 1) / 3) & 1 -- tiles start at
-                // a multiple of six frames) is fetched behind it unless this is the CTA's last frame
-                auto recurse = [&](auto Ic, auto GENc, int t0, bool more) {
-                    constexpr int I = decltype(Ic)::value;
-                    constexpr bool GEN = decltype(GENc)::value;
-                    constexpr int NS = (I + 1) % 3;
-                    const uint32_t nacc = NS == 0 ? acc0 : NS == 1 ? acc1 : acc2;
-                    if (!GEN || more) {
-                        mbar_wait(barAccFull + 8 * NS, ((I + 1) / 3) & 1);
-                        tc_fence_after();
-                    }
-                    const int t = t0 + I;
-                    if (!GEN) {
-                        uint32_t sbk[MC];
-#pragma unroll
-                        for (int k = 0; k < MC; k++) {
-                            sbk[k] = 0;
-                            v3_step(W[k], Wx[k], aex(k), ev[k], sbk[k]);
-                            tmem_ld8(nacc + 8u * k, ev[k]);
-                        }
-                        sb = sbk[0];
-                        if (MC == 2) sb = __byte_perm(sbk[0], sbk[1], 0x3340);
-                        if (MC == 3) sb = __byte_perm(__byte_perm(sbk[0], sbk[1], 0x3340), sbk[2], 0x3410);
-                        bpp[bpo] = sb;
-                    } else {
-                        if (t < Tt) {
-                            if (t == 0) {
-#pragma unroll
-                                for (int k = 0; k < MC; k++) W[k][0] = sTr[(mbeg + k) * TC_TRQ + 2].y + __uint_as_float(ev[k][0]);
-                            } else if (t == 1) {
-#pragma unroll
-                                for (int k = MC - 1; k >= 0; k--) v3_step_entry(W[k], Wx[k], sTr[(mbeg + k) * TC_TRQ + 2].y, ev[k], sb);
-                            } else {
-#pragma unroll
-                                for (int k = MC - 1; k >= 0; k--) v3_step(W[k], Wx[k], aex(k), ev[k], sb);
-                            }
-                            bpp[bpo] = sb;
-                        }
-                        if (more) {
-#pragma unroll
-                            for (int k = 0; k < MC; k++) tmem_ld8(nacc + 8u * k, ev[k]);
-                        }
-                    }
-                    bpo += bstride;
-                    if (!GEN || more) {
-                        tmem_ld_wait();
-                        tc_fence_before();
-                        __syncwarp();
-                        if (lane0) mbar_arrive(barAccEmpty + 8 * NS);
-                    }
-                };
-                constexpr std::integral_constant<bool, false> LEAN{};
-                constexpr std::integral_constant<bool, true> GENERIC{};
-                for (int t0 = 0; t0 < Tpad; t0 += V5_FB) {
-                    if (t0 != 0 && t0 + V5_FB < Tpad) {
-                        recurse(std::integral_constant<int, 0>{}, LEAN, t0, true); recurse(std::integral_constant<int, 1>{}, LEAN, t0, true);
-                        recurse(std::integral_constant<int, 2>{}, LEAN, t0, true); recurse(std::integral_constant<int, 3>{}, LEAN, t0, true);
-                        recurse(std::integral_constant<int, 4>{}, LEAN, t0, true); recurse(std::integral_constant<int, 5>{}, LEAN, t0, true);
-                    } else {
-                        const bool more = t0 + V5_FB < Tpad || tiles_left > 0;
-                        recurse(std::integral_constant<int, 0>{}, GENERIC, t0, true); recurse(std::integral_constant<int, 1>{}, GENERIC, t0, true);
-                        recurse(std::integral_constant<int, 2>{}, GENERIC, t0, true); recurse(std::integral_constant<int, 3>{}, GENERIC, t0, true);
-                        recurse(std::integral_constant<int, 4>{}, GENERIC, t0, true); recurse(std::integral_constant<int, 5>{}, GENERIC, t0, more);
-                    }
-#pragma unroll
-                    for (int k = 0; k < MC; k++) {
-                        float bk = baseS[k * 32];
-                        v3_renorm(W[k], Wx[k], bk);
-                        baseS[k * 32] = bk;
-                    }
-                }
-                if (ul < p.nu) {
-#pragma unroll
-                    for (int k = 0; k < MC; k++) {
-                        const float4 cm = sTr[(mbeg + k) * TC_TRQ + 2];
-                        const double sc = (Wx[k] > -INFINITY) ? ((double)Wx[k] + (double)baseS[k * 32]) + ((double)cm.z + (double)cm.w) : -INFINITY;
-                        p.scores[(size_t)ul * M + mbeg + k] = sc;
-                    }
-                }
-            }
-        };
-        const int mcnt = p.nmod[g];
-        if (mcnt == 3) run(std::integral_constant<int, 3>{});
         else if (mcnt == 2) run(std::integral_constant<int, 2>{});
         else if (mcnt == 1) run(std::integral_constant<int, 1>{});
         else __trap();
@@ -1156,9 +840,7 @@ int sapr_viterbi_v3_launch(sapr_ctx *ctx, sapr_models *m, const float *X, int ld
     const int Tt = (first_frames > 0 && first_frames < max_T) ? first_frames : max_T;
     if (Tt < 2 || ((uintptr_t)X & 15u) || nck % 2) return SAPR_OK;
     V3Params prm;
-    const char *vk_env = getenv("SAPR_VK");
-    const bool use_v4 = !(vk_env && vk_env[0] == '3') && (nck == 10 || nck == 4) && M >= TC_GROUPS;
-    const bool use_v5 = use_v4 && vk_env && vk_env[0] == '5';          // measured variant, not the default: three accumulator + two A stages (k_viterbi_v5)
+    const bool use_v4 = (nck == 10 || nck == 4) && M >= TC_GROUPS;
     const int npairs = nck / 2;
     if (use_v4) {      // models over the four recursion groups, as evenly as they go
         int ma = 0;
@@ -1191,10 +873,8 @@ int sapr_viterbi_v3_launch(sapr_ctx *ctx, sapr_models *m, const float *X, int ld
     const uint32_t rw = (uint32_t)(nck + 1) * 16u;
     V3Smem L = v3_smem_layout(M, nck, ncols, rw);
     if (use_v4) L.total = v4_smem_layout(M, nck, ncols, rw).total;
-    if (use_v5) L.total = v5_smem_layout(M, nck, ncols, rw).total + V4_REC_WARPS * 32 * 3 * (uint32_t)sizeof(float);
-    if (L.total > 227 * 1024 || (use_v5 ? 3 * ncols + 2 * 8 * nck : 2 * ncols + 4 * 8 * nck) > 512) return SAPR_OK;
-    const int fb = use_v5 ? V5_FB : V3_FB;
-    const int Tpad = (Tt + fb - 1) / fb * fb;
+    if (L.total > 227 * 1024 || 2 * ncols + 4 * 8 * nck > 512) return SAPR_OK;
+    const int Tpad = (Tt + V3_FB - 1) / V3_FB * V3_FB;
     const int64_t per_utt = (int64_t)TC_GROUPS * Tpad * sizeof(uint32_t);
     int chunk = (int)std::min<int64_t>(B, std::max<int64_t>(TC_ROWS, ((int64_t)1024 << 20) / per_utt));
     if (const char *ce = getenv("SAPR_V_CHUNK")) chunk = std::max(1, std::min(chunk, atoi(ce)));     // tests: force the multi-chunk path
@@ -1215,26 +895,14 @@ int sapr_viterbi_v3_launch(sapr_ctx *ctx, sapr_models *m, const float *X, int ld
     V3Map map;
     for (int g = 0; g < TC_GROUPS; g++)
         for (int k = 0; k < prm.nmod[g]; k++) { map.grp[prm.mod0[g] + k] = g; map.shift[prm.mod0[g] + k] = 8 * k; }
-    const int exp_flags = getenv("SAPR_V_EXP") ? atoi(getenv("SAPR_V_EXP")) : 0;
-    // SAPR_V_SPLIT=1: column-half products (model groups 0-1 | 2-3 split the accumulator at a multiple of 16 columns).  MEASURED SLOWER
-    // (0.93 vs 0.84 ms per 94 720 utterances) although an N = 48 product costs half an N = 96 one (24 vs 48 cycles,
-    // tools/ubench/umma_contend.cu); kept as the record of that experiment
-    prm.split_col = 8 * prm.mod0[2];
-    const char *sp_env = getenv("SAPR_V_SPLIT");
-    const bool split = use_v4 && !use_v5 && !exp_flags && (sp_env && sp_env[0] == '1') && prm.split_col >= 16 && prm.split_col % 16 == 0 &&
-                       ncols - prm.split_col >= 16 && (ncols - prm.split_col) % 16 == 0;
-    auto kern = use_v5 ? (nck == 10 ? k_viterbi_v5<5> : k_viterbi_v5<2>)
-                : use_v4 ? (nck == 10 ? (exp_flags ? k_viterbi_v4<5, false, true> : split ? k_viterbi_v4<5, false, false, true> : k_viterbi_v4<5>)
-                                      : (split ? k_viterbi_v4<2, false, false, true> : k_viterbi_v4<2>))
+    auto kern = use_v4 ? (nck == 10 ? k_viterbi_v4<5> : k_viterbi_v4<2>)
                        : (nck == 10) ? k_viterbi_v3<5> : (nck == 4) ? k_viterbi_v3<2> : k_viterbi_v3<0>;
     const int nthreads = use_v4 ? V4_THREADS : V3_THREADS;
-    // SAPR_V_HALF=0: the partial round as ordinary one-CTA tiles
-    const char *hf_env = getenv("SAPR_V_HALF");
-    const bool can_half = use_v4 && !use_v5 && !exp_flags && (!hf_env || hf_env[0] != '0') && prm.split_col >= 16 && prm.split_col % 16 == 0 &&
-                          ncols - prm.split_col >= 16 && (ncols - prm.split_col) % 16 == 0;
-    auto kern_half = !can_half ? nullptr : nck == 10 ? k_viterbi_v4<5, false, false, true> : k_viterbi_v4<2, false, false, true>;
+    // column halves for the partial round: model groups 0-1 | 2-3 split the accumulator at a multiple of 16 columns
+    prm.split_col = 8 * prm.mod0[2];
+    const bool can_half = use_v4 && prm.split_col >= 16 && prm.split_col % 16 == 0 && ncols - prm.split_col >= 16 && (ncols - prm.split_col) % 16 == 0;
+    auto kern_half = !can_half ? nullptr : nck == 10 ? k_viterbi_v4<5, false, true> : k_viterbi_v4<2, false, true>;
     if (kern_half) SAPR_CUDA(ctx, cudaFuncSetAttribute(kern_half, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total));
-    prm.halves = 0;
     if (can_half) {
         // a half's two model groups (1-3 models each) are dealt to the four recursion warp groups of its CTA: 3 -> 2 + 1, 2 -> 1 + 1,
         // 1 -> 1 + idle; a warp group keeps the bytes its models have in the group's decision word
@@ -1268,16 +936,15 @@ int sapr_viterbi_v3_launch(sapr_ctx *ctx, sapr_models *m, const float *X, int ld
         prm.sb = (const float *)((const char *)m->tc_image + w);
         prm.trp = (const float4 *)((const char *)m->tc_image + w + gsz);
         prm.bp = (uint32_t *)ctx->ws[0]; prm.Bpad = (uint32_t)chunk; prm.scores = (double *)ctx->ws[1]; prm.rw = rw;
-        prm.flags = exp_flags;
         prm.trace = nullptr;
         const char *trace_path = getenv("SAPR_V_TRACE");
-        if (trace_path && use_v4 && !use_v5 && nck == 10 && u0 == 0) {      // tuning aid: one traced launch, stamps to a text file
+        if (trace_path && use_v4 && nck == 10 && u0 == 0) {      // tuning aid: one traced launch, stamps to a text file
             const size_t nrec = (size_t)V4_TRACE_ROLES * V4_TRACE_FRAMES * 4;
             long long *dtr = nullptr;
             SAPR_CUDA(ctx, cudaMalloc(&dtr, nrec * sizeof(long long)));
             SAPR_CUDA(ctx, cudaMemsetAsync(dtr, 0, nrec * sizeof(long long), ctx->stream));
             prm.trace = dtr;
-            auto tk = exp_flags ? k_viterbi_v4<5, true, true> : split ? k_viterbi_v4<5, true, false, true> : k_viterbi_v4<5, true, false>;
+            auto tk = k_viterbi_v4<5, true>;
             SAPR_CUDA(ctx, cudaFuncSetAttribute(tk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total));
             tk<<<std::min(prm.ntiles, ctx->sm_count), nthreads, L.total, ctx->stream>>>(prm, tmap);
             std::vector<long long> h(nrec);
@@ -1313,9 +980,7 @@ int sapr_viterbi_v3_launch(sapr_ctx *ctx, sapr_models *m, const float *X, int ld
                 if (kern_half && 2 * prm.ntiles <= ctx->sm_count) {
                     // the partial round leaves most SMs idle: two CTAs per tile, each with the products and the recursion warps of
                     // one column half (model groups 0-1 | 2-3); both convert the tile's features
-                    prm.halves = 1;
                     kern_half<<<2 * prm.ntiles, nthreads, L.total, ctx->stream>>>(prm, tmap);
-                    prm.halves = 0;
                 } else
                     kern<<<std::min(prm.ntiles, ctx->sm_count), nthreads, L.total, ctx->stream>>>(prm, tmap);
                 prm.u0 = u0; prm.bp = bp0; prm.scores = sc0;

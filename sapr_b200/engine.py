@@ -178,20 +178,6 @@ class WordModels:
                                            ptr(stats), ptr(loglik), ptr(gamma)))
         return stats, loglik, gamma
 
-    def estep_grouped(self, X, T, model_start):
-        """E-step for a batch stored grouped by word, equal-length and contiguous (``X`` float32 [B*T, ldx], utterances
-        ``model_start[m] .. model_start[m+1]-1`` belong to model m): the fused kernel of csrc/estep_grouped.cu (fp32)."""
-        torch = _torch()
-        ms = np.ascontiguousarray(model_start, dtype=np.int32)
-        assert len(ms) == self.M + 1
-        B = int(ms[-1])
-        assert X.dtype == torch.float32 and X.is_cuda and X.is_contiguous() and X.shape[0] == B * T
-        stats = torch.empty((self.M, self.stats_stride()), dtype=torch.float64, device=X.device)
-        loglik = torch.zeros(B, dtype=torch.float64, device=X.device)
-        self.ctx.check(self.lib.sapr_estep_grouped(self.ctx.h, self.h, ptr(X), int(X.shape[1]), int(T), B, ptr(ms), ptr(stats),
-                                                   ptr(loglik)))
-        return stats, loglik
-
     def mstep(self, stats, floor_var):
         fv = np.ascontiguousarray(np.broadcast_to(np.asarray(floor_var, dtype=np.float64), (self.M,)))
         self.ctx.check(self.lib.sapr_mstep(self.ctx.h, self.h, ptr(stats), ptr(fv)))
@@ -214,31 +200,6 @@ def group_by_model(labels):
     """order[B] (stable, utterances grouped by model) computed on device (torch: plumbing only)."""
     torch = _torch()
     return torch.sort(labels.to(torch.int64), stable=True).indices.to(torch.int32).contiguous()
-
-
-class GroupedBatch:
-    """An equal-length batch re-stored grouped by word model -- the layout the reference trains from (train.py:94
-    ``load_mfccs_by_word`` feeds each word's utterances to its own model).  Built once per fit (torch gather: plumbing);
-    every Baum-Welch iteration then runs the fused grouped E-step."""
-
-    def __init__(self, batch: PackedBatch, labels, M: int):
-        torch = _torch()
-        assert batch.min_T == batch.max_T, "GroupedBatch needs equal-length utterances"
-        self.T, self.B, self.D, self.ldx = batch.max_T, batch.B, batch.D, batch.ldx
-        lab = labels.to(torch.int64)
-        order = torch.sort(lab, stable=True).indices
-        identity = bool((order == torch.arange(self.B, device=order.device)).all().item())
-        self.order = order
-        self.X = batch.X if identity else batch.X.view(self.B, self.T * self.ldx)[order].contiguous().view(self.B * self.T, self.ldx)
-        self.labels = lab[order].to(torch.int32)
-        counts = torch.bincount(lab, minlength=M).cpu().numpy()
-        self.model_start = np.zeros(M + 1, dtype=np.int32)
-        self.model_start[1:] = np.cumsum(counts)
-
-    @staticmethod
-    def eligible(models: "WordModels", batch: PackedBatch, precision) -> bool:
-        return (precision == FP32 and models.emission == EMIT_DIAG and models.topology == TOPO_ENTRY_EXIT and models.N == 8
-                and models.M <= 12 and models.D <= 47 and batch.B > 0 and batch.min_T == batch.max_T and batch.max_T >= 16)
 
 
 def init_flat_start(batch: PackedBatch, N: int, var_floor_factor: float = 0.001, ctx=None, dist=None):
@@ -280,24 +241,14 @@ def train_words(models: WordModels, batch: PackedBatch, labels, n_iter: int, flo
     batched E-step over all utterances (each against its own word model), ONE all-reduce of the packed
     statistics when sharded, then the M-step replicated on every GPU.  Returns per-iteration per-model LL."""
     torch = _torch()
-    import os
-    grouped = None
-    # the fused grouped kernel (csrc/estep_grouped.cu) moves 30 % less DRAM traffic but is slower than the general path at every
-    # size measured (tools/train_bench.py: 0.32 vs 0.25 ms at 330 utterances, 4.6 vs 3.9 ms at 200 k): opt-in
-    if GroupedBatch.eligible(models, batch, precision) and os.environ.get("SAPR_GROUPED", "0") == "1":
-        grouped = GroupedBatch(batch, labels, models.M)       # once per fit: utterances re-stored grouped by word
-    elif order is None:
+    if order is None:
         order = group_by_model(labels)
     history = []
     prev = None
     for it in range(n_iter):
         ll_m = torch.zeros(models.M, dtype=torch.float64, device=batch.X.device)
-        if grouped is not None:
-            stats, loglik = models.estep_grouped(grouped.X, grouped.T, grouped.model_start)
-            ll_m.index_add_(0, grouped.labels.to(torch.int64), loglik)
-        else:
-            stats, loglik, _ = models.estep(batch, labels, order, precision)
-            ll_m.index_add_(0, labels.to(torch.int64), loglik)
+        stats, loglik, _ = models.estep(batch, labels, order, precision)
+        ll_m.index_add_(0, labels.to(torch.int64), loglik)
         if dist is not None:
             packed = torch.cat([stats.reshape(-1), ll_m])
             dist.allreduce_(packed)

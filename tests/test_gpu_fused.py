@@ -267,12 +267,14 @@ def test_moderate_batch_against_oracle(eng):
 
 
 @pytest.mark.parametrize("B,M,D,T,first", [(300, 11, 39, 37, 0), (129, 5, 13, 24, 0), (128, 11, 39, 9, 0), (77, 3, 20, 8, 0),
-                                           (260, 11, 13, 40, 13)])
+                                           (260, 11, 13, 40, 13), (300, 11, 30, 37, 0), (260, 8, 24, 24, 0)])
 def test_viterbi_equal_length_batch_tma_vs_oracle(eng, B, M, D, T, first, monkeypatch):
-    """Equal-length batches (the BASELINE cfg-2 shape) take the TMA tensor-map kernel k_viterbi_tma: words, scores and
-    paths against the CPU oracle (custom_hmm.py:462-514 x all models + decoder.py:42-47); batch sizes that are not a
-    multiple of the 128-utterance tile (zero-filled rows), T down to N (exit never reachable: -inf), first_frames (D3);
-    and the per-row bulk-copy kernel (SAPR_TMA=0) must agree with it on words and to 1e-6 on scores."""
+    """Equal-length batches (the BASELINE cfg-2 shape) take one of the TMA-fed kernels, chosen by shape: k_viterbi_v4 for
+    10 or 4 feature chunks (D 32-39, 8-15) and M >= 4; k_viterbi_v3 for 8 chunks (D 24-31) and 8 <= M <= 12 (the last two
+    shapes); k_viterbi_tma otherwise (M = 3).  Words, scores and paths against the CPU oracle (custom_hmm.py:462-514 x all
+    models + decoder.py:42-47); batch sizes that are not a multiple of the 128-utterance tile (zero-filled rows), T down to N
+    (exit never reachable: -inf), first_frames (D3); and the call with SAPR_TMA=0 (per-row bulk-copy kernel where k_viterbi_tma
+    ran) must agree with it on words and to 1e-6 on scores."""
     from sapr_b200 import synth
     feats, labels, mu, sd = synth.make_corpus(B, M, 8, D, T, T, seed=1000 + B + T)
     A, means, var = synth.truth_models(mu, sd, 0.9)
@@ -299,49 +301,6 @@ def test_viterbi_equal_length_batch_tma_vs_oracle(eng, B, M, D, T, first, monkey
     out0 = m.viterbi(batch, None, eng.FP32, first, want_scores=True, want_path=True)
     assert_close(out0["scores"].cpu().numpy(), got, 1e-6, what="scores (bulk-copy kernel vs tma kernel)")
     assert np.mean(out0["best_word"].cpu().numpy() == w) > 0.995
-
-
-@pytest.mark.parametrize("B,M,D,T", [(700, 11, 39, 40), (150, 3, 13, 24), (1300, 11, 39, 16), (260, 5, 20, 33)])
-def test_estep_grouped_fused_vs_oracle(eng, B, M, D, T):
-    """Fused grouped E-step (csrc/estep_grouped.cu: forward sweep, backward sweep with Gamma^T.[x, x^2, 1] on the tensor
-    cores) against the CPU oracle (custom_hmm.py:417-439 + :372-386 restated): log-likelihoods, occupancies, xi sums and
-    the feature sums; model groups that do not fill a 128-utterance tile, several tiles per model, an empty model."""
-    import torch
-    from sapr_b200 import synth
-    feats, labels, mu, sd = synth.make_corpus(B, M, 8, D, T, T, seed=500 + B)
-    labels = np.asarray(labels).copy()
-    if M == 5:
-        labels[labels == 2] = 3                                   # model 2 gets no utterance at all
-    A, means, var = synth.truth_models(mu, sd, 0.9)
-    # evaluate away from the generating parameters, like an early Baum-Welch iteration
-    rng = np.random.default_rng(B)
-    means = means + 0.3 * np.sqrt(var) * rng.standard_normal(means.shape)
-    m = eng.WordModels(M, 8, D)
-    m.set(means, var, A)
-    batch = eng.PackedBatch.from_features(feats)
-    lab = torch.as_tensor(labels.astype(np.int32), device="cuda")
-    gb = eng.GroupedBatch(batch, lab, M)
-    stats, ll = m.estep_grouped(gb.X, gb.T, gb.model_start)
-    order = gb.order.cpu().numpy()
-    X, offs = orc.pack([feats[i] for i in order])
-    ost, oll = orc.estep_batch(X, offs, labels[order], A, means, var)
-    assert_close(ll.cpu().numpy(), oll, 1e-6, what="loglik")
-    st = stats.cpu().numpy()
-    S = 10
-    # G, Xi, occ: sums of posteriors over up to B*T/M frames
-    d3 = np.abs(st[:, :3 * S] - ost[:, :3 * S])
-    assert np.max(d3) < 3e-5 * T * max(1, B // M), ("occupancies", [float(d3[:, k * S:(k + 1) * S].max()) for k in range(3)],
-                                                    np.unravel_index(np.argmax(d3), d3.shape), st[:, :3 * S][d3 > 0.5], ost[:, :3 * S][d3 > 0.5])
-    occ = np.maximum(ost[:, 2 * S:3 * S], 1.0)                    # (M, S)
-    s1 = st[:, 3 * S:3 * S + S * D].reshape(M, S, D); o1 = ost[:, 3 * S:3 * S + S * D].reshape(M, S, D)
-    s2 = st[:, 3 * S + S * D:].reshape(M, S, D); o2 = ost[:, 3 * S + S * D:].reshape(M, S, D)
-    sig = np.sqrt(var)
-    # per-frame mean shift rel. to sigma <= 1e-4, second moment rel. to sigma^2 <= 1e-3 (the M-step tolerances)
-    assert np.max(np.abs(s1 - o1) / (occ[:, :, None] * sig)) < 1e-4, np.max(np.abs(s1 - o1) / (occ[:, :, None] * sig))
-    assert np.max(np.abs(s2 - o2) / (occ[:, :, None] * var)) < 1e-3, np.max(np.abs(s2 - o2) / (occ[:, :, None] * var))
-    # and against the general path of this library (k_estep_tc + k_stats_diag8) after the M-step both feed
-    stats_g, ll_g, _ = m.estep(batch, lab, None, eng.FP32)
-    assert_close(ll.cpu().numpy(), ll_g.cpu().numpy()[order], 1e-6, what="loglik vs general path")
 
 
 def test_estep_short_and_ragged_utterances_tc_vs_float64(eng):
@@ -549,26 +508,3 @@ def test_viterbi_equal_length_shape_sweep_vs_oracle(eng, M, D):
         else:
             # no model reaches the exit below 9 frames: every score is -inf, decoder.py:42-47 picks no word and returns no path
             assert np.all(out["best_word"].cpu().numpy() == -1) and np.all(np.isneginf(sc))
-
-
-def test_train_words_grouped_path_matches_general(eng, monkeypatch):
-    """engine.train_words: the opt-in fused grouped E-step (SAPR_GROUPED=1) and the default general path give the same
-    Baum-Welch trajectory (custom_hmm.py:402-460 for the whole vocabulary) on an equal-length corpus."""
-    import torch
-    from sapr_b200 import synth
-    feats, labels, mu, sd = synth.make_corpus(600, 11, 8, 39, 40, 40, seed=33)
-    A, means, var = synth.truth_models(mu, sd, 0.9)
-    rng = np.random.default_rng(1)
-    means0 = means + 0.2 * np.sqrt(var) * rng.standard_normal(means.shape)
-    batch = eng.PackedBatch.from_features(feats)
-    lab = torch.as_tensor(np.asarray(labels, dtype=np.int32), device="cuda")
-    out = {}
-    for mode in ("0", "1"):
-        monkeypatch.setenv("SAPR_GROUPED", mode)
-        m = eng.WordModels(11, 8, 39)
-        m.set(means0, var, A)
-        hist = eng.train_words(m, batch, lab, 3, 1e-3, eng.FP32, tol=0.0)
-        out[mode] = (hist, m.get())
-    assert_close(out["1"][0], out["0"][0], 1e-6, what="log-likelihood history")
-    assert np.max(np.abs(out["1"][1][0] - out["0"][1][0]) / np.sqrt(var)) < 1e-3          # means, relative to sigma
-    assert_close(out["1"][1][2], out["0"][1][2], 1e-4, atol=1e-6, what="transitions")
