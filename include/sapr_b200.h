@@ -68,7 +68,7 @@ int sapr_sync(sapr_ctx *ctx);
  * 2 = fused E-step forward/backward, 3 = E-step feature statistics, 4 = ergodic tensor-core emission,
  * 5 = ergodic tensor-core forward, 6 = fp32 word near-tie re-decoding, 7 = dense-topology fused Viterbi (its arg-max / back-trace
  * counts as 1), 8 = float64 re-decoding of dense-topology word near-ties, 9 = dense-topology fp32 E-step forward / backward,
- * 10 = its feature statistics) since the last sapr_profile(ctx, 1). */
+ * 10 = its feature statistics, 11 = hmmlearn M-step) since the last sapr_profile(ctx, 1). */
 int sapr_profile(sapr_ctx *ctx, int enable);
 int sapr_profile_read(sapr_ctx *ctx, int which, double *ms, int64_t *launches);
 
@@ -213,6 +213,14 @@ int sapr_ergodic_score(sapr_ctx *ctx, sapr_models *m, int mi, const float *X, in
 int64_t sapr_hl_stats_len(int S, int D);
 int sapr_hl_estep(sapr_ctx *ctx, sapr_models *m, int mi, const float *X, int ldx, const int64_t *offsets, int B,
                   int64_t total_frames, double *stats, double *logprob);
+/* hmmlearn GaussianHMM._do_mstep ('diag') for every model of a DENSE + DIAG set, from the statistics sapr_estep gives it
+ * (per model [start S | trans S*S | post S | obs S*D | obs2 S*D], after any all-reduce).  Updates the device parameters in
+ * place and re-derives the fp32 image (sapr_models_prepare).  Bit for bit with the numpy expressions (operation order, no FMA
+ * contraction, NaN-propagating maximum, numpy's pairwise row sums); S <= 1024.
+ *   priors     DEVICE float64[M * (S + S*S + 3*S*D + 1)], per model
+ *              [startprob_prior S | transmat_prior S*S | means_prior S*D | means_weight S*D | covars_prior S*D | covars_weight]
+ *   flags_host HOST int32[M]: bit 0 's', 1 't', 2 'm', 3 'c' (GaussianHMM.params); 0 leaves the model untouched       */
+int sapr_hl_mstep(sapr_ctx *ctx, sapr_models *m, const double *stats, const double *priors, const int32_t *flags_host);
 
 /* ---- evaluation metrics: assignment2/eval.py:28-38 (sklearn confusion_matrix + accuracy_score over the label indices).
  * truth / pred int32[B] (device), cm int64[M][M + 1] (device, zeroed by the call; column M = no model reachable, pred < 0),

@@ -64,6 +64,7 @@ SIGNATURES = {
     "sapr_hl_decode": (_i32, [_vp, _vp, _i32, _vp, _i32, _vp, _i32, _i64, _vp, _vp]),
     "sapr_hl_stats_len": (_i64, [_i32, _i32]),
     "sapr_hl_estep": (_i32, [_vp, _vp, _i32, _vp, _i32, _vp, _i32, _i64, _vp, _vp]),
+    "sapr_hl_mstep": (_i32, [_vp, _vp, _vp, _vp, _vp]),
     "sapr_viterbi_flagged": (_i32, [_vp, _vp]),
     "sapr_confusion": (_i32, [_vp, _vp, _vp, _i32, _i32, _vp, _vp]),
     "sapr_comm_unique_id": (_i32, [_vp]),

@@ -429,3 +429,107 @@ extern "C" int sapr_hl_estep(sapr_ctx *ctx, sapr_models *m, int mi, const float 
     SAPR_LAUNCH_CHECK(ctx);
     return SAPR_OK;
 }
+
+// ---- hmmlearn 0.3.3 GaussianHMM._do_mstep ('diag'), every model of the set at once, bit for bit with the numpy expression of
+// hmmlearn_hmm.py: same operation order, no FMA contraction (__d*_rn), numpy's NaN-propagating maximum and its pairwise sum.
+__device__ __forceinline__ double np_maximum(double a, double b) { return (a >= b || a != a) ? a : b; }
+
+// numpy's pairwise_sum of a contiguous float64 row (what sp.sum() and tm.sum(axis=1) run): sequential below 8 elements, eight
+// strided accumulators up to 128, above that split at n/2 rounded down to a multiple of 8.  L bounds the recursion: the larger
+// half is at most n/2 + 8, so 5 levels take n <= 1024 down to <= 128.
+__device__ __forceinline__ double np_block_sum(const double *a, int n) {
+    if (n < 8) {
+        double r = -0.0;
+        for (int i = 0; i < n; i++) r = __dadd_rn(r, a[i]);
+        return r;
+    }
+    double r[8];
+    for (int k = 0; k < 8; k++) r[k] = a[k];
+    int i = 8;
+    for (; i < n - (n % 8); i += 8)
+        for (int k = 0; k < 8; k++) r[k] = __dadd_rn(r[k], a[i + k]);
+    double s = __dadd_rn(__dadd_rn(__dadd_rn(r[0], r[1]), __dadd_rn(r[2], r[3])), __dadd_rn(__dadd_rn(r[4], r[5]), __dadd_rn(r[6], r[7])));
+    for (; i < n; i++) s = __dadd_rn(s, a[i]);
+    return s;
+}
+template <int L> __device__ double np_pairwise_sum(const double *a, int n) {
+    if (n <= 128) return np_block_sum(a, n);
+    int n2 = n / 2;
+    n2 -= n2 % 8;
+    return __dadd_rn(np_pairwise_sum<L - 1>(a, n2), np_pairwise_sum<L - 1>(a + n2, n - n2));
+}
+template <> __device__ double np_pairwise_sum<0>(const double *a, int n) { return np_block_sum(a, n); }
+// numpy's sum reduction adds the pairwise sum to its identity 0.0
+__device__ __forceinline__ double np_sum(const double *a, int n) { return __dadd_rn(0.0, np_pairwise_sum<5>(a, n)); }
+
+// one CTA per model: thread 0 the start probabilities, a thread per transmat row, a thread per (state, dim) for the mean and the
+// variance (the variance reads the new mean from the same thread).  The normalisations work in place: a row's zero mask reads
+// the old value of the element it replaces.
+__global__ void k_hl_mstep(int S, int D, const double *__restrict__ stats, const double *__restrict__ priors,
+                           const int32_t *__restrict__ flags, double *__restrict__ mean, double *__restrict__ cov,
+                           double *__restrict__ A, double *__restrict__ pi) {
+    const int mi = blockIdx.x;
+    const int f = flags[mi];
+    if (!f) return;
+    const size_t SD = (size_t)S * D;
+    const double *start = stats + (size_t)mi * (S + (size_t)S * S + S + 2 * SD), *trans = start + S, *post = trans + (size_t)S * S,
+                 *obs = post + S, *obs2 = obs + SD;
+    const double *spp = priors + (size_t)mi * (S + (size_t)S * S + 3 * SD + 1), *tmp = spp + S, *mp = tmp + (size_t)S * S,
+                 *mw = mp + SD, *cp = mw + SD;
+    double *pim = pi + (size_t)mi * S, *Am = A + (size_t)mi * S * S, *mu = mean + (size_t)mi * SD, *var = cov + (size_t)mi * SD;
+    if ((f & 1) && threadIdx.x == 0) {                 // 's': sp = max(startprob_prior - 1 + start, 0), masked, / sp.sum()
+        for (int j = 0; j < S; j++) {
+            const double v = np_maximum(__dadd_rn(__dsub_rn(spp[j], 1.0), start[j]), 0.0);
+            pim[j] = (pim[j] == 0.0) ? 0.0 : v;
+        }
+        const double s = np_sum(pim, S);
+        for (int j = 0; j < S; j++) pim[j] = __ddiv_rn(pim[j], s);
+    }
+    if (f & 2)                                         // 't': the same per row; a row summing to 0 is divided by 1
+        for (int i = threadIdx.x; i < S; i += blockDim.x) {
+            double *row = Am + (size_t)i * S;
+            const double *tr = trans + (size_t)i * S, *tp = tmp + (size_t)i * S;
+            for (int j = 0; j < S; j++) {
+                const double v = np_maximum(__dadd_rn(__dsub_rn(tp[j], 1.0), tr[j]), 0.0);
+                row[j] = (row[j] == 0.0) ? 0.0 : v;
+            }
+            double rs = np_sum(row, S);
+            if (rs == 0.0) rs = 1.0;
+            for (int j = 0; j < S; j++) row[j] = __ddiv_rn(row[j], rs);
+        }
+    if (f & 12) {
+        const double cwm = __dsub_rn(cp[SD], 1.0);     // max(covars_weight - 1, 0), Python's max
+        const double cw0 = (0.0 > cwm) ? 0.0 : cwm;
+        for (size_t k = threadIdx.x; k < SD; k += blockDim.x) {
+            const double denom = post[k / D];
+            double m = mu[k];
+            if (f & 4)                                 // 'm': (mw * mp + obs) / (mw + post)
+                m = __ddiv_rn(__dadd_rn(__dmul_rn(mw[k], mp[k]), obs[k]), __dadd_rn(mw[k], denom));
+            if (f & 8) {                               // 'c': (cp + c_n) / max(c_d, 1e-5) around the (new) mean
+                const double md = __dsub_rn(m, mp[k]);
+                const double cn = __dadd_rn(__dsub_rn(__dadd_rn(__dmul_rn(mw[k], __dmul_rn(md, md)), obs2[k]), __dmul_rn(__dmul_rn(2.0, m), obs[k])),
+                                            __dmul_rn(__dmul_rn(m, m), denom));
+                var[k] = __ddiv_rn(__dadd_rn(cp[k], cn), np_maximum(__dadd_rn(cw0, denom), 1e-5));
+            }
+            mu[k] = m;
+        }
+    }
+}
+
+extern "C" int sapr_hl_mstep(sapr_ctx *ctx, sapr_models *m, const double *stats, const double *priors, const int32_t *flags_host) {
+    if (!ctx || !m || !stats || !priors || !flags_host) return SAPR_E_INVALID;
+    if (m->topology != SAPR_TOPO_DENSE || m->emission != SAPR_EMIT_DIAG)
+        SAPR_FAIL(ctx, SAPR_E_INVALID, "hl_mstep: needs DENSE topology + DIAG emission");
+    if (!m->valid) SAPR_FAIL(ctx, SAPR_E_INVALID, "hl_mstep: model parameters not set");
+    if (m->S > HL_MAX_S_CTA) SAPR_FAIL(ctx, SAPR_E_RANGE, "hl_mstep: more than 1024 states");
+    int rc = sapr_ws_reserve(ctx, 5, sizeof(int32_t) * m->M);
+    if (rc) return rc;
+    // a copy from pageable memory has consumed the source when it returns: no stream synchronisation is needed
+    SAPR_CUDA(ctx, cudaMemcpyAsync(ctx->ws[5], flags_host, sizeof(int32_t) * m->M, cudaMemcpyHostToDevice, ctx->stream));
+    {
+        ProfScope ps(ctx, 11);
+        k_hl_mstep<<<m->M, 256, 0, ctx->stream>>>(m->S, m->D, stats, priors, (const int32_t *)ctx->ws[5], m->mean, m->cov, m->A, m->pi);
+    }
+    SAPR_LAUNCH_CHECK(ctx);
+    return sapr_models_prepare(m);
+}

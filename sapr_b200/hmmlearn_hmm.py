@@ -10,8 +10,10 @@ float64 kernels of csrc/hmmlearn.cu.  ``HMMLearnModel`` is the reference's wrapp
 ``decode`` is one model at a time, as decoder.py:43 calls it.  To recognise many utterances against a vocabulary of such
 models at once, ``Decoder.decode_batch`` stacks them into one DENSE ``WordModels`` set (fp32 fused kernel of
 csrc/viterbi_dense.cu for up to 32 states; its float64 verification mode equals this class's ``decode`` bit for bit).
-``fit`` is one model at a time too; ``fit_vocabulary`` fits every word's model at once, with one E-step over all utterances
-of the vocabulary per iteration (csrc/estep_dense.cu) and each model's own M-step.
+``fit`` is one model at a time too; ``fit_vocabulary`` fits every word's model at once: per iteration one E-step over all
+utterances of the vocabulary (csrc/estep_dense.cu) and one device M-step for every active model (``sapr_hl_mstep``, bit for bit
+with ``GaussianHMM._do_mstep``), with the parameters resident on the device from the first iteration to the last.  Given a
+``dist.Dist`` it shards the utterances over the ranks and sums the statistics in one all-reduce per iteration.
 """
 from __future__ import annotations
 
@@ -279,16 +281,59 @@ class HMMLearnModel:
             logging.error(f"Error occurred while training {self.model_name} HMM: {e}")
 
 
-def fit_vocabulary(models: List[GaussianHMM], features, precision: str = "fp32") -> List[GaussianHMM]:
+_PARAM_BITS = {"s": 1, "t": 2, "m": 4, "c": 8}
+
+
+def expand_priors(models: List[GaussianHMM]) -> np.ndarray:
+    """The priors of every model as the float64 block ``sapr_hl_mstep`` reads, one row per model:
+    [startprob_prior S | transmat_prior S*S | means_prior S*D | means_weight S*D | covars_prior S*D | covars_weight].
+    Each prior is a scalar or an array of exactly its parameter's shape (``startprob_prior`` (S,), ``transmat_prior`` (S, S),
+    the means and covariance priors (S, D)); ``covars_weight`` is a scalar, as ``_do_mstep`` passes it to Python's ``max``.
+    ValueError otherwise."""
+    rows = []
+    for i, mdl in enumerate(models):
+        S, D = np.shape(mdl.means_)
+        parts = []
+        for name, shape in (("startprob_prior", (S,)), ("transmat_prior", (S, S)), ("means_prior", (S, D)),
+                            ("means_weight", (S, D)), ("covars_prior", (S, D)), ("covars_weight", ())):
+            v = np.asarray(getattr(mdl, name), dtype=np.float64)
+            if v.shape not in ((), shape):
+                raise ValueError(f"model {i}: {name} must be a scalar" + (f" or shaped {shape}" if shape else "") +
+                                 f"; got shape {v.shape}")
+            parts.append(np.broadcast_to(v, shape).ravel())
+        rows.append(np.concatenate(parts))
+    return np.stack(rows)
+
+
+def param_flags(models: List[GaussianHMM]) -> np.ndarray:
+    """int32[M]: the letters of each model's ``params`` as ``sapr_hl_mstep``'s flag bits ('s' 1, 't' 2, 'm' 4, 'c' 8)."""
+    return np.array([sum(b for c, b in _PARAM_BITS.items() if c in mdl.params) for mdl in models], dtype=np.int32)
+
+
+def vocabulary_shards(lengths, world: int):
+    """(u_begin, u_end) per rank over the model-grouped utterance list (``lengths`` = frames per utterance, every utterance of
+    model 0, then of model 1, ...): contiguous, frame-balanced ranges that cover every utterance once (``dist.shard_bounds``)."""
+    from .dist import shard_bounds
+    return shard_bounds(np.concatenate([[0], np.cumsum(np.asarray(lengths, dtype=np.int64))]), world)
+
+
+def fit_vocabulary(models: List[GaussianHMM], features, precision: str = "fp32", dist=None) -> List[GaussianHMM]:
     """Fit every model of a vocabulary at once: ``features[m]`` is model m's list of (D, T) arrays.  The end state equals
-    ``models[m].fit(X_m, lengths_m)`` for each m: every iteration runs ONE dense E-step over all utterances (each against its
-    own word's model), then, for each model still active, its own ``_do_mstep`` and ``monitor_.report`` -- the order
-    ``GaussianHMM.fit`` uses -- so priors, ``params`` and the zero masks of ``startprob_`` / ``transmat_`` behave as in the
-    per-model fit.  A model leaves the active set when its monitor has converged (its own ``n_iter`` and ``tol``); its
-    parameters then stay as they are.  ``precision="fp64"`` runs GaussianHMM.fit's float64 E-step per model and is bit-identical
-    to the per-model fits; ``"fp32"`` is the fused kernel (up to 32 states).  Returns ``models``."""
+    ``models[m].fit(X_m, lengths_m)`` for each m.  The parameters stay on the device for the whole fit: every iteration runs ONE
+    dense E-step over all utterances (each against its own word's model), then ``sapr_hl_mstep`` -- hmmlearn's ``_do_mstep``
+    for every model still active, bit for bit -- then each active model's ``monitor_.report``: the order ``GaussianHMM.fit``
+    uses, so priors, ``params`` and the zero masks of ``startprob_`` / ``transmat_`` behave as in the per-model fit.  A model
+    leaves the active set when its monitor has converged (its own ``n_iter`` and ``tol``); its parameters then stay as they
+    are.  The fitted parameters are written back to the models once, at the end.  ``precision="fp64"`` runs GaussianHMM.fit's
+    float64 E-step per model and is bit-identical to the per-model fits; ``"fp32"`` is the fused kernel (up to 32 states).
+
+    ``dist`` (a ``dist.Dist``) shards the utterances over its ranks: every rank passes the whole vocabulary and runs the
+    E-step on its contiguous, frame-balanced share of the model-grouped utterance list; the statistics and the per-model
+    log-likelihood sums are summed over the ranks in ONE all-reduce per iteration, so every rank takes the same M-step and
+    convergence decisions and ends with the same parameters and histories.  Returns ``models``."""
     from ._lib import FP32, FP64
     from .decoder import stack_hmmlearn_models
+    torch = _torch()
     if precision not in ("fp32", "fp64"):
         raise ValueError("precision must be 'fp32' or 'fp64'")
     if len(models) != len(features):
@@ -299,29 +344,66 @@ def fit_vocabulary(models: List[GaussianHMM], features, precision: str = "fp32")
         mdl._check()
     means, var, tm, sp = stack_hmmlearn_models(models)
     M, S, D = means.shape
+    priors, flags = expand_priors(models), param_flags(models)
     feats = [np.asarray(x, dtype=np.float32) for f in features for x in f]
     if any(x.ndim != 2 or x.shape[0] != D for x in feats):
         raise ValueError(f"every utterance must be a (D, T) array with D = {D} features")
     counts = np.array([len(f) for f in features])
     bounds = np.concatenate([[0], np.cumsum(counts)])
-    batch = PackedBatch.from_features(feats, labels=np.repeat(np.arange(M), counts))
+    labels = np.repeat(np.arange(M), counts)
+    sharded = dist is not None and dist.world > 1
+    u0, u1 = vocabulary_shards([x.shape[1] for x in feats], dist.world)[dist.rank] if sharded else (0, len(feats))
+    # a rank whose shard is empty still takes part in every all-reduce, with zero statistics
+    batch = PackedBatch.from_features(feats[u0:u1], labels=labels[u0:u1]) if u1 > u0 else None
     dev = WordModels(M, S, D, EMIT_DIAG, TOPO_DENSE)
+    dev.set(means, var, tm, sp)
+    device = dev.ctx.device
+    d_priors = torch.as_tensor(priors, device=device)
     prec = FP64 if precision == "fp64" else FP32
+    lab = None if batch is None else batch.labels.to(torch.int64)
+    ll_host = torch.empty(M if sharded else u1 - u0, dtype=torch.float64, pin_memory=True)
     for mdl in models:
         mdl.monitor_ = ConvergenceMonitor(mdl.tol, mdl.n_iter, mdl.verbose)
         mdl.monitor_._reset()
     active = [i for i, mdl in enumerate(models) if mdl.n_iter > 0]
     while active:
-        dev.set(*stack_hmmlearn_models(models))
-        stats, loglik, _ = dev.estep(batch, batch.labels, None, prec)
-        st = dev.unpack_stats(stats)
-        ll = loglik.cpu().numpy()
+        if batch is not None:
+            stats, loglik, _ = dev.estep(batch, batch.labels, None, prec)
+        else:
+            stats = torch.zeros((M, dev.stats_stride()), dtype=torch.float64, device=device)
+            loglik = torch.zeros(0, dtype=torch.float64, device=device)
+        if sharded:
+            ll_m = torch.zeros(M, dtype=torch.float64, device=device)
+            if lab is not None:
+                ll_m.index_add_(0, lab, loglik)
+            packed = torch.cat([stats.reshape(-1), ll_m])
+            dist.allreduce_(packed)
+            stats, loglik = packed[:-M], packed[-M:]
+        ll_host.copy_(loglik, non_blocking=True)        # the host reads it while the M-step runs
+        copied = torch.cuda.Event()
+        copied.record()
+        step = np.zeros(M, dtype=np.int32)
+        step[active] = flags[active]
+        dev.ctx.check(dev.lib.sapr_hl_mstep(dev.ctx.h, dev.h, ptr(stats), ptr(d_priors), ptr(step)))
+        copied.synchronize()
+        ll = ll_host.numpy()
         still = []
         for i in active:
             mdl = models[i]
-            mdl._do_mstep({k: v[i] for k, v in st.items()})
-            mdl.monitor_.report(float(ll[bounds[i]:bounds[i + 1]].sum()))
+            mdl.monitor_.report(float(ll[i]) if sharded else float(ll[bounds[i]:bounds[i + 1]].sum()))
             if not mdl.monitor_.converged:
                 still.append(i)
         active = still
+    means, var, tm, sp = dev.get()
+    for i, mdl in enumerate(models):
+        if mdl.monitor_.iter == 0:
+            continue
+        if "s" in mdl.params:
+            mdl.startprob_ = sp[i].copy()
+        if "t" in mdl.params:
+            mdl.transmat_ = tm[i].copy()
+        if "m" in mdl.params:
+            mdl.means_ = means[i].copy()
+        if "c" in mdl.params:
+            mdl._covars = var[i].copy()
     return models

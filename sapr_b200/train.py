@@ -7,7 +7,9 @@ Not rebuilt: ``plot_training_progress`` (train.py:16-48, matplotlib figure) -- t
 histories it would plot are returned in ``train_hmm.histories`` instead.
 
 ``batched=True`` (hmmlearn models only) fits the whole vocabulary at once with ``hmmlearn_hmm.fit_vocabulary``: one E-step over
-every word's utterances per iteration instead of one per word, same pickles, return value and histories.
+every word's utterances per iteration instead of one per word, same pickles, return value and histories.  With ``dist`` (a
+``dist.Dist``) it shards the utterances over the ranks; every rank returns the same models and histories and rank 0 alone
+writes the pickles.
 
 ``semantics`` is an addition: ``"sapr"`` (default) = custom_hmm.py as written, ``"standard"`` = diagonal
 Gaussian emission over all frames (SURVEY 0.1); it is forwarded to the custom ``HMM`` only.
@@ -52,9 +54,11 @@ def save_model(model, model_path: Path) -> None:
 def train_hmm(implementation: Literal["custom", "hmmlearn"] = "hmmlearn", num_states: int = 8, num_features: int = 13,
               n_iter: int = 15, min_covar: float = 0.01, var_floor_factor: float = 0.001,
               feature_set_path: str = "feature_set", models_dir: str = "trained_models", vocabs: List[str] = None,
-              semantics: str = "sapr", batched: bool = False) -> Dict[str, Union[HMM, HMMLearnModel]]:
+              semantics: str = "sapr", batched: bool = False, dist=None) -> Dict[str, Union[HMM, HMMLearnModel]]:
     if batched and implementation != "hmmlearn":
         raise ValueError("batched=True fits hmmlearn models; custom models train per word (engine.train_words batches them)")
+    if dist is not None and not batched:
+        raise ValueError("dist shards the batched fit (batched=True); the per-word loop runs in one process")
     vocabs = list(VOCABS if vocabs is None else vocabs)
     impl_dir = Path(models_dir) / implementation
     impl_dir.mkdir(parents=True, exist_ok=True)
@@ -70,10 +74,11 @@ def train_hmm(implementation: Literal["custom", "hmmlearn"] = "hmmlearn", num_st
             hmms[word] = HMMLearnModel(num_states=num_states, model_name=word, n_iter=n_iter, min_covar=min_covar,
                                        feature_set=feature_set)
         logging.info(f"Training {len(vocabs)} hmmlearn models at once in {n_iter} iterations...")
-        fit_vocabulary([hmms[w].model for w in vocabs], [features[w] for w in vocabs])
+        fit_vocabulary([hmms[w].model for w in vocabs], [features[w] for w in vocabs], dist=dist)
         for word in vocabs:
             histories[word] = list(hmms[word].model.monitor_.history)
-            save_model(hmms[word].model, impl_dir / f"{word}_{implementation}_{n_iter}.pkl")
+            if dist is None or dist.rank == 0:
+                save_model(hmms[word].model, impl_dir / f"{word}_{implementation}_{n_iter}.pkl")
         train_hmm.histories = histories
         return hmms
     for word in vocabs:

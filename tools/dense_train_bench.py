@@ -2,7 +2,9 @@
 
 reference: 330 utterances, T ~ U{80..120}, D = 13, S = 10, M = 11, 15 iterations -- train_hmm("hmmlearn") per word (one
            GaussianHMM.fit per word, float64 E-steps) against train_hmm(..., batched=True) (one fp32 dense E-step per iteration for
-           the whole vocabulary), wall time around synchronised work, per-word log-likelihood histories compared.
+           the whole vocabulary), wall time around synchronised work, per-word log-likelihood histories compared.  The batched run
+           alternates the parent's fit_vocabulary (host M-step, parameters re-uploaded every iteration) with the device-resident
+           one, and one profiled run of each splits an iteration into E-step kernels, M-step kernel and the remainder.
 throughput: 100 000 utterances x 200 frames, 11 models, S = 10, D in {13, 39}, left-to-right (2S - 2 arcs) and Dirichlet-dense
            transitions, utterances grouped by word.  The fp32 E-step's kernel time comes from the profile classes (9 = forward /
            backward, 10 = feature statistics), averaged over the timed calls; the float64 path (SAPR_FP64 = sapr_hl_estep per
@@ -29,28 +31,112 @@ from tools.dense_bench import LANES, SMS, gpu_info, make_models   # noqa: E402
 WORDS = ["heed", "hid", "head", "had", "hard", "hud", "hod", "hoard", "hood", "whod", "heard"]
 
 
-def reference_size(tmp):
+def parent_fit_vocabulary(models, features, precision="fp32"):
+    """fit_vocabulary as it was before the device M-step, for the comparison: every iteration uploads every model's parameters
+    (dev.set), downloads the statistics and runs one numpy _do_mstep per active model."""
+    from sapr_b200._lib import EMIT_DIAG, FP32, FP64, TOPO_DENSE
+    from sapr_b200.decoder import stack_hmmlearn_models
+    from sapr_b200.engine import PackedBatch, WordModels
+    from sapr_b200.hmmlearn_hmm import ConvergenceMonitor
+    for mdl in models:
+        mdl._check()
+    means, _, _, _ = stack_hmmlearn_models(models)
+    M, S, D = means.shape
+    feats = [np.asarray(x, dtype=np.float32) for f in features for x in f]
+    counts = np.array([len(f) for f in features])
+    bounds = np.concatenate([[0], np.cumsum(counts)])
+    batch = PackedBatch.from_features(feats, labels=np.repeat(np.arange(M), counts))
+    dev = WordModels(M, S, D, EMIT_DIAG, TOPO_DENSE)
+    prec = FP64 if precision == "fp64" else FP32
+    for mdl in models:
+        mdl.monitor_ = ConvergenceMonitor(mdl.tol, mdl.n_iter, mdl.verbose)
+    active = [i for i, mdl in enumerate(models) if mdl.n_iter > 0]
+    while active:
+        dev.set(*stack_hmmlearn_models(models))
+        stats, loglik, _ = dev.estep(batch, batch.labels, None, prec)
+        st = dev.unpack_stats(stats)
+        ll = loglik.cpu().numpy()
+        still = []
+        for i in active:
+            models[i]._do_mstep({k: v[i] for k, v in st.items()})
+            models[i].monitor_.report(float(ll[bounds[i]:bounds[i + 1]].sum()))
+            if not models[i].monitor_.converged:
+                still.append(i)
+        active = still
+    return models
+
+
+def reference_size(tmp, rounds=3):
+    """train_hmm per word, then train_hmm(batched=True) with the parent's fit_vocabulary and with this one, alternated; the
+    fit_vocabulary calls are timed on their own too, and one profiled run of each splits an iteration into E-step kernels
+    (classes 9 + 10), M-step (class 11) and the remainder (launches, copies, host work)."""
     import torch
-    from sapr_b200 import synth
+    from sapr_b200 import _lib, hmmlearn_hmm, synth, train
     from sapr_b200.train import train_hmm
     feats, labels, _, _ = synth.make_corpus(330, 11, 8, 13, 80, 120, seed=2024)
     fs = os.path.join(tmp, "feature_set")
     os.makedirs(fs)
     for u, (x, w) in enumerate(zip(feats, labels)):
         np.save(os.path.join(fs, f"sp{u // 11:02d}a_w{u:03d}_{WORDS[w]}.npy"), x)
-    out = {}
-    for name, batched in (("warmup", True), ("per_word", False), ("batched", True)):
+    impls = {"parent": parent_fit_vocabulary, "this": hmmlearn_hmm.fit_vocabulary}
+    fit_s = []
+
+    def timed(fn):
+        def run(*a, **k):
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            r = fn(*a, **k)
+            torch.cuda.synchronize()
+            fit_s.append(time.perf_counter() - t0)
+            return r
+        return run
+
+    def batched_run(impl, tag):
+        train.fit_vocabulary = timed(impls[impl])
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        train_hmm("hmmlearn", 8, 13, n_iter=15, feature_set_path=fs, models_dir=os.path.join(tmp, name), batched=batched)
+        train_hmm("hmmlearn", 8, 13, n_iter=15, feature_set_path=fs, models_dir=os.path.join(tmp, tag), batched=True)
         torch.cuda.synchronize()
-        out[name] = (time.perf_counter() - t0, dict(train_hmm.histories))
-    hp, hb = out["per_word"][1], out["batched"][1]
+        return time.perf_counter() - t0, fit_s[-1], dict(train_hmm.histories)
+
+    try:
+        batched_run("this", "warmup")
+        batched_run("parent", "warmup")
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        train_hmm("hmmlearn", 8, 13, n_iter=15, feature_set_path=fs, models_dir=os.path.join(tmp, "per_word"))
+        torch.cuda.synchronize()
+        per_word = (time.perf_counter() - t0, dict(train_hmm.histories))
+        runs = {"parent": [], "this": []}
+        for r in range(rounds):
+            for impl in ("parent", "this"):
+                runs[impl].append(batched_run(impl, f"{impl}{r}"))
+        ctx = _lib.default_context()
+        split = {}
+        for impl in ("parent", "this"):
+            ctx.profile(True)
+            _, fit, hist = batched_run(impl, f"{impl}_prof")
+            c9, c10, c11 = (ctx.profile_read(k)[0] for k in (9, 10, 11))
+            ctx.profile(False)
+            n = max(len(h) for h in hist.values())
+            split[impl] = {"iterations": n, "fit_ms_per_iteration": round(fit * 1e3 / n, 3),
+                           "estep_kernels_ms": round((c9 + c10) / n, 4), "mstep_kernel_ms": round(c11 / n, 4),
+                           "remainder_ms": round((fit * 1e3 - c9 - c10 - c11) / n, 3)}
+    finally:
+        train.fit_vocabulary = hmmlearn_hmm.fit_vocabulary
+    hp = per_word[1]
+    hb, hq = runs["this"][-1][2], runs["parent"][-1][2]
     n = {w: min(len(hp[w]), len(hb[w])) for w in WORDS}          # a word may converge (tol) one iteration apart
     rel = max(float(np.max(np.abs(np.array(hb[w][:n[w]]) - np.array(hp[w][:n[w]])) / np.abs(np.array(hp[w][:n[w]]))))
               for w in WORDS)
-    return {"utts": 330, "iters": 15, "per_word_s": round(out["per_word"][0], 4), "batched_s": round(out["batched"][0], 4),
-            "speedup": round(out["per_word"][0] / out["batched"][0], 2), "history_max_rel_diff": rel,
+    med = {k: float(np.median([x[0] for x in v])) for k, v in runs.items()}
+    return {"utts": 330, "iters": 15, "per_word_s": round(per_word[0], 4), "batched_s": round(med["this"], 4),
+            "parent_batched_s": round(med["parent"], 4), "batched_s_runs": [round(x[0], 4) for x in runs["this"]],
+            "parent_batched_s_runs": [round(x[0], 4) for x in runs["parent"]],
+            "fit_s": round(float(np.median([x[1] for x in runs["this"]])), 4),
+            "parent_fit_s": round(float(np.median([x[1] for x in runs["parent"]])), 4),
+            "histories_equal_parent": hb == hq, "iteration_split": split,
+            "speedup": round(per_word[0] / med["this"], 2), "history_max_rel_diff": rel,
             "iterations_per_word": [len(hp[w]) for w in WORDS], "iterations_batched": [len(hb[w]) for w in WORDS]}
 
 
