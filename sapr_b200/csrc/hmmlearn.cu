@@ -104,23 +104,26 @@ __global__ void k_hl_backward_stats(const double *__restrict__ lf, const double 
 
 // obs = post^T X, obs2 = post^T X^2: one thread per (state, dim) and frame chunk (HL_OBS_CHUNK frames in order), then a
 // fixed-order sum over the chunks -- deterministic, and parallel over frames (one thread per output walking every frame
-// serially took seconds at 10^7 frames)
+// serially took seconds at 10^7 frames).  gridDim.y stops at 65535, so a y-block takes chunks blockIdx.y, + gridDim.y, ...
 #define HL_OBS_CHUNK 512
-__global__ void k_hl_obs_partial(const float *__restrict__ X, int ldx, int64_t total_frames, int D, int S,
+#define HL_OBS_MAX_GRID_Y 65535
+__global__ void k_hl_obs_partial(const float *__restrict__ X, int ldx, int64_t total_frames, int nchunk, int D, int S,
                                  const double *__restrict__ post, double *__restrict__ part) {
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= S * D) return;
     const int j = idx / D, d = idx % D;
-    const int64_t f0 = (int64_t)blockIdx.y * HL_OBS_CHUNK, f1 = min(f0 + HL_OBS_CHUNK, total_frames);
-    double a = 0.0, b = 0.0;
-    for (int64_t f = f0; f < f1; f++) {
-        const double g = post[f * S + j];
-        const double x = (double)X[f * ldx + d];
-        a += g * x;
-        b += g * x * x;
+    for (int c = blockIdx.y; c < nchunk; c += gridDim.y) {
+        const int64_t f0 = (int64_t)c * HL_OBS_CHUNK, f1 = min(f0 + HL_OBS_CHUNK, total_frames);
+        double a = 0.0, b = 0.0;
+        for (int64_t f = f0; f < f1; f++) {
+            const double g = post[f * S + j];
+            const double x = (double)X[f * ldx + d];
+            a += g * x;
+            b += g * x * x;
+        }
+        part[((size_t)c * 2 + 0) * S * D + idx] = a;
+        part[((size_t)c * 2 + 1) * S * D + idx] = b;
     }
-    part[((size_t)blockIdx.y * 2 + 0) * S * D + idx] = a;
-    part[((size_t)blockIdx.y * 2 + 1) * S * D + idx] = b;
 }
 __global__ void k_hl_obs_reduce(const double *__restrict__ part, int nchunk, int SD, double *__restrict__ obs, double *__restrict__ obs2) {
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
@@ -175,8 +178,9 @@ __global__ void k_hl_viterbi(const double *__restrict__ lf, const int64_t *__res
 }
 
 // ---- one CTA per utterance, one thread per destination state (32 < S <= 1024) ----
+// __launch_bounds__(HL_MAX_S_CTA) caps these kernels at 64 registers, so a 1024-thread block always fits the register file
 #define HL_MAX_S_CTA 1024
-__global__ void k_hl_forward_cta(const double *__restrict__ lf, const int64_t *__restrict__ offsets, int S,
+__global__ void __launch_bounds__(HL_MAX_S_CTA) k_hl_forward_cta(const double *__restrict__ lf, const int64_t *__restrict__ offsets, int S,
                                  const double *__restrict__ logpi, const double *__restrict__ logA,
                                  double *__restrict__ fwd_out, double *__restrict__ logprob) {
     extern __shared__ double sh_prev[];   // [S]
@@ -229,7 +233,11 @@ __device__ __forceinline__ double hl_block_reduce(double v, bool is_max, double 
 
 // backward + posteriors + statistics, one CTA per utterance at a time (CTA b takes utterances b, b + grid, ...),
 // one thread per state; the CTA's partial statistics [start S | trans S*S | post S] accumulate in pc[b] (zeroed here).
-__global__ void k_hl_backward_stats_cta(const double *__restrict__ lf, const double *__restrict__ fwd,
+// Capped at 64 registers for 1024 threads this kernel spills (32 / 40 bytes of stores / loads a thread), so blocks of up to
+// HL_BWD_CTA_NOSPILL threads take an instance bounded at 768 threads: 80 registers, no spills.  Same arithmetic in both.
+#define HL_BWD_CTA_NOSPILL 768
+template <int MAX_THREADS>
+__global__ void __launch_bounds__(MAX_THREADS, 1) k_hl_backward_stats_cta(const double *__restrict__ lf, const double *__restrict__ fwd,
                                         const int64_t *__restrict__ offsets, int B, int S,
                                         const double *__restrict__ logA, const double *__restrict__ logprob,
                                         double *__restrict__ bwd_ws, double *__restrict__ post_out, double *__restrict__ pc) {
@@ -299,7 +307,7 @@ __global__ void k_hl_backward_stats_cta(const double *__restrict__ lf, const dou
     }
 }
 
-__global__ void k_hl_viterbi_cta(const double *__restrict__ lf, const int64_t *__restrict__ offsets, int S,
+__global__ void __launch_bounds__(HL_MAX_S_CTA) k_hl_viterbi_cta(const double *__restrict__ lf, const int64_t *__restrict__ offsets, int S,
                                  const double *__restrict__ logpi, const double *__restrict__ logA,
                                  double *__restrict__ delta_ws, double *__restrict__ logprob, int32_t *__restrict__ path) {
     const int u = blockIdx.x, j = threadIdx.x;
@@ -413,8 +421,8 @@ extern "C" int sapr_hl_estep(sapr_ctx *ctx, sapr_models *m, int mi, const float 
         const int threads = (S + 31) / 32 * 32;
         k_hl_forward_cta<<<B, threads, sizeof(double) * S, ctx->stream>>>(lf, offsets, S, logpi, logA, fwd, logprob);
         SAPR_LAUNCH_CHECK(ctx);
-        k_hl_backward_stats_cta<<<nslots, threads, sizeof(double) * (S + 32), ctx->stream>>>(lf, fwd, offsets, B, S, logA, logprob,
-                                                                                             bwd, post, pu);
+        auto *bwd_stats = threads <= HL_BWD_CTA_NOSPILL ? k_hl_backward_stats_cta<HL_BWD_CTA_NOSPILL> : k_hl_backward_stats_cta<HL_MAX_S_CTA>;
+        bwd_stats<<<nslots, threads, sizeof(double) * (S + 32), ctx->stream>>>(lf, fwd, offsets, B, S, logA, logprob, bwd, post, pu);
         SAPR_LAUNCH_CHECK(ctx);
     }
     k_hl_sum_pu<<<(len + 63) / 64, 64, 0, ctx->stream>>>(pu, nslots, len, stats);
@@ -422,7 +430,8 @@ extern "C" int sapr_hl_estep(sapr_ctx *ctx, sapr_models *m, int mi, const float 
     const int nchunk = (int)((total_frames + HL_OBS_CHUNK - 1) / HL_OBS_CHUNK);
     if ((rc = sapr_ws_reserve(ctx, 5, sizeof(double) * (size_t)std::max(nchunk, 1) * 2 * S * D))) return rc;
     if (nchunk > 0) {
-        k_hl_obs_partial<<<dim3((S * D + 63) / 64, nchunk), 64, 0, ctx->stream>>>(X, ldx, total_frames, D, S, post, (double *)ctx->ws[5]);
+        k_hl_obs_partial<<<dim3((S * D + 63) / 64, std::min(nchunk, HL_OBS_MAX_GRID_Y)), 64, 0, ctx->stream>>>(
+            X, ldx, total_frames, nchunk, D, S, post, (double *)ctx->ws[5]);
         SAPR_LAUNCH_CHECK(ctx);
     }
     k_hl_obs_reduce<<<(S * D + 63) / 64, 64, 0, ctx->stream>>>((const double *)ctx->ws[5], nchunk, S * D, stats + len, stats + len + (size_t)S * D);

@@ -74,7 +74,8 @@ def _same(a, b):
     return a.shape == b.shape and np.array_equal(a, b, equal_nan=True)
 
 
-@pytest.mark.parametrize("S,D", [(3, 13), (10, 13), (32, 13), (3, 39), (10, 39), (32, 39), (40, 13), (130, 39)])
+@pytest.mark.parametrize("S,D", [(3, 13), (10, 13), (32, 13), (3, 39), (10, 39), (32, 39), (40, 13), (130, 39), (801, 13),
+                                 (1024, 39)])
 def test_hl_mstep_bit_identical_to_do_mstep(eng, S, D):
     """Every (params, priors) pair of a set at once; statistics from a real float64 E-step, with a transmat row without counts
     and a state without posterior mass written in; the models whose flag is 0 stay unchanged bit for bit."""
