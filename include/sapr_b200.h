@@ -68,7 +68,8 @@ int sapr_sync(sapr_ctx *ctx);
  * 2 = fused E-step forward/backward, 3 = E-step feature statistics, 4 = ergodic tensor-core emission,
  * 5 = ergodic tensor-core forward, 6 = fp32 word near-tie re-decoding, 7 = dense-topology fused Viterbi (its arg-max / back-trace
  * counts as 1), 8 = float64 re-decoding of dense-topology word near-ties, 9 = dense-topology fp32 E-step forward / backward,
- * 10 = its feature statistics, 11 = hmmlearn M-step) since the last sapr_profile(ctx, 1). */
+ * 10 = its feature statistics, 11 = hmmlearn M-step, 12 = dense-topology fp32 forward of sapr_score_words (its arg-max counts
+ * as 1), 13 = float64 re-scoring of its word near-ties) since the last sapr_profile(ctx, 1). */
 int sapr_profile(sapr_ctx *ctx, int enable);
 int sapr_profile_read(sapr_ctx *ctx, int which, double *ms, int64_t *launches);
 
@@ -113,7 +114,8 @@ int sapr_viterbi(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, const i
 /* fp32 production mode (tensor-core kernels or the DENSE kernel, all models, all_paths == NULL): an utterance whose best and second-best word
  * scores differ by less than 8e-6 |best| -- closer than the fp32 scores resolve -- is re-decoded in float64 inside the same
  * call (word, score, score row and path then are the verification mode's), so the recognised word equals the float64 one
- * except on exact float64 ties (decoder.py:42-47 keeps the first).  n = utterances flagged by the last call on this context
+ * except on exact float64 ties (decoder.py:42-47 keeps the first).  n = utterances flagged by the last sapr_viterbi or
+ * sapr_score_words call on this context
  * (synchronises the stream); at most 8192 per 1 GB scratch chunk are re-decoded.  SAPR_EXACT_WORDS=0 disables the pass.
  * Stream order: part of an equal-length batch's arg-max / back-trace may run on a context-owned auxiliary stream beside the
  * last launch of the main kernel; it is joined back into the context's stream before the call returns, so work the caller
@@ -209,6 +211,20 @@ int sapr_hl_decode(sapr_ctx *ctx, sapr_models *m, int mi, const float *X, int ld
  * hmmlearn_hmm.py:46-75. */
 int sapr_ergodic_score(sapr_ctx *ctx, sapr_models *m, int mi, const float *X, int ldx, const int64_t *offsets, int B,
                        int max_T, double *logprob);
+/* Batched GaussianHMM.score for every utterance x model of a DENSE + DIAG set, and recognition by total likelihood: scores[u*M + m]
+ * = log P(X_u | model m) (the forward log-likelihood, natural log; an empty utterance scores 0, one no state sequence of the
+ * model can produce -inf), best_word[u] the strict-'>' arg-max over the models (first best wins, -1 when every model scores
+ * -inf), best_score[u] its score.  Each output is nullable; at least one must be given.
+ *   SAPR_FP64  verification: sapr_hl_score per model + a running arg-max, bit for bit with GaussianHMM.score per model (any S
+ *              sapr_hl_score takes).
+ *   SAPR_FP32  fused fp32 forward of csrc/score_dense.cu (S <= 32, else SAPR_E_RANGE: SAPR_FP64, or sapr_ergodic_score for
+ *              64-256 states): per-frame log-shifted linear recursion, so utterances far from a model and transitions below the
+ *              fp32 range stay finite.  Utterances whose best and second-best scores differ by less than 8e-6 |best| are
+ *              re-scored in float64 in the same call (word, score and score row then are the verification mode's; at most 8192
+ *              per call, counted by sapr_viterbi_flagged; SAPR_EXACT_WORDS=0 disables the pass).
+ * ENTRY_EXIT or SAPR-emission sets, ldx % 4 != 0 and an unknown precision are refused with SAPR_E_INVALID. */
+int sapr_score_words(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, const int64_t *offsets, int B,
+                     int64_t total_frames, int precision, int32_t *best_word, double *best_score, double *scores);
 /* stats = [start S | trans S*S | post S | obs S*D | obs2 S*D] float64, zeroed by the call */
 int64_t sapr_hl_stats_len(int S, int D);
 int sapr_hl_estep(sapr_ctx *ctx, sapr_models *m, int mi, const float *X, int ldx, const int64_t *offsets, int B,

@@ -61,6 +61,7 @@ SIGNATURES = {
     "sapr_decode_compat": (_i32, [_vp, _vp, _i32, _vp, _i32, _i32, _i32, _vp, _vp]),
     "sapr_hl_score": (_i32, [_vp, _vp, _i32, _vp, _i32, _vp, _i32, _i64, _vp]),
     "sapr_ergodic_score": (_i32, [_vp, _vp, _i32, _vp, _i32, _vp, _i32, _i32, _vp]),
+    "sapr_score_words": (_i32, [_vp, _vp, _vp, _i32, _vp, _i32, _i64, _i32, _vp, _vp, _vp]),
     "sapr_hl_decode": (_i32, [_vp, _vp, _i32, _vp, _i32, _vp, _i32, _i64, _vp, _vp]),
     "sapr_hl_stats_len": (_i64, [_i32, _i32]),
     "sapr_hl_estep": (_i32, [_vp, _vp, _i32, _vp, _i32, _vp, _i32, _i64, _vp, _vp]),
@@ -131,7 +132,7 @@ class Context:
         self.check(self.lib.sapr_sync(self.h))
 
     def viterbi_flagged(self) -> int:
-        """Utterances the last fp32 Viterbi call flagged as word near-ties and re-decoded in float64."""
+        """Utterances the last fp32 Viterbi or word-scoring call flagged as word near-ties and re-decoded in float64."""
         n = _i64(0)
         self.check(self.lib.sapr_viterbi_flagged(self.h, C.byref(n)))
         return int(n.value)

@@ -1,7 +1,7 @@
 // api.cu -- context / model-set lifetime, workspace, and the derived-parameter kernels.
 #include "common.cuh"
 
-extern "C" int sapr_version(void) { return 102; }
+extern "C" int sapr_version(void) { return 103; }
 
 extern "C" int sapr_ctx_create(int device, void *cuda_stream, sapr_ctx **out) {
     if (!out) return SAPR_E_INVALID;

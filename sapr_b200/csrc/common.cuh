@@ -37,7 +37,7 @@ struct sapr_ctx {
     struct ProfRec { cudaEvent_t a, b; int which; };
     std::vector<ProfRec> prof;       // used records
     std::vector<ProfRec> prof_pool;  // recycled event pairs
-    bool flag_valid = false;         // ws[8] holds the flag counters of the last fp32 Viterbi call (sapr_viterbi_flagged)
+    bool flag_valid = false;         // ws[8] holds the flag counters of the last fp32 Viterbi or word-scoring call (sapr_viterbi_flagged)
     int flag_maxT = 0, flag_M = 0;   // longest utterance / models of that call (size the re-decoding scratch)
 };
 

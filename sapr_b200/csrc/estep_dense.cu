@@ -27,25 +27,12 @@
 // rebased to 0), so stats and loglik equal GaussianHMM.fit's E-step for that word bit for bit.
 #include <vector>
 
-#include "common.cuh"
+#include "dense_common.cuh"
 
 // estep.cu: grouping of utterances by model
 __global__ void k_model_start(const int32_t *__restrict__ model_of_utt, const int32_t *__restrict__ order, int B, int M,
                               int32_t *__restrict__ model_start);
 __global__ void k_group_by_model(const int32_t *__restrict__ model_of_utt, int B, int M, int32_t *__restrict__ order);
-
-#define DE_LOG2E 1.4426950408889634f
-
-__device__ __forceinline__ float de_ex2(float x) {
-    float r;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
-    return r;
-}
-__device__ __forceinline__ float de_lg2(float x) {
-    float r;
-    asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
-    return r;
-}
 
 // tiles of up to 32 utterances of one model: tile_start[m] = sum over m' < m of ceil(n_m' / 32)
 __global__ void k_dense_tiles(const int32_t *__restrict__ model_start, int M, int32_t *__restrict__ tile_start) {
@@ -65,35 +52,6 @@ __device__ __forceinline__ int de_tile_model(const int32_t *__restrict__ tile_st
         if (tile_start[mid] <= tile) lo = mid; else hi = mid - 1;
     }
     return lo;
-}
-
-// emission of one frame in log2 units for the first S states
-template <int NMAX>
-__device__ __forceinline__ void de_emit(const float *__restrict__ xrow, const float4 *__restrict__ piv, const float *__restrict__ w,
-                                        const float *__restrict__ cst, int S, int nch, float (&e)[NMAX]) {
-#pragma unroll
-    for (int j = 0; j < NMAX; j++) e[j] = (j < S) ? cst[j] : 0.f;
-    for (int c = 0; c < nch; c++) {
-        float4 x = __ldg(reinterpret_cast<const float4 *>(xrow) + c);
-        const float4 p = piv[c];
-        x.x -= p.x; x.y -= p.y; x.z -= p.z; x.w -= p.w;
-        const float4 x2 = make_float4(x.x * x.x, x.y * x.y, x.z * x.z, x.w * x.w);
-        const float4 *wc = reinterpret_cast<const float4 *>(w + (size_t)c * S * 8);
-#pragma unroll
-        for (int j = 0; j < NMAX; j++) {
-            if (j < S) {
-                const float4 a = wc[2 * j], b = wc[2 * j + 1];
-                float v = e[j];
-                v = fmaf(a.x, x.x, v); v = fmaf(b.x, x2.x, v);
-                v = fmaf(a.y, x.y, v); v = fmaf(b.y, x2.y, v);
-                v = fmaf(a.z, x.z, v); v = fmaf(b.z, x2.z, v);
-                v = fmaf(a.w, x.w, v); v = fmaf(b.w, x2.w, v);
-                e[j] = v;
-            }
-        }
-    }
-#pragma unroll
-    for (int j = 0; j < NMAX; j++) e[j] *= DE_LOG2E;
 }
 
 struct DeSmem {   // byte offsets of the dynamic shared memory of k_dense_fb
@@ -180,27 +138,7 @@ k_dense_fb(const float *__restrict__ X, int ldx, const int64_t *__restrict__ off
 #pragma unroll
             for (int j = 0; j < NMAX; j++) if (j < S) e[j] += slpi[j];
         } else {
-#pragma unroll
-            for (int j = 0; j < NMAX; j++) {
-                if (j < S) {
-                    float s = 0.f;
-                    const int k0 = sstartd[j], k1 = sstartd[j + 1];
-                    for (int k = k0; k < k1; k++) {
-                        const int i = (int)sarcd[k].y;
-                        s = fmaf(col[i * 32], sA[i * S + j], s);
-                    }
-                    if (s >= 0x1p-64f) {
-                        e[j] += de_lg2(s);
-                    } else {                                // the predecessors' mass is (near) underflow: log domain
-                        float mx = NINF;
-                        for (int k = k0; k < k1; k++) mx = fmaxf(mx, lcol[(int)sarcd[k].y * 32] + sarcd[k].x * DE_LOG2E);
-                        float s2 = 0.f;
-                        if (mx > NINF)
-                            for (int k = k0; k < k1; k++) s2 += de_ex2(lcol[(int)sarcd[k].y * 32] + sarcd[k].x * DE_LOG2E - mx);
-                        e[j] = (mx > NINF) ? e[j] + mx + de_lg2(s2) : NINF;
-                    }
-                }
-            }
+            de_fwd_step<NMAX>(col, lcol, sA, sarcd, sstartd, S, e);
         }
         float c = NINF;
 #pragma unroll

@@ -22,9 +22,7 @@
 // SAPR_FP64 (verification): sapr_hl_decode per model + a running arg-max kernel.
 #include <stdlib.h>
 
-#include "common.cuh"
-
-#define DN_TF 16   // frames of the tile staged per round
+#include "dense_common.cuh"
 
 template <int NMAX> struct DnBits {
     static constexpr int NB = NMAX <= 8 ? 3 : (NMAX <= 16 ? 4 : 5);   // bits per state
@@ -174,41 +172,14 @@ k_dense_viterbi(const float *__restrict__ X, int ldx, const int64_t *__restrict_
     int flast = 0;
     for (int t0 = 0; t0 < Tmax; t0 += DN_TF) {
         __syncthreads();                                   // the previous stage is consumed
-        for (int idx = tid; idx < DN_TF * 32 * nch; idx += nthr) {
-            const int c = idx % nch, r = (idx / nch) & 31, f = idx / (32 * nch), t = t0 + f;
-            if (t < s_T[r]) {
-                float4 v = __ldg(reinterpret_cast<const float4 *>(X + (size_t)(s_off[r] + t) * ldx) + c);
-                const float4 p = __ldg(reinterpret_cast<const float4 *>(piv_g) + c);
-                v.x -= p.x; v.y -= p.y; v.z -= p.z; v.w -= p.w;
-                sx[(f * 32 + r) * L.xs4 + c] = v;
-            }
-        }
+        dn_stage(X, ldx, piv_g, s_off, s_T, t0, nch, L.xs4, sx, tid, nthr);
         __syncthreads();
         if (!active) continue;
         const int nf = min(DN_TF, Tmax - t0);
         for (int f = 0; f < nf; f++) {
             const int t = t0 + f;
             float acc[NMAX];
-#pragma unroll
-            for (int j = 0; j < NMAX; j++) acc[j] = (j < S) ? cm[j] : 0.f;
-            const float4 *xr = sx + (size_t)(f * 32 + lane) * L.xs4;
-            for (int c = 0; c < nch; c++) {
-                const float4 x = xr[c];
-                const float4 x2 = make_float4(x.x * x.x, x.y * x.y, x.z * x.z, x.w * x.w);
-                const float4 *wc = reinterpret_cast<const float4 *>(wm + (size_t)c * S * 8);
-#pragma unroll
-                for (int j = 0; j < NMAX; j++) {
-                    if (j < S) {
-                        const float4 a = wc[2 * j], b = wc[2 * j + 1];
-                        float e = acc[j];
-                        e = fmaf(a.x, x.x, e); e = fmaf(b.x, x2.x, e);
-                        e = fmaf(a.y, x.y, e); e = fmaf(b.y, x2.y, e);
-                        e = fmaf(a.z, x.z, e); e = fmaf(b.z, x2.z, e);
-                        e = fmaf(a.w, x.w, e); e = fmaf(b.w, x2.w, e);
-                        acc[j] = e;
-                    }
-                }
-            }
+            dn_emit_tile<NMAX>(sx + (size_t)(f * 32 + lane) * L.xs4, wm, cm, S, nch, acc);
             uint32_t bits[BB::NW];
 #pragma unroll
             for (int w = 0; w < BB::NW; w++) bits[w] = 0u;
@@ -320,16 +291,7 @@ __global__ void __launch_bounds__(32) k_dense_redo(const float *__restrict__ X, 
         const double *mu = mean + ((size_t)mi * S + (j < S ? j : 0)) * D, *vr = var + ((size_t)mi * S + (j < S ? j : 0)) * D;
         double dv = -INFINITY;
         for (int t = 0; t < T; t++) {
-            double e;
-            {
-                double ld = 0.0, q = 0.0;
-                for (int d = 0; d < D; d++) {
-                    ld += log(vr[d]);
-                    const double df = (double)X[(off + t) * ldx + d] - mu[d];
-                    q += df * df / vr[d];
-                }
-                e = -0.5 * (D * SAPR_LOG2PI + ld + q);
-            }
+            const double e = dn_emit64(X + (off + t) * ldx, mu, vr, D);
             if (t == 0) {
                 dv = lpi[j < S ? j : 0] + e;
             } else {

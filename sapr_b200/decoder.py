@@ -3,7 +3,9 @@
 every utterance against every word model in ONE fused Viterbi launch (the per-model Python loop of
 decoder.py:42-47 becomes the in-kernel argmax).  ``decode_batch`` takes custom models trained with
 semantics="standard" (left-to-right, entry/exit states) and hmmlearn-style models (every state emits,
-dense transmat + startprob, up to 32 states; csrc/viterbi_dense.cu).
+dense transmat + startprob, up to 32 states; csrc/viterbi_dense.cu).  ``score_batch`` recognises hmmlearn-style models by
+total likelihood instead (the arg-max over the models of GaussianHMM.score) and returns the whole utterance x model
+log-likelihood matrix, from one fused forward launch (csrc/score_dense.cu).
 
 Model order: the reference iterates ``impl_dir.glob(pattern)`` (filesystem order, SURVEY D8) and keeps the
 first best under strict ``>``; pass ``vocab_order`` to fix the order explicitly.
@@ -120,6 +122,27 @@ class Decoder:
         offs = batch.offsets_host
         words = [self.vocab[i] if i >= 0 else None for i in bw]
         return words, bs, [p[offs[u]:offs[u + 1]].tolist() for u in range(batch.B)]
+
+    def score_batch(self, features: List[np.ndarray], true_labels=None):
+        """Recognition by total likelihood for hmmlearn models: features is a list of (D, T_u) arrays.  Returns (words,
+        best_scores, loglik): loglik is the [B, M] numpy matrix of GaussianHMM.score for every utterance and model in vocabulary
+        order, words the arg-max over the models (first best wins ties; None when no model can produce the utterance).
+        ``precision="fp64"`` (constructor) gives GaussianHMM.score per model bit for bit; the fp32 default re-scores word
+        near-ties in float64, so its words are the float64 ones.  ``true_labels`` fills ``self.last_confusion`` as
+        ``decode_batch`` does.  Custom models raise ValueError."""
+        if self.implementation != "hmmlearn":
+            raise ValueError("score_batch needs hmmlearn-style models (every state emits, dense transmat + startprob)")
+        dev = self._word_models()
+        batch = PackedBatch.from_features(features)
+        out = dev.score_words(batch, FP64 if self.precision == "fp64" else FP32, want_scores=True)
+        if true_labels is not None:
+            import torch
+            from .engine import confusion_on_device
+            cm, acc = confusion_on_device(torch.as_tensor(np.asarray(true_labels, dtype=np.int32)), out["best_word"], len(self.vocab), dev.ctx)
+            self.last_confusion = (cm.cpu().numpy(), acc)
+        bw = out["best_word"].cpu().numpy()
+        words = [self.vocab[i] if i >= 0 else None for i in bw]
+        return words, out["best_score"].cpu().numpy(), out["scores"].cpu().numpy()
 
     def decode_word_samples(self, word: str, feature_set: str = "feature_set") -> List[Dict]:
         if word not in self.vocab:

@@ -130,6 +130,22 @@ class WordModels:
                                              ptr(best_word), ptr(best_score), ptr(scores), ptr(path), ptr(allp)))
         return dict(best_word=best_word, best_score=best_score, scores=scores, path=path, all_paths=allp)
 
+    # ---- scoring (GaussianHMM.score per model + the arg-max over the models: recognition by total likelihood) ----
+    def score_words(self, batch: PackedBatch, precision=FP32, want_scores=True):
+        """log P(X_u | model m) for every utterance x model of a DENSE set, and the strict-'>' arg-max over the models (first
+        best wins, -1 when no model can produce the utterance).  Returns dict(best_word, best_score, scores [B, M] or None).
+        FP64 = GaussianHMM.score per model, bit for bit; FP32 = the fused forward of csrc/score_dense.cu (S <= 32), which
+        re-scores word near-ties in float64 (``ctx.viterbi_flagged()`` counts them)."""
+        torch = _torch()
+        dev = batch.X.device
+        B, M = batch.B, self.M
+        best_word = torch.empty(B, dtype=torch.int32, device=dev)
+        best_score = torch.empty(B, dtype=torch.float64, device=dev)
+        scores = torch.empty((B, M), dtype=torch.float64, device=dev) if want_scores else None
+        self.ctx.check(self.lib.sapr_score_words(self.ctx.h, self.h, ptr(batch.X), batch.ldx, ptr(batch.offsets), B,
+                                                 batch.total_frames, precision, ptr(best_word), ptr(best_score), ptr(scores)))
+        return dict(best_word=best_word, best_score=best_score, scores=scores)
+
     def tc_emission(self, batch: PackedBatch):
         """Debug/parity: the tensor-core emission tile, float32 [sum_T, ncols] (column m*8 + j-1)."""
         torch = _torch()
