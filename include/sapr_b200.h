@@ -148,7 +148,8 @@ int sapr_viterbi_host(sapr_ctx *ctx, sapr_models *m, const float *X_host, int ld
  * [start S | trans S*S | post S | obs S*D | obs2 S*D] as sapr_hl_estep gives it; loglik = log P(X_u); gamma_out [sum_T][S]
  * (fp32 in SAPR_FP32, float64 in SAPR_FP64).  SAPR_FP64 runs sapr_hl_estep per model on that model's utterances in batch order,
  * so stats and loglik equal GaussianHMM.fit's E-step for the word bit for bit (any S sapr_hl_estep takes).  SAPR_FP32 is the
- * fused kernel of csrc/estep_dense.cu (S <= 32, else SAPR_E_RANGE; max_T must cover the longest utterance): per-frame
+ * fused kernel of csrc/estep_dense.cu (S <= 32, and one model's parameters and accumulators within the device's opt-in shared
+ * memory per block, about D <= 228 at S = 32 on a B200; else SAPR_E_RANGE; max_T must cover the longest utterance): per-frame
  * log-shifted linear recursions, so utterances far from their model stay finite; an utterance the model cannot produce gets
  * loglik -inf and contributes nothing.  Two identical calls give identical bits.  */
 int64_t sapr_stats_stride(int N, int D);

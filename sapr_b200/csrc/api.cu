@@ -149,6 +149,7 @@ extern "C" int sapr_models_create(sapr_ctx *ctx, int M, int N, int D, int emissi
         rc |= dalloc(ctx, &arc, (size_t)M * S * S);
         rc |= dalloc(ctx, &m->dn_start, (size_t)M * (S + 1));
         rc |= dalloc(ctx, &arcs, (size_t)M * S * S);
+        rc |= dalloc(ctx, &m->dn_lg2s, (size_t)M * S * S);
         rc |= dalloc(ctx, &m->dn_starts, (size_t)M * (S + 1));
         m->dn_arc = arc; m->dn_arcs = arcs;
     }
@@ -167,7 +168,7 @@ extern "C" int sapr_models_destroy(sapr_models *m) {
     cudaStreamSynchronize(m->ctx->stream);
     void *ptrs[] = {m->mean, m->cov, m->A, m->pi, m->logA, m->logpi, m->la64, m->lb64, m->la32, m->lb32,
                     m->pk64, m->pk32, m->cst64, m->cst32, m->P, m->cstS, m->tc_image, m->dn_piv, m->dn_w, m->dn_cst,
-                    m->dn_lpi, m->dn_arc, m->dn_start, m->dn_arcs, m->dn_starts};
+                    m->dn_lpi, m->dn_arc, m->dn_start, m->dn_arcs, m->dn_lg2s, m->dn_starts};
     for (void *p : ptrs) if (p) cudaFree(p);
     delete m;
     return SAPR_OK;

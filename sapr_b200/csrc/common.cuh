@@ -91,8 +91,9 @@ struct sapr_models {
     // DENSE + DIAG sets with S <= 32 (viterbi_dense.cu): pivot p[Dp]; per model [chunk][state][8] = (a x4, b x4) with
     // a = (mu - p) / var, b = -1 / (2 var); cst[S] = -0.5 (D ln 2pi + sum ln var + sum (mu - p)^2 / var); ln pi [S];
     // finite arcs (ln A, source) grouped by destination [S*S] float2 with start[S + 1]; the same arcs (A, destination) grouped
-    // by source with starts[S + 1] (the E-step's backward sweep, estep_dense.cu)
-    float *dn_piv = nullptr, *dn_w = nullptr, *dn_cst = nullptr, *dn_lpi = nullptr;
+    // by source with starts[S + 1] (the E-step's backward sweep, estep_dense.cu), and log2 A of those source-grouped arcs
+    // [S*S] (computed in float64: the backward sweep's log-domain branch, where fp32 A of a transition below 2^-126 is 0)
+    float *dn_piv = nullptr, *dn_w = nullptr, *dn_cst = nullptr, *dn_lpi = nullptr, *dn_lg2s = nullptr;
     void *dn_arc = nullptr, *dn_arcs = nullptr;
     int32_t *dn_start = nullptr, *dn_starts = nullptr;
     bool valid = false;

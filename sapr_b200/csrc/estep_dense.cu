@@ -12,7 +12,8 @@
 //     - backward, from the emission of frame t+1 recomputed: w(j) = e_{t+1}(j) + log2 bhat_{t+1}(j),
 //       q(j) = 2^(w(j) - max w), r(i) = sum_j A_ij q(j) over the arcs grouped by source, log2 bhat_t(i) = log2 r(i);
 //       a linear sum below 2^-64 (a left-to-right chain cannot re-enter a state whose mass fell below the fp32 range) is
-//       redone in the log domain for that state, so no reachable state is lost and utterances far from the model stay finite;
+//       redone in the log domain for that state, with log2 A_ij from float64 (k_dense_prepare), so no reachable state is lost,
+//       utterances far from the model stay finite and an arc below the fp32 range keeps its share of beta and xi;
 //       gamma_t(i) ~ 2^(log2 ahat_t(i) + log2 bhat_t(i)), normalised per frame by its own sum, and
 //       xi_t(i, j) = gamma_t(i) A_ij q(j) / r(i) (so sum_j xi_t(i, j) = gamma_t(i));
 //     - start / trans / post accumulate in fp32 per lane (trans in shared memory, one column per lane), then in float64 per
@@ -55,7 +56,7 @@ __device__ __forceinline__ int de_tile_model(const int32_t *__restrict__ tile_st
 }
 
 struct DeSmem {   // byte offsets of the dynamic shared memory of k_dense_fb
-    size_t w, cst, lpi, piv, A, arcd, startd, arcs, starts, col, lcol, acc, total;
+    size_t w, cst, lpi, piv, A, arcd, startd, arcs, lg2s, starts, col, lcol, acc, total;
 };
 static DeSmem de_smem(int S, int nch) {
     DeSmem L;
@@ -69,6 +70,7 @@ static DeSmem de_smem(int S, int nch) {
     L.arcd = take((size_t)S * S * sizeof(float2));
     L.startd = take((size_t)(S + 1) * sizeof(int32_t));
     L.arcs = take((size_t)S * S * sizeof(float2));
+    L.lg2s = take((size_t)S * S * sizeof(float));
     L.starts = take((size_t)(S + 1) * sizeof(int32_t));
     L.col = take((size_t)S * 32 * sizeof(float));
     L.lcol = take((size_t)S * 32 * sizeof(float));
@@ -84,8 +86,9 @@ k_dense_fb(const float *__restrict__ X, int ldx, const int64_t *__restrict__ off
            const int32_t *__restrict__ model_start, const int32_t *__restrict__ tile_start, int M, int S, int nch, int k0,
            const float *__restrict__ piv_g, const float *__restrict__ w_g, const float *__restrict__ cst_g,
            const float *__restrict__ lpi_g, const float2 *__restrict__ arcd_g, const int32_t *__restrict__ startd_g,
-           const float2 *__restrict__ arcs_g, const int32_t *__restrict__ starts_g, DeSmem L, float *__restrict__ scr, int maxT,
-           float *__restrict__ gamma, double *__restrict__ part, int64_t plen, double *__restrict__ loglik) {
+           const float2 *__restrict__ arcs_g, const float *__restrict__ lg2s_g, const int32_t *__restrict__ starts_g, DeSmem L,
+           float *__restrict__ scr, int maxT, float *__restrict__ gamma, double *__restrict__ part, int64_t plen,
+           double *__restrict__ loglik) {
     const int tile = k0 + blockIdx.x;
     if (tile >= tile_start[M]) return;
     const int m = de_tile_model(tile_start, M, tile), lane = threadIdx.x;
@@ -98,6 +101,7 @@ k_dense_fb(const float *__restrict__ X, int ldx, const int64_t *__restrict__ off
     float2 *sarcd = reinterpret_cast<float2 *>(s_de + L.arcd);
     int32_t *sstartd = reinterpret_cast<int32_t *>(s_de + L.startd);
     float2 *sarcs = reinterpret_cast<float2 *>(s_de + L.arcs);
+    float *slg2s = reinterpret_cast<float *>(s_de + L.lg2s);                      // log2 A of sarcs[k], from float64
     int32_t *sstarts = reinterpret_cast<int32_t *>(s_de + L.starts);
     float *col = reinterpret_cast<float *>(s_de + L.col) + lane;                 // col[j * 32]: this lane's state vector
     float *lcol = reinterpret_cast<float *>(s_de + L.lcol) + lane;               // the same in log2 units
@@ -106,7 +110,10 @@ k_dense_fb(const float *__restrict__ X, int ldx, const int64_t *__restrict__ off
     for (int i = lane; i < nch * S * 8; i += 32) sw[i] = w_g[(size_t)m * nch * S * 8 + i];
     for (int i = lane; i < S; i += 32) { scst[i] = cst_g[(size_t)m * S + i]; slpi[i] = lpi_g[(size_t)m * S + i] * DE_LOG2E; }
     for (int i = lane; i < nch; i += 32) spiv[i] = reinterpret_cast<const float4 *>(piv_g)[i];
-    for (int i = lane; i < S * S; i += 32) { sA[i] = 0.f; sarcd[i] = arcd_g[(size_t)m * S * S + i]; sarcs[i] = arcs_g[(size_t)m * S * S + i]; }
+    for (int i = lane; i < S * S; i += 32) {
+        sA[i] = 0.f; sarcd[i] = arcd_g[(size_t)m * S * S + i]; sarcs[i] = arcs_g[(size_t)m * S * S + i];
+        slg2s[i] = lg2s_g[(size_t)m * S * S + i];
+    }
     for (int i = lane; i <= S; i += 32) { sstartd[i] = startd_g[(size_t)m * (S + 1) + i]; sstarts[i] = starts_g[(size_t)m * (S + 1) + i]; }
     for (int i = lane; i < nacc * 32; i += 32) acc[i] = 0.f;
     __syncwarp();
@@ -201,10 +208,10 @@ k_dense_fb(const float *__restrict__ X, int ldx, const int64_t *__restrict__ off
                         lb[i] = de_lg2(r);                  // log2 bhat_t(i) = log2 r(i)
                     } else {                                // the successors' mass is (near) underflow: log domain
                         float mx = NINF;
-                        for (int k = k0; k < k1; k++) mx = fmaxf(mx, de_lg2(sarcs[k].x) + lcol[(int)sarcs[k].y * 32]);
+                        for (int k = k0; k < k1; k++) mx = fmaxf(mx, slg2s[k] + lcol[(int)sarcs[k].y * 32]);
                         float s2 = 0.f;
                         if (mx > NINF)
-                            for (int k = k0; k < k1; k++) s2 += de_ex2(de_lg2(sarcs[k].x) + lcol[(int)sarcs[k].y * 32] - mx);
+                            for (int k = k0; k < k1; k++) s2 += de_ex2(slg2s[k] + lcol[(int)sarcs[k].y * 32] - mx);
                         lb[i] = (mx > NINF) ? mx + de_lg2(s2) : NINF;
                         redo |= 1u << i;
                     }
@@ -240,7 +247,7 @@ k_dense_fb(const float *__restrict__ X, int ldx, const int64_t *__restrict__ off
                         }
                     } else {                                   // A_ij q(j) / r(i) in the log domain
                         for (int k = k0; k < k1; k++)
-                            xi[k * 32] += g * de_ex2(de_lg2(sarcs[k].x) + lcol[(int)sarcs[k].y * 32] - lb[i]);
+                            xi[k * 32] += g * de_ex2(slg2s[k] + lcol[(int)sarcs[k].y * 32] - lb[i]);
                     }
                 }
             }
@@ -351,8 +358,8 @@ static int dense_estep_fp32(sapr_ctx *ctx, sapr_models *m, const float *X, int l
         ProfScope ps(ctx, 9);
         kern<<<nk, 32, L.total, ctx->stream>>>(X, ldx, offsets, order, model_start, tile_start, M, S, nch, k0, m->dn_piv, m->dn_w,
                                                m->dn_cst, m->dn_lpi, (const float2 *)m->dn_arc, m->dn_start,
-                                               (const float2 *)m->dn_arcs, m->dn_starts, L, (float *)ctx->ws[0], max_T, gamma, part,
-                                               plen, loglik);
+                                               (const float2 *)m->dn_arcs, m->dn_lg2s, m->dn_starts, L, (float *)ctx->ws[0], max_T,
+                                               gamma, part, plen, loglik);
         SAPR_LAUNCH_CHECK(ctx);
     }
     {
@@ -464,6 +471,13 @@ int sapr_estep_dense(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, con
     if (precision != SAPR_FP64 && precision != SAPR_FP32) SAPR_FAIL(ctx, SAPR_E_INVALID, "estep (dense): bad precision");
     if (precision == SAPR_FP32 && (m->S > 32 || !m->dn_w))
         SAPR_FAIL(ctx, SAPR_E_RANGE, "estep (dense): S > 32 states in SAPR_FP32 (SAPR_FP64 runs sapr_hl_estep per model)");
+    if (precision == SAPR_FP32) {   // one model's parameters, arc lists and per-lane accumulators in one CTA's shared memory
+        int smem_max = 0;
+        SAPR_CUDA(ctx, cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
+        if (de_smem(m->S, m->Dp / 4).total > (size_t)smem_max)
+            SAPR_FAIL(ctx, SAPR_E_RANGE, "estep (dense): S and D too large for SAPR_FP32's shared memory (SAPR_FP64 runs "
+                                         "sapr_hl_estep per model)");
+    }
     if (precision == SAPR_FP64 && m->S > 1024) SAPR_FAIL(ctx, SAPR_E_RANGE, "estep (dense): more than 1024 states");
     const int M = m->M;
     SAPR_CUDA(ctx, cudaMemsetAsync(stats, 0, sizeof(double) * (size_t)M * sapr_hl_stats_len(m->S, m->D), ctx->stream));
