@@ -98,6 +98,12 @@ int sapr_init_stats(sapr_ctx *ctx, const float *X, int ldx, const int64_t *offse
  * SAPR_FP64 equals sapr_hl_decode per model bit for bit; SAPR_FP32 is the fused fp32 kernel (csrc/viterbi_dense.cu) with the
  * near-tie pass below.  DENSE sets refuse first_frames > 0, all_paths and model_of_utt (SAPR_E_INVALID); max_T must cover the
  * longest utterance.
+ * DIAG emission + ENTRY_EXIT topology: N <= 31 (else SAPR_E_RANGE).  One model's packed parameters take (D+3)/4 * N * 64 B in
+ * SAPR_FP64 and half that in fp32; the all-models call stages up to 16 of them per CTA, fewer when they do not fit 227 KB, and
+ * model_of_utt stages all M (M <= 45 float64 / 90 fp32 models at N = 8, D = 39); a shape that does not fit is SAPR_E_RANGE before
+ * any launch.  SAPR_FP32 takes the tensor-core kernels for N = 8, M <= 12, D <= 47 when every emitting state's self-loop is
+ * non-zero (the tensor-core image folds ln A[j][j] into the emission; re-checked after every sapr_models_set / sapr_mstep), and
+ * the SIMT kernel (as SAPR_FP32_SIMT) otherwise.
  *   model_of_utt  int32[B] or NULL; NULL = score against all M models
  *   max_T         the longest utterance of the batch; it sizes the scratch, and an utterance longer than max_T is decoded
  *                 on its first max_T frames only (never past the scratch)
@@ -116,7 +122,9 @@ int sapr_viterbi(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, const i
  * call (word, score, score row and path then are the verification mode's), so the recognised word equals the float64 one
  * except on exact float64 ties (decoder.py:42-47 keeps the first).  n = utterances flagged by the last sapr_viterbi or
  * sapr_score_words call on this context
- * (synchronises the stream); at most 8192 per 1 GB scratch chunk are re-decoded.  SAPR_EXACT_WORDS=0 disables the pass.
+ * (synchronises the stream); the first 8192 flagged utterances of each 1 GB back-pointer chunk are re-decoded, at any length
+ * (utterances whose emissions exceed the shared-memory staging use a global-memory scratch).  ENTRY_EXIT sets have this pass on
+ * the tensor-core kernels only; the SIMT fp32 kernel keeps its fp32 words.  SAPR_EXACT_WORDS=0 disables the pass.
  * Stream order: part of an equal-length batch's arg-max / back-trace may run on a context-owned auxiliary stream beside the
  * last launch of the main kernel; it is joined back into the context's stream before the call returns, so work the caller
  * enqueues on that stream afterwards sees every output. */
@@ -142,7 +150,11 @@ int sapr_viterbi_host(sapr_ctx *ctx, sapr_models *m, const float *X_host, int ld
  *           G[S] = sum gamma[:-1] | Xi[S] = sum xi(j,j) | occ[S] | sum gamma (x-mu_old) [S*D] |
  *           sum gamma (x-mu_old)^2 [S*D]
  *   loglik  float64[B]  logsumexp(alpha_scaled[T-1,:]) as the reference reports it (SURVEY D6)
- *   gamma_out float32/float64 [sum_T * N] nullable debug output (emitting states only)            */
+ *   gamma_out float32/float64 [sum_T * N] nullable debug output (emitting states only)
+ * Range: N <= 31, D <= 256.  Off the tensor-core path (SAPR_FP64, and SAPR_FP32 outside N = 8, M <= 12, D <= 47 or with a zero
+ * emitting self-loop) one CTA stages every model: M * ((D+3)/4 * N * 64 + 16) B in float64, half in fp32, within 227 KB (M <= 45
+ * float64 / 90 fp32 at N = 8, D = 39); the statistics kernel keeps 8 * 4 * 2 * N * (D+3)/4*4 B (D <= 116 at N = 31).  A shape
+ * outside these is SAPR_E_RANGE before any launch. */
 /* DIAG emission + DENSE topology (hmmlearn GaussianHMM.fit's E-step, every model at once): model_of_utt is required (NULL =
  * SAPR_E_INVALID), order as above.  stats float64[M * sapr_hl_stats_len(S, D)], zeroed by the call, per model
  * [start S | trans S*S | post S | obs S*D | obs2 S*D] as sapr_hl_estep gives it; loglik = log P(X_u); gamma_out [sum_T][S]

@@ -311,6 +311,12 @@ int sapr_models_prepare(sapr_models *m) {
         if (m->tc_image) {
             int rc = sapr_tc_prepare(m);
             if (rc) return rc;
+            std::vector<double> la((size_t)M * S);
+            SAPR_CUDA(ctx, cudaMemcpyAsync(la.data(), m->la64, sizeof(double) * la.size(), cudaMemcpyDeviceToHost, ctx->stream));
+            SAPR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+            m->tc_loops_finite = true;
+            for (int i = 0; i < M; i++)
+                for (int j = 1; j <= m->N; j++) m->tc_loops_finite &= la[(size_t)i * S + j] > -INFINITY;
         }
         if (m->dn_w) {
             int rc = sapr_dense_prepare(m);

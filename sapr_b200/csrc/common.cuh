@@ -38,7 +38,7 @@ struct sapr_ctx {
     std::vector<ProfRec> prof;       // used records
     std::vector<ProfRec> prof_pool;  // recycled event pairs
     bool flag_valid = false;         // ws[8] holds the flag counters of the last fp32 Viterbi or word-scoring call (sapr_viterbi_flagged)
-    int flag_maxT = 0, flag_M = 0;   // longest utterance / models of that call (size the re-decoding scratch)
+    int flag_maxT = 0;               // longest utterance of that call (sizes the float64 re-decoding)
 };
 
 // RAII bracket: records an event pair around one kernel launch when profiling is on
@@ -88,6 +88,9 @@ struct sapr_models {
     // tensor-core Viterbi image (viterbi_tc.cu): fp16 hi/lo weights in shared-memory layout + (g, s) + transitions
     void *tc_image = nullptr;
     int tc_ctas_per_sm = 1;
+    // every emitting state's self-loop is non-zero (refreshed by sapr_models_prepare): the image folds ln A[j][j] into the emission
+    // constant, so a zero self-loop would make that state's emission NaN; such sets take the SIMT fp32 kernels
+    bool tc_loops_finite = false;
     // DENSE + DIAG sets with S <= 32 (viterbi_dense.cu): pivot p[Dp]; per model [chunk][state][8] = (a x4, b x4) with
     // a = (mu - p) / var, b = -1 / (2 var); cst[S] = -0.5 (D ln 2pi + sum ln var + sum (mu - p)^2 / var); ln pi [S];
     // finite arcs (ln A, source) grouped by destination [S*S] float2 with start[S + 1]; the same arcs (A, destination) grouped
@@ -128,7 +131,7 @@ struct sapr_models {
 // listed (arg-max kernels) and re-decoded in float64 (sapr_viterbi_redo_flagged), so the recognised word is the float64 one
 struct SaprFlag {
     int32_t *list = nullptr;    // [cap] utterance indices
-    int32_t *count = nullptr;   // [0] entries of this chunk (may exceed cap: the surplus is not re-decoded), [1] running total of the call
+    int32_t *count = nullptr;   // [0] entries of this chunk (may exceed cap: the surplus is not listed), [1] running total of the call
     int32_t *done = nullptr;    // [SAPR_FLAG_CAP] models completed per list entry (k_redo_fused; zero between launches)
     int cap = 0;
     float rel = 0.f;
@@ -146,7 +149,7 @@ __device__ __forceinline__ void sapr_flag_word(const SaprFlag &f, int u, double 
 #define SAPR_FLAG_CAP 8192
 #define SAPR_FLAG_REL 8e-6f
 int sapr_viterbi_redo_flagged(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, const int64_t *offsets, int first_frames,
-                              const SaprFlag &flag, int32_t *best_word, double *best_score, double *scores, uint8_t *best_path);
+                              int nu, const SaprFlag &flag, int32_t *best_word, double *best_score, double *scores, uint8_t *best_path);
 int sapr_flag_setup(sapr_ctx *ctx, SaprFlag *flag, bool first_chunk);   // workspace slot 8; zeroes the per-chunk counter
 int sapr_ws_reserve(sapr_ctx *ctx, int slot, size_t bytes);   // grows ctx->ws[slot]
 int sapr_pin_reserve(sapr_ctx *ctx, int slot, size_t bytes);  // grows ctx->pin[slot]
@@ -156,7 +159,8 @@ int sapr_viterbi_dense(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, c
                        int max_T, const int32_t *model_of_utt, int precision, int first_frames, int32_t *best_word, double *best_score,
                        double *scores, uint8_t *best_path, uint8_t *all_paths);
 // float64 emission matrix E[total_frames][S] of model mi for a batch (DIAG or SAPR emission)
-bool sapr_tc_eligible(const sapr_models *m);
+bool sapr_tc_eligible(const sapr_models *m);    // shape only: whether the set has a tensor-core image
+bool sapr_tc_usable(const sapr_models *m);      // the image exists and every emitting self-loop is non-zero
 size_t sapr_tc_image_bytes(const sapr_models *m, int *nck_out, int *ncols_out);
 int sapr_tc_prepare(sapr_models *m);
 int sapr_viterbi_tc_launch(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, const int64_t *offsets, int B,

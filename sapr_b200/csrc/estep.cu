@@ -139,6 +139,7 @@ k_estep_fused(const float *__restrict__ X, int ldx, const int64_t *__restrict__ 
     }
     // reported log-likelihood (SURVEY D6): logaddexp.reduce(alpha[T-1, :]) - max(alpha)
     bool xi_live = true;
+    double xi_lsum = 0.0;      // ln of the reference's per-frame sum of un-normalised xi, before the scale term (see below)
     if (T > 0) {
         R r = (T == 1) ? R(0) : NINF;                  // alpha[T-1, entry]
 #pragma unroll
@@ -151,6 +152,7 @@ k_estep_fused(const float *__restrict__ X, int ldx, const int64_t *__restrict__ 
         // ax - r < ln(2^-1075) every arc underflows to 0 in float64, the `if np.sum(xi[t]) > 0` guard (:319) skips the
         // normalisation and the utterance adds nothing to the transition statistics.
         xi_live = !((double)ax - (double)r < -745.13);
+        xi_lsum = (double)ax - (double)r;
     }
 
     // ---------------- backward + gamma + xi (custom_hmm.py:213-322) ----------------
@@ -202,6 +204,23 @@ k_estep_fused(const float *__restrict__ X, int ldx, const int64_t *__restrict__ 
         for (int j = 0; j < NMAX; j++)
             if (j < N) xn = lae(xn, (j < N - 1) ? lg[j] : at[j] + self[j]);
         R *go = gamma_out ? gamma_out + (size_t)(off + t) * N : nullptr;
+        // float64: the reference's un-normalised xi of an arc is its normalised value times exp(L), L = ax - r less the forward
+        // scale max(alpha) on the frames whose beta it shifts (custom_hmm.py:241-246, :270-320).  For L below ~ -700 the arcs are
+        // subnormal or flushed to 0 in its arithmetic and the per-frame normalisation divides those rounded values, so they are
+        // formed the same way here; above, every arc is exact to 1e-16 and the log-domain ratio is used.
+        const double L = xi_lsum - ((t + 1 < T - 1) ? amax : 0.0);
+        const bool sub_xi = sizeof(R) == 8 && L < -700.0 && !anan && xn > NINF;
+        double xsum = 0.0;
+        if (sub_xi) {
+            const double sh = L - (double)xn;
+            if (t == 0) xsum += exp((double)b0 + sh);
+#pragma unroll
+            for (int j = 0; j < NMAX; j++)
+                if (j < N) {
+                    xsum += exp((double)(at[j] + self[j]) + sh);
+                    if (j < N - 1) xsum += exp((double)(at[j] + lb[j + 1] + w[j + 1]) + sh);
+                }
+        }
 #pragma unroll
         for (int j = 0; j < NMAX; j++) {
             if (j < N) {
@@ -209,7 +228,9 @@ k_estep_fused(const float *__restrict__ X, int ldx, const int64_t *__restrict__ 
                 gG[j] += g; gO[j] += g;
                 if (go) go[j] = g;
                 R xs = at[j] + self[j];
-                if (xi_live && xn > NINF && xs > NINF) gX[j] += fexp(xs - xn);
+                if (sub_xi) {
+                    if (xsum > 0.0) gX[j] += (R)(exp((double)xs + (L - (double)xn)) / xsum);     // the `sum > 0` guard (:319)
+                } else if (xi_live && xn > NINF && xs > NINF) gX[j] += fexp(xs - xn);
             }
         }
         // next beta, renormalised (offsets cancel in gamma / xi, so they are not kept)
@@ -281,7 +302,7 @@ __device__ __forceinline__ int find_tile(const int32_t *model_start, int M, int 
     return -1;
 }
 
-// blockDim = (Dp, STATS_SLOTS).  partial[tile][2][N][Dp] float64.
+// blockDim = (Dp or fewer dims, STATS_SLOTS).  partial[tile][2][N][Dp] float64.
 template <typename R, int NMAX>
 __global__ void k_stats_diag(const float *__restrict__ X, int ldx, const int64_t *__restrict__ offsets,
                              const int32_t *__restrict__ order, const int32_t *__restrict__ model_start, int M, int N,
@@ -291,58 +312,64 @@ __global__ void k_stats_diag(const float *__restrict__ X, int ldx, const int64_t
     if (threadIdx.x == 0 && threadIdx.y == 0) s_m = find_tile(model_start, M, upc, blockIdx.x, &s_tim);
     __syncthreads();
     const int m = s_m;
-    const int d = threadIdx.x, slot = threadIdx.y;
+    const int slot = threadIdx.y;
     double *out = partial + (size_t)blockIdx.x * 2 * N * Dp;
     extern __shared__ double s_red[];   // [STATS_SLOTS][2][N][Dp]
-    double a1[NMAX], a2[NMAX];
+    // blockDim.x may be below Dp (the NMAX 16 / 31 instances use too many registers for Dp x STATS_SLOTS threads): dims in rounds
+    for (int d0 = 0; d0 < Dp; d0 += blockDim.x) {
+        const int d = d0 + threadIdx.x;
+        const bool live = d < Dp;
+        double a1[NMAX], a2[NMAX];
 #pragma unroll
-    for (int j = 0; j < NMAX; j++) { a1[j] = 0.0; a2[j] = 0.0; }
-    if (m >= 0) {
-        R c[NMAX];
+        for (int j = 0; j < NMAX; j++) { a1[j] = 0.0; a2[j] = 0.0; }
+        if (m >= 0) {
+            R c[NMAX];
 #pragma unroll
-        for (int j = 0; j < NMAX; j++) c[j] = (j < N && d < D) ? (R)mean[((size_t)m * S + j + 1) * D + d] : R(0);
-        const int pbeg = model_start[m] + s_tim * upc;
-        const int pend = min(pbeg + upc, model_start[m + 1]);
-        for (int p = pbeg; p < pend; p++) {
-            const int u = order[p];
-            const int64_t off = offsets[u];
-            const int T = (int)(offsets[u + 1] - off);
-            R f1[NMAX], f2[NMAX];
+            for (int j = 0; j < NMAX; j++) c[j] = (j < N && d < D) ? (R)mean[((size_t)m * S + j + 1) * D + d] : R(0);
+            const int pbeg = model_start[m] + s_tim * upc;
+            const int pend = min(pbeg + upc, model_start[m + 1]);
+            for (int p = pbeg; p < pend; p++) {
+                const int u = order[p];
+                const int64_t off = offsets[u];
+                const int T = (int)(offsets[u + 1] - off);
+                R f1[NMAX], f2[NMAX];
 #pragma unroll
-            for (int j = 0; j < NMAX; j++) { f1[j] = R(0); f2[j] = R(0); }
-            for (int t = slot; t < T; t += STATS_SLOTS) {
-                const R x = (d < D) ? (R)__ldg(X + (size_t)(off + t) * ldx + d) : R(0);
-                const R *g = gamma + (size_t)(off + t) * N;
+                for (int j = 0; j < NMAX; j++) { f1[j] = R(0); f2[j] = R(0); }
+                for (int t = slot; t < T; t += STATS_SLOTS) {
+                    const R x = (d < D) ? (R)__ldg(X + (size_t)(off + t) * ldx + d) : R(0);
+                    const R *g = gamma + (size_t)(off + t) * N;
 #pragma unroll
-                for (int j = 0; j < NMAX; j++) {
-                    if (j < N) {
-                        R gj = __ldg(g + j);
-                        R xc = x - c[j];
-                        R gx = gj * xc;
-                        f1[j] += gx;
-                        f2[j] = fma(gx, xc, f2[j]);
+                    for (int j = 0; j < NMAX; j++) {
+                        if (j < N) {
+                            R gj = __ldg(g + j);
+                            R xc = x - c[j];
+                            R gx = gj * xc;
+                            f1[j] += gx;
+                            f2[j] = fma(gx, xc, f2[j]);
+                        }
                     }
                 }
-            }
 #pragma unroll
-            for (int j = 0; j < NMAX; j++) { a1[j] += (double)f1[j]; a2[j] += (double)f2[j]; }
-        }
-    }
-    // fixed-order reduction over the frame slots
-#pragma unroll
-    for (int j = 0; j < NMAX; j++)
-        if (j < N) {
-            s_red[((size_t)(slot * 2 + 0) * N + j) * Dp + d] = a1[j];
-            s_red[((size_t)(slot * 2 + 1) * N + j) * Dp + d] = a2[j];
-        }
-    __syncthreads();
-    if (slot == 0) {
-        for (int k = 0; k < 2; k++)
-            for (int j = 0; j < N; j++) {
-                double s = 0.0;
-                for (int sl = 0; sl < STATS_SLOTS; sl++) s += s_red[((size_t)(sl * 2 + k) * N + j) * Dp + d];
-                out[((size_t)k * N + j) * Dp + d] = s;
+                for (int j = 0; j < NMAX; j++) { a1[j] += (double)f1[j]; a2[j] += (double)f2[j]; }
             }
+        }
+        // fixed-order reduction over the frame slots
+#pragma unroll
+        for (int j = 0; j < NMAX; j++)
+            if (j < N && live) {
+                s_red[((size_t)(slot * 2 + 0) * N + j) * Dp + d] = a1[j];
+                s_red[((size_t)(slot * 2 + 1) * N + j) * Dp + d] = a2[j];
+            }
+        __syncthreads();
+        if (slot == 0 && live) {
+            for (int k = 0; k < 2; k++)
+                for (int j = 0; j < N; j++) {
+                    double s = 0.0;
+                    for (int sl = 0; sl < STATS_SLOTS; sl++) s += s_red[((size_t)(sl * 2 + k) * N + j) * Dp + d];
+                    out[((size_t)k * N + j) * Dp + d] = s;
+                }
+        }
+        __syncthreads();
     }
 }
 
@@ -643,6 +670,19 @@ static int launch_estep(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, 
     const int N = m->N, M = m->M, D = m->D, Dp = m->Dp, S = m->S, nchunk = Dp / 4;
     const int64_t stride = sapr_stats_stride(N, D);
     int rc;
+    // shapes whose shared memory does not fit are refused before the first launch
+    const bool use_tc = std::is_same<R, float>::value && sapr_tc_usable(m);
+    const size_t smem = (size_t)M * model_stride<R>((size_t)nchunk * N * 8) * sizeof(R);
+    if (!use_tc && smem > 227 * 1024)
+        SAPR_FAIL(ctx, SAPR_E_RANGE, "estep: the model set does not fit in shared memory (the E-step stages every model)");
+    const int upc = std::max(8, std::min(256, B / (4 * ctx->sm_count)));
+    const int ncons = (Dp / 4) * 2 * STATS2_SLOTS;
+    const size_t ssm2 = std::max(sizeof(float) * STATS2_SLOTS * (2 * N * Dp + N), (size_t)STATS2_STAGES * STATS2_CF * (ldx * 4 + 32));
+    const bool use_stats8 = std::is_same<R, float>::value && N == 8 && ssm2 <= 227 * 1024 && ncons <= 640 && ncons % 32 == 0 &&
+                            upc <= STATS2_MAXUPC;
+    const size_t ssm = sizeof(double) * STATS_SLOTS * 2 * N * Dp;
+    if (!use_stats8 && ssm > 227 * 1024)
+        SAPR_FAIL(ctx, SAPR_E_RANGE, "estep: the feature statistics of N states x D dims do not fit in shared memory");
     // grouping
     if ((rc = sapr_ws_reserve(ctx, 2, sizeof(int32_t) * ((size_t)B + M + 2)))) return rc;
     int32_t *order_ws = (int32_t *)ctx->ws[2];
@@ -661,12 +701,10 @@ static int launch_estep(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, 
         if ((rc = sapr_ws_reserve(ctx, 3, sizeof(R) * (size_t)total_frames * N))) return rc;
         gamma = (R *)ctx->ws[3];
     }
-    const int upc = std::max(8, std::min(256, B / (4 * ctx->sm_count)));
     const int ntile_max = (B + upc - 1) / upc + M;
     if ((rc = sapr_ws_reserve(ctx, 4, sizeof(double) * (size_t)ntile_max * 2 * N * Dp))) return rc;
     double *partial = (double *)ctx->ws[4];
-    bool tc_done = false;
-    if (std::is_same<R, float>::value && m->tc_image && sapr_tc_eligible(m)) {
+    if (use_tc) {
         // production fp32 path: emission on the tensor cores, forward and backward sweep of a tile in one persistent CTA
         if ((rc = sapr_ws_reserve(ctx, 1, sizeof(float) * (size_t)B * 3 * N))) return rc;
         if ((rc = sapr_estep_tc_launch(ctx, m, X, ldx, offsets, B, max_T, order, model_start, (float *)gamma,
@@ -675,9 +713,7 @@ static int launch_estep(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, 
         k_reduce_triples<float><<<dim3(3 * N, M), 256, 0, ctx->stream>>>(model_start, N, S, (const float *)ctx->ws[1], 0, B,
                                                                          stats, stride);
         SAPR_LAUNCH_CHECK(ctx);
-        tc_done = true;
-    }
-    if (!tc_done) {
+    } else {
     // forward/backward lattice scratch, chunked over pairs so it stays bounded (<= ~1 GB)
     const size_t per_pair = (size_t)max_T * N * sizeof(R) * 2;
     int chunk = (int)std::min<int64_t>(B, std::max<int64_t>(128, ((int64_t)1 << 30) / (int64_t)per_pair));
@@ -693,8 +729,6 @@ static int launch_estep(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, 
     const R *la = std::is_same<R, float>::value ? (const R *)m->la32 : (const R *)m->la64;
     const R *lb = std::is_same<R, float>::value ? (const R *)m->lb32 : (const R *)m->lb64;
     auto kern = k_estep_fused<R, NMAX, std::is_same<R, float>::value>;
-    size_t smem = (size_t)M * model_stride<R>((size_t)nchunk * N * 8) * sizeof(R);
-    if (smem > 227 * 1024) SAPR_FAIL(ctx, SAPR_E_RANGE, "estep: model set does not fit in shared memory");
     SAPR_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     for (int p0 = 0; p0 < B; p0 += chunk) {
         const int np = std::min(chunk, B - p0);
@@ -712,27 +746,25 @@ static int launch_estep(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, 
     }
     // feature statistics over the whole batch
     const int ntiles = ntile_max;
-    if (std::is_same<R, float>::value && N == 8) {
-        const int ncons = (Dp / 4) * 2 * STATS2_SLOTS;
+    if (use_stats8) {
         dim3 sb2(ncons + 32);                          // + the producer warp
-        const size_t ssm2 = std::max(sizeof(float) * STATS2_SLOTS * (2 * N * Dp + N), (size_t)STATS2_STAGES * STATS2_CF * (ldx * 4 + 32));
-        if (ssm2 <= 227 * 1024 && ncons <= 640 && ncons % 32 == 0 && upc <= STATS2_MAXUPC) {
-            SAPR_CUDA(ctx, cudaFuncSetAttribute(k_stats_diag8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ssm2));
-            {
-                ProfScope ps(ctx, 3);
-                k_stats_diag8<<<ntiles, sb2, ssm2, ctx->stream>>>(X, ldx, offsets, order, model_start, M, D, Dp, S, upc, m->mean,
-                                                                  (const float *)gamma, partial);
-            }
-            SAPR_LAUNCH_CHECK(ctx);
-            k_reduce_partials<<<(M * 2 * N * D + 127) / 128, 128, 0, ctx->stream>>>(model_start, M, N, D, Dp, S, upc, partial,
-                                                                                    stats, stride);
-            SAPR_LAUNCH_CHECK(ctx);
-            return SAPR_OK;
+        SAPR_CUDA(ctx, cudaFuncSetAttribute(k_stats_diag8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ssm2));
+        {
+            ProfScope ps(ctx, 3);
+            k_stats_diag8<<<ntiles, sb2, ssm2, ctx->stream>>>(X, ldx, offsets, order, model_start, M, D, Dp, S, upc, m->mean,
+                                                              (const float *)gamma, partial);
         }
+        SAPR_LAUNCH_CHECK(ctx);
+        k_reduce_partials<<<(M * 2 * N * D + 127) / 128, 128, 0, ctx->stream>>>(model_start, M, N, D, Dp, S, upc, partial,
+                                                                                stats, stride);
+        SAPR_LAUNCH_CHECK(ctx);
+        return SAPR_OK;
     }
-    dim3 sb(Dp, STATS_SLOTS);
-    size_t ssm = sizeof(double) * STATS_SLOTS * 2 * N * Dp;
     auto skern = k_stats_diag<R, NMAX>;
+    cudaFuncAttributes fa;
+    SAPR_CUDA(ctx, cudaFuncGetAttributes(&fa, skern));
+    const int bx = Dp * STATS_SLOTS <= fa.maxThreadsPerBlock ? Dp : fa.maxThreadsPerBlock / STATS_SLOTS / 32 * 32;
+    dim3 sb(bx, STATS_SLOTS);
     SAPR_CUDA(ctx, cudaFuncSetAttribute(skern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ssm));
     {
         ProfScope ps(ctx, 3);

@@ -310,7 +310,6 @@ static int score_fp32(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, co
     const bool exact = !ex_env || ex_env[0] != '0';
     SaprFlag flag;
     if (exact) {
-        ctx->flag_maxT = 0; ctx->flag_M = M;            // the re-scoring keeps one score per model and entry, no per-frame scratch
         if ((rc = sapr_flag_setup(ctx, &flag, true))) return rc;
     }
     {

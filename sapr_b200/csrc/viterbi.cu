@@ -280,7 +280,10 @@ k_viterbi_finish_fast(const int64_t *__restrict__ offsets, int u0, int nu, int N
 #pragma unroll
         for (int j = CH - 1; j >= 0; j--) {
             sp[w][lane][j] = (uint8_t)(reachable ? cur : (t0 + j == Te - 1 ? S - 1 : 0));
-            cur -= (int)(((bits[j] << 1) >> cur) & 1u);
+            if (sizeof(BP) == 4)      // N = 31: the exit's bit is bit 31, shifted out of a 32-bit word
+                cur -= (int)((((unsigned long long)bits[j] << 1) >> cur) & 1u);
+            else
+                cur -= (int)(((bits[j] << 1) >> cur) & 1u);
         }
         __syncwarp();
         for (int row = 0; row < 32; row++) {
@@ -332,11 +335,16 @@ static int launch_viterbi(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx
     if (rc) return rc;
     BP *bp = (BP *)ctx->ws[0];
     double *sc_ws = (double *)ctx->ws[1];
-    const int mpc = own ? 1 : std::min(m->M, 16);
+    // all-models mode stages the models of its CTA (up to 16, fewer when they do not fit); own-model mode stages every model
+    const size_t per_model = (size_t)nchunk * m->N * 8 * sizeof(R);
+    int mpc = own ? 1 : std::min(m->M, 16);
+    while (!own && mpc > 1 && mpc * per_model > 227 * 1024) mpc--;
     const int nm_stage = own ? m->M : mpc;
-    size_t smem = (size_t)nm_stage * nchunk * m->N * 8 * sizeof(R);
+    size_t smem = (size_t)nm_stage * per_model;
     auto kern = k_viterbi_fused<R, BP, NMAX, std::is_same<R, float>::value>;
-    if (smem > 227 * 1024) SAPR_FAIL(ctx, SAPR_E_RANGE, "viterbi: model set does not fit in shared memory");
+    if (smem > 227 * 1024)
+        SAPR_FAIL(ctx, SAPR_E_RANGE, own ? "viterbi: the own-model mode stages every model, and the model set does not fit in shared memory"
+                                         : "viterbi: one model does not fit in shared memory");
     SAPR_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const R *pk = std::is_same<R, float>::value ? (const R *)m->pk32 : (const R *)m->pk64;
     const R *cst = std::is_same<R, float>::value ? (const R *)m->cst32 : (const R *)m->cst64;
@@ -379,25 +387,36 @@ static int launch_viterbi(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx
 //      bit-identical to the verification mode's
 //   3. the block that completes an entry's last model (a counter per entry) takes the arg-max over the models and traces the
 //      winner's path, overwriting the entry's word, score, score row and path.
+//   GSE: the emissions and the back-trace words of an item live in a per-block global-memory scratch (gse, (maxT * 8 + 8)
+//   doubles + maxT * 3 bytes per block) instead of shared memory: utterances too long for the shared-memory staging.
+// One launch takes list entries [e0, e0 + seg): the back-pointer and score scratch hold seg entries.
+// Bytes of one block's global scratch, rounded up to 256 so that every block's double and uint16 arrays stay aligned.
+__host__ __device__ inline size_t redo_gse_stride(int maxT) {
+    return ((((size_t)maxT * 8 + 8) * sizeof(double) + (size_t)maxT * 3) + 255) / 256 * 256;
+}
+template <bool GSE>
 __global__ void __launch_bounds__(256) k_redo_fused(const float *__restrict__ X, int ldx, const int64_t *__restrict__ offsets,
-                                                    const int32_t *__restrict__ utt_list, const int32_t *__restrict__ utt_count, int cap, int M, int N,
+                                                    const int32_t *__restrict__ utt_list, const int32_t *__restrict__ utt_count, int e0, int seg, int M, int N,
                                                     int nchunk, int maxT, int xs, int first_frames, const double *__restrict__ pk,
                                                     const double *__restrict__ cst_g, const double *__restrict__ la_g, const double *__restrict__ lb_g,
                                                     uint16_t *bp, int64_t Bpad, double *sc, int32_t *done, int32_t *__restrict__ best_word,
-                                                    double *__restrict__ best_score, double *__restrict__ scores_out, uint8_t *__restrict__ best_path) {
+                                                    double *__restrict__ best_score, double *__restrict__ scores_out, uint8_t *__restrict__ best_path,
+                                                    unsigned char *gse) {
     extern __shared__ __align__(16) unsigned char s_rd[];
-    double *se = reinterpret_cast<double *>(s_rd);                                              // [maxT][8] + a zero slot
-    double2 *sp = reinterpret_cast<double2 *>(s_rd + ((size_t)maxT * 8 + 8) * sizeof(double));   // [nchunk][4 fields][8]
+    const size_t se_bytes = ((size_t)maxT * 8 + 8) * sizeof(double);
+    unsigned char *g_blk = GSE ? gse + (size_t)blockIdx.x * redo_gse_stride(maxT) : nullptr;
+    double *se = reinterpret_cast<double *>(GSE ? g_blk : s_rd);                                  // [maxT][8] + a zero slot
+    double2 *sp = reinterpret_cast<double2 *>(GSE ? s_rd : s_rd + se_bytes);                      // [nchunk][4 fields][8]
     unsigned char *s_x = reinterpret_cast<unsigned char *>(sp) + (size_t)nchunk * 8 * 64;
     float4 *sx = reinterpret_cast<float4 *>(s_x);                                               // [xs frames][nchunk]
-    uint16_t *sw = reinterpret_cast<uint16_t *>(s_x);                                           // step 3 reuses the feature slab
+    uint16_t *sw = reinterpret_cast<uint16_t *>(GSE ? g_blk + se_bytes : s_x);                  // step 3 reuses the feature slab
     uint8_t *spath = reinterpret_cast<uint8_t *>(sw + maxT);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, S = N + 2;
     const double NINF = -INFINITY;
-    const int n = min(*utt_count, cap);
+    const int n = min(min(*utt_count, SAPR_FLAG_CAP) - e0, seg);
     for (int w = blockIdx.x; w < n * M; w += gridDim.x) {
         const int pos = w / M, m = w % M;
-        const int u = utt_list[pos];
+        const int u = utt_list[e0 + pos];
         const int64_t off = offsets[u];
         const int T = (int)(offsets[u + 1] - off);
         const int Te = min((first_frames > 0 && first_frames < T) ? first_frames : T, maxT);
@@ -503,11 +522,11 @@ __global__ void __launch_bounds__(256) k_redo_fused(const float *__restrict__ X,
         __threadfence();
         __syncwarp();
         int last = 0;
-        if (lane == 0) last = atomicAdd(&done[pos], 1) == M - 1;
+        if (lane == 0) last = atomicAdd(&done[e0 + pos], 1) == M - 1;
         last = __shfl_sync(0xffffffffu, last, 0);
         if (!last) continue;
         __threadfence();
-        if (lane == 0) done[pos] = 0;                                        // ready for the next call
+        if (lane == 0) done[e0 + pos] = 0;                                      // ready for the next call
         double bs = NINF;
         int bslot = 0x7fffffff;
         for (int s0 = lane; s0 < M; s0 += 32) {
@@ -554,40 +573,56 @@ int sapr_flag_setup(sapr_ctx *ctx, SaprFlag *flag, bool first_chunk) {
     int32_t *base = (int32_t *)ctx->ws[8];
     if (fresh) SAPR_CUDA(ctx, cudaMemsetAsync(base, 0, need, ctx->stream));      // the counters are left at zero by every launch
     flag->done = base + 4 + SAPR_FLAG_CAP;
-    // list capacity: the re-decoding scratch (float64 emissions of every model and frame) stays below 256 MB
-    const int64_t per = (int64_t)std::max(ctx->flag_M, 1) * std::max(ctx->flag_maxT, 1) * 8 * (int64_t)sizeof(double);
-    flag->count = base; flag->list = base + 4; flag->rel = SAPR_FLAG_REL;
-    flag->cap = (int)std::max<int64_t>(32, std::min<int64_t>(SAPR_FLAG_CAP, ((int64_t)256 << 20) / per));
+    flag->count = base; flag->list = base + 4; flag->rel = SAPR_FLAG_REL; flag->cap = SAPR_FLAG_CAP;
     SAPR_CUDA(ctx, cudaMemsetAsync(base, 0, sizeof(int32_t) * (first_chunk ? 2 : 1), ctx->stream));
     ctx->flag_valid = true;
     return SAPR_OK;
 }
 
 // float64 re-decoding of the listed utterances on the context's stream, behind the fp32 arg-max / back-trace whose word, score,
-// score row and path it overwrites; the kernel reads the list length on the device (no host round trip)
+// score row and path it overwrites; the kernel reads the list length on the device (no host round trip).  Every listed entry
+// (up to SAPR_FLAG_CAP) is re-decoded: the back-pointer scratch holds seg entries (<= 256 MB), one launch per seg entries of the
+// chunk's possible list length min(nu, SAPR_FLAG_CAP); a launch past the actual list returns at once.  Utterances whose emissions do not fit the shared-memory staging are
+// re-decoded with a per-block global-memory emission scratch.
 int sapr_viterbi_redo_flagged(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, const int64_t *offsets, int first_frames,
-                              const SaprFlag &flag, int32_t *best_word, double *best_score, double *scores, uint8_t *best_path) {
+                              int nu, const SaprFlag &flag, int32_t *best_word, double *best_score, double *scores, uint8_t *best_path) {
     if (m->N > 8) return SAPR_OK;
     const int maxT = ctx->flag_maxT;
     const int Tm = (first_frames > 0 && first_frames < maxT) ? first_frames : maxT;
     const int Tq = Tm > 0 ? Tm : 1, nchunk = m->Dp / 4;
-    const int xs = std::min(Tq, 256);
+    int xs = std::min(Tq, 256);
+    const size_t se_bytes = ((size_t)Tq * 8 + 8) * sizeof(double);
     const size_t x_bytes = std::max((size_t)xs * nchunk * 16, ((size_t)Tq * 3 + 31) / 16 * 16);
-    const size_t smem = ((size_t)Tq * 8 + 8) * sizeof(double) + (size_t)nchunk * 8 * 64 + x_bytes;
-    if (smem > 220 * 1024) return SAPR_OK;      // utterances too long for the shared-memory emission staging: no re-decoding
-    const size_t bp_bytes = ((size_t)m->M * Tq * flag.cap * sizeof(uint16_t) + 255) / 256 * 256;
-    const size_t sc_bytes = ((size_t)flag.cap * m->M * sizeof(double) + 255) / 256 * 256;
-    int rc = sapr_ws_reserve(ctx, 4, bp_bytes + sc_bytes);
+    size_t smem = se_bytes + (size_t)nchunk * 8 * 64 + x_bytes;
+    const bool gse = smem > 220 * 1024;
+    if (gse) {
+        while (xs > 1 && (size_t)nchunk * 8 * 64 + (size_t)xs * nchunk * 16 > 220 * 1024) xs /= 2;
+        smem = (size_t)nchunk * 8 * 64 + (size_t)xs * nchunk * 16;
+    }
+    const int64_t per_entry = (int64_t)m->M * Tq * (int64_t)sizeof(uint16_t);
+    const int nlist = std::min(flag.cap, nu);                        // a chunk of nu utterances lists at most nu
+    const int seg = (int)std::max<int64_t>(1, std::min<int64_t>(nlist, ((int64_t)256 << 20) / per_entry));
+    const size_t bp_bytes = ((size_t)per_entry * seg + 255) / 256 * 256;
+    const size_t sc_bytes = ((size_t)seg * m->M * sizeof(double) + 255) / 256 * 256;
+    const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(4, (200 * 1024) / smem));
+    const int grid = (gse ? 1 : per_sm) * ctx->sm_count;
+    const size_t g_bytes = gse ? (size_t)grid * redo_gse_stride(Tq) : 0;
+    int rc = sapr_ws_reserve(ctx, 4, bp_bytes + sc_bytes + g_bytes);
     if (rc) return rc;
     uint16_t *bp = (uint16_t *)ctx->ws[4];
     double *sc = (double *)((char *)ctx->ws[4] + bp_bytes);
-    SAPR_CUDA(ctx, cudaFuncSetAttribute(k_redo_fused, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(4, (200 * 1024) / smem));
-    ProfScope ps(ctx, 6);
-    k_redo_fused<<<per_sm * ctx->sm_count, 256, smem, ctx->stream>>>(X, ldx, offsets, flag.list, flag.count, flag.cap, m->M, m->N, nchunk, Tq, xs,
-                                                                     first_frames, m->pk64, m->cst64, m->la64, m->lb64, bp, (int64_t)flag.cap, sc,
-                                                                     flag.done, best_word, best_score, scores, best_path);
-    SAPR_LAUNCH_CHECK(ctx);
+    unsigned char *gs = gse ? (unsigned char *)ctx->ws[4] + bp_bytes + sc_bytes : nullptr;
+    auto kern = gse ? k_redo_fused<true> : k_redo_fused<false>;
+    SAPR_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    for (int e0 = 0; e0 < nlist; e0 += seg) {
+        {
+            ProfScope ps(ctx, 6);
+            kern<<<grid, 256, smem, ctx->stream>>>(X, ldx, offsets, flag.list, flag.count, e0, seg, m->M, m->N, nchunk, Tq, xs,
+                                                   first_frames, m->pk64, m->cst64, m->la64, m->lb64, bp, (int64_t)seg, sc, flag.done,
+                                                   best_word, best_score, scores, best_path, gs);
+        }
+        SAPR_LAUNCH_CHECK(ctx);
+    }
     return SAPR_OK;
 }
 
@@ -607,7 +642,7 @@ extern "C" int sapr_viterbi_flagged(sapr_ctx *ctx, int64_t *n) {
 extern "C" int sapr_debug_tc_emission(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, const int64_t *offsets, int B,
                                       int64_t total_frames, int max_T, float *E_out, int *ncols_out) {
     if (!ctx || !m || !X || !offsets || !E_out) return SAPR_E_INVALID;
-    if (!m->valid || !m->tc_image || !sapr_tc_eligible(m)) SAPR_FAIL(ctx, SAPR_E_RANGE, "tc emission: model set not eligible");
+    if (!m->valid || !sapr_tc_usable(m)) SAPR_FAIL(ctx, SAPR_E_RANGE, "tc emission: model set not eligible");
     int ncols = 0;
     sapr_tc_image_bytes(m, nullptr, &ncols);
     if (ncols_out) *ncols_out = ncols;
@@ -633,7 +668,7 @@ extern "C" int sapr_viterbi(sapr_ctx *ctx, sapr_models *m, const float *X, int l
 #define GO(R, BP, NM)                                                                                       \
     return launch_viterbi<R, BP, NM>(ctx, m, X, ldx, offsets, B, total_frames, max_T, model_of_utt,        \
                                      first_frames, best_word, best_score, scores, best_path, all_paths)
-    if (precision == SAPR_FP32 && !model_of_utt && m->tc_image && sapr_tc_eligible(m))
+    if (precision == SAPR_FP32 && !model_of_utt && sapr_tc_usable(m))
         return sapr_viterbi_tc_launch(ctx, m, X, ldx, offsets, B, total_frames, max_T, first_frames, best_word, best_score,
                                       scores, best_path, all_paths, nullptr);
     if (precision == SAPR_FP32 || precision == SAPR_FP32_SIMT) {

@@ -418,7 +418,6 @@ static int dense_fp32(sapr_ctx *ctx, sapr_models *m, const float *X, int ldx, co
     const char *ex_env = getenv("SAPR_EXACT_WORDS");
     const bool exact = !ex_env || ex_env[0] != '0';
     SaprFlag flag;
-    ctx->flag_maxT = max_T; ctx->flag_M = M;
     for (int u0 = 0; u0 < B; u0 += chunk) {
         const int nu = std::min(chunk, B - u0);
         if (exact) {

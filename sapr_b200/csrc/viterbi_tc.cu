@@ -938,6 +938,8 @@ bool sapr_tc_eligible(const sapr_models *m) {
            m->D + 1 <= 48;
 }
 
+bool sapr_tc_usable(const sapr_models *m) { return m->tc_image && sapr_tc_eligible(m) && m->tc_loops_finite; }
+
 static void tc_geometry(const sapr_models *m, int *nck_out, int *ncols_out) {
     int nck = (m->D + 1 + 3) / 4;
     nck = (nck + 1) / 2 * 2;
@@ -1067,7 +1069,7 @@ int sapr_viterbi_tc_launch(sapr_ctx *ctx, sapr_models *m, const float *X, int ld
     const char *ex_env = getenv("SAPR_EXACT_WORDS");
     const bool exact = !dbgE && !all_paths && (!ex_env || ex_env[0] != '0');
     SaprFlag flag;
-    ctx->flag_maxT = max_T; ctx->flag_M = m->M;
+    ctx->flag_maxT = max_T;
     for (int u0 = 0; u0 < B; u0 += chunk) {
         const int nu = std::min(chunk, B - u0);
         if (exact && (rc = sapr_flag_setup(ctx, &flag, u0 == 0))) return rc;
@@ -1140,7 +1142,7 @@ int sapr_viterbi_tc_launch(sapr_ctx *ctx, sapr_models *m, const float *X, int ld
         if ((rc = sapr_viterbi_finish_u16(ctx, offsets, u0, nu, m->N, M, first_frames, bp, Bpad, Tm, sc_ws, best_word, best_score,
                                           scores, M, best_path, all_paths, total_frames, exact ? &flag : nullptr)))
             return rc;
-        if (exact && (rc = sapr_viterbi_redo_flagged(ctx, m, X, ldx, offsets, first_frames, flag, best_word, best_score, scores, best_path)))
+        if (exact && (rc = sapr_viterbi_redo_flagged(ctx, m, X, ldx, offsets, first_frames, nu, flag, best_word, best_score, scores, best_path)))
             return rc;
     }
     return SAPR_OK;

@@ -926,7 +926,7 @@ int sapr_viterbi_v3_launch(sapr_ctx *ctx, sapr_models *m, const float *X, int ld
     const char *ex_env = getenv("SAPR_EXACT_WORDS");
     const bool exact = !ex_env || ex_env[0] != '0';
     SaprFlag flag;
-    ctx->flag_maxT = max_T; ctx->flag_M = m->M;
+    ctx->flag_maxT = max_T;
     for (int u0 = 0; u0 < B; u0 += chunk) {
         const int nu = std::min(chunk, B - u0);
         if (exact && (rc = sapr_flag_setup(ctx, &flag, u0 == 0))) return rc;
@@ -1006,7 +1006,7 @@ int sapr_viterbi_v3_launch(sapr_ctx *ctx, sapr_models *m, const float *X, int ld
         }
         SAPR_LAUNCH_CHECK(ctx);
         if (tail) SAPR_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev[9], 0));
-        if (exact && (rc = sapr_viterbi_redo_flagged(ctx, m, X, ldx, offsets, first_frames, flag, best_word, best_score, scores, best_path))) return rc;
+        if (exact && (rc = sapr_viterbi_redo_flagged(ctx, m, X, ldx, offsets, first_frames, nu, flag, best_word, best_score, scores, best_path))) return rc;
     }
     *taken = true;
     return SAPR_OK;
